@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — benchmark of the msmd_b200 hot path (contract: DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one batch of synthetic input.
 Workloads (BASELINE.json configs):
@@ -86,6 +86,26 @@ def ncu_traffic(kernel_key):
         return None
 
 
+DUMP_BYTES = 60 << 20      # --dump-outputs stays under 64 MB, .npy headers included
+
+
+def dump_outputs(outputs, out_dir, max_bytes=DUMP_BYTES, seed=0):
+    """Write each {name: tensor} as out_dir/<name>.npy in float32.  An output larger than an even share of max_bytes keeps
+    a fixed seeded sample of its matrices (one per index of all but the last two dims, e.g. one mesh per frame), in
+    ascending order: two builds run with the same arguments store the same entries."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = max_bytes // len(outputs)
+    for name, t in outputs.items():
+        rows = t.reshape(-1, *t.shape[max(1, t.dim() - 2):])
+        k = share // (rows[0].numel() * 4)
+        assert k > 0, f'{name}: one {tuple(rows.shape[1:])} matrix is larger than its {share}-byte share of the dump'
+        if k < rows.shape[0]:
+            idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(seed))[:k].sort().values
+            t = rows[idx.to(rows.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------
 class FlameWorkload:
     """configs[1]: standalone FLAME lbs decode, 8192 frames x 5023 verts, 300 shape + 100 expr, fp32."""
@@ -129,6 +149,10 @@ class FlameWorkload:
 
     def profile_step(self):
         return self.step()
+
+    def outputs(self, ret):
+        """{name: tensor} of what step() returned."""
+        return dict(vertices=ret)
 
     def step_e2e(self):
         sh, ex, po, ey = [h.to(self.device, non_blocking=True) for h in self.host]
@@ -355,6 +379,12 @@ class SamplerWorkload:
             return self._run_sharded(self.dev)
         return self._run(self.dev)
 
+    def outputs(self, ret):
+        """{name: tensor} of what step() produced: the codes and vertices it returned, or with total_clips the rank-0 host
+        buffers every clip was gathered into."""
+        codes, verts = (self.host_out, self.host_verts) if self.total_clips else ret
+        return dict(codes=codes, vertices=verts)
+
     def profile_step(self):
         # 10 eager bf16 sampling steps of the window left open by the last step(): only the per-step GEMMs are timed
         eng = self.model._eng
@@ -500,11 +530,18 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip the flame / pure-bf16 sub-records of the default line')
     ap.add_argument('--precision', default='hybrid', choices=['hybrid', 'bf16', 'fp16', 'fp32'],
                     help="sampler arithmetic; 'hybrid' (default, headline) keeps every step within 1e-3 of the fp32 reference")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy in float32, '
+                         'under 64 MB in all: large outputs keep a fixed seeded sample of their frames')
     a = ap.parse_args()
     if a.steps is None:
         a.steps = DEFAULT_STEPS[a.workload][0]
     if a.warmup is None:
         a.warmup = DEFAULT_STEPS[a.workload][1]
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs writes what the GPU path computed; the reference arm only times the CPU oracle')
     rank = int(os.environ.get('RANK', 0))
     local = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -558,6 +595,7 @@ def main():
     W = max(3, a.warmup)      # timing rule: at least 3 untimed warm-up steps
 
     def timed(fn, steps, profile=False, warm=None):
+        """(ms of `steps` timed calls of fn, what the last call returned)"""
         for _ in range(W if warm is None else warm):
             fn()
         barrier()
@@ -566,13 +604,14 @@ def main():
             _lib.lib().msmd_profile_enable(1)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()          # only the last result is held: each earlier one is freed before the next step allocates
         e1.record()
         barrier()
         if profile:
             _lib.lib().msmd_profile_enable(0)
-        return max_over_ranks(e0.elapsed_time(e1))
+        return max_over_ranks(e0.elapsed_time(e1)), last
 
     def kernel_time(w):
         timed(w.profile_step, 1, profile=True, warm=1)
@@ -582,10 +621,13 @@ def main():
         return kms / max(1, kn)
 
     with ClockSampler(local) as cs:
-        ms = timed(wl.step, a.steps)
+        ms, last = timed(wl.step, a.steps)
     clocks = cs.summary()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(wl.outputs(last), a.dump_outputs)
+    del last
     kernel_ms = kernel_time(wl)       # dominant-kernel duration, measured live with CUDA events on the launching stream
-    ms_e2e = timed(wl.step_e2e, a.steps, warm=1)
+    ms_e2e = timed(wl.step_e2e, a.steps, warm=1)[0]
     h2d, d2h = wl.e2e_bytes()
     dtype = wl.dtype_str() if isinstance(wl, SamplerWorkload) else wl.dtype
 
@@ -614,7 +656,7 @@ def main():
     if extras:
         # (1) the same workload in pure bf16 (every step one bf16 graph replay): the looser-precision figure, for reference
         wl.model.precision = wl.model.denoising_net.precision = 'bf16'
-        ms_b = timed(wl.step, 1, warm=1)
+        ms_b = timed(wl.step, 1, warm=1)[0]
         out['pure_bf16_mode'] = dict(value=wl.units(world) / (ms_b * 1e-3), unit=wl.unit, ms_per_step=ms_b, dtype='bf16',
                                      headline_over_this=(ms_b * a.steps) / ms,
                                      note='misses the 1e-3 per-step tolerance on the last ~9 of 500 steps (x0_hat error 6.5e-3 '
@@ -624,9 +666,9 @@ def main():
         torch.cuda.empty_cache()
         fw = FlameWorkload()
         fw.setup(device, rank, world)
-        ms_f = timed(fw.step, 20, warm=5)
+        ms_f = timed(fw.step, 20, warm=5)[0]
         k_f = kernel_time(fw)
-        ms_fe = timed(fw.step_e2e, 10, warm=2)
+        ms_fe = timed(fw.step_e2e, 10, warm=2)[0]
         fh2d, fd2h = fw.e2e_bytes()
         out['flame'] = dict(metric=fw.metric, value=fw.units(world) * 20 / (ms_f * 1e-3), unit=fw.unit, ms_per_step=ms_f / 20,
                             dtype=fw.dtype, config=fw.config(world),

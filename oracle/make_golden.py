@@ -331,12 +331,110 @@ def gen_denoiser_parts():
     print('denoiser_parts.npz', dyn.shape, sta.shape, alp.shape)
 
 
+VAR_GOLD = dict(N=2, T=4, seed=5, weight_seed=1234, stride=3)     # every 3rd frame is stored (size)
+VARIANTS = [dict(cfg_cond=[], flexibility=0.3), dict(cfg_cond=['audio'], flexibility=0.0),
+            dict(cfg_cond=['style'], flexibility=0.5), dict(cfg_cond=['audio', 'style'], flexibility=1.0, cfg_mode='independent')]
+
+
+def variant_kwargs(v):
+    return dict(cfg_mode=v.get('cfg_mode', 'incremental'), cfg_cond=v['cfg_cond'], cfg_scale=[1.3, 1.6][:len(v['cfg_cond'])],
+                flexibility=v['flexibility'])
+
+
+def dropin_state_dict(weight_seed, **over):
+    """state_dict of the package's drop-in MSMD with synth weights (key for key the reference's, see
+    tests/test_oracle_denoiser.py::test_dropin_state_dict_layout)."""
+    import torch.nn as nn
+    from msmd_b200 import model as M
+    m = M.MSMD(ref_shims.pinned_args(**over), 'cpu', True, use_head_alpha=False, regularize_alpha="None",
+               audio_encoder=nn.Identity())
+    m.load_state_dict(synth.fill_state_dict(synth.param_spec(m), weight_seed), strict=False)
+    return {k: v.detach() for k, v in m.state_dict().items()}
+
+
+# The two sections below store what tests compare with the reference live.  The committed files were written without the
+# reference (source = 'oracle'): by oracle/denoiser.py, oracle/rotations.py and oracle/flame_lbs.py, unchanged since the
+# commits whose live tests pinned them to the unmodified reference (sampler variants: rel-L2 < 5e-6; rotations: 3e-6
+# absolute; FLAME vertices and lbs joints: rel-L2 < 1e-6).  With the reference mounted they are written from it.
+def gen_sampler_variants():
+    """MSMD.sample for guidance sets other than the default (none / audio only / style only / independent), sigma
+    'flexibility' > 0, and models with and without the indicator input: 4 sampling steps each."""
+    from . import denoiser as D
+    c, live, res = VAR_GOLD, ref_shims.available(), {}
+    i = synth.sampler_inputs(c['N'], c['T'], c['seed'])
+    for use_indicator in (True, False):
+        ind = i['indicator'] if use_indicator else None
+        if live:
+            ref, args = ref_msmd(c['weight_seed'], n_diff_steps=c['T'], use_indicator=use_indicator)
+        else:
+            sd = dropin_state_dict(c['weight_seed'], n_diff_steps=c['T'], use_indicator=use_indicator)
+            args = ref_shims.pinned_args(n_diff_steps=c['T'], use_indicator=use_indicator)
+        for k, v in enumerate(VARIANTS):
+            if live:
+                with ref_shims.inject_randn_like([i['z'][t] for t in range(c['T'], 1, -1)]):
+                    out, _, _ = ref.sample(i['audio_feat'], i['shape'], i['style'], motion_at_T=i['x_T'], indicator=ind,
+                                           **variant_kwargs(v))
+            else:
+                out, _, _ = D.sample(sd, args, i['audio_feat'], i['shape'], i['style'], x_T=i['x_T'], z=i['z'],
+                                     indicator=ind, **variant_kwargs(v))
+            res[f'indicator{int(use_indicator)}_variant{k}'] = out[:, ::c['stride']].numpy()
+    res['source'] = np.array('reference' if live else 'oracle')
+    np.savez_compressed(os.path.join(OUT, 'sampler_variants.npz'), **res)
+    print('sampler_variants.npz', res['source'], len(res) - 1)
+
+
+REF_MOD_GOLD = dict(rot_n=128, rot_seed=99, conventions=('ZYX', 'YZX'), raw_seed=5, V=300, n_shape=100, n_exp=50, B=16,
+                    seed=8, stride=3)     # every 3rd vertex is stored (size)
+
+
+def gen_ref_modules():
+    """Euler conventions ZYX / YZX both ways, FLAME.forward and lbs (vertices + posed joints) on a 300-vertex model with
+    100 + 50 betas, and the MSMD state_dict layout (key -> shape, audio encoder excluded)."""
+    from . import flame_lbs, rotations as R
+    c, live, res = REF_MOD_GOLD, ref_shims.available(), {}
+    i = rot_inputs(n=c['rot_n'], seed=c['rot_seed'])
+    assets = synth.flame_assets(c['raw_seed'], c['V'], c['n_shape'], c['n_exp'])
+    sh, ex, po, ey = synth.flame_inputs(c['B'], c['n_shape'], c['n_exp'], c['seed'])
+    full = flame_lbs.flame_full_pose(po, ey, c['B'])
+    betas = torch.cat([sh, ex], 1)
+    if live:
+        m = ref_shims.ref_modules()
+        for conv in c['conventions']:
+            mats = m.rc.euler_angles_to_matrix(i['euler'], conv)
+            res[f'euler_angles_to_matrix_{conv}'] = mats.numpy()
+            res[f'matrix_to_euler_angles_{conv}'] = m.rc.matrix_to_euler_angles(mats, conv).numpy()
+        fl = ref_shims.ref_flame(synth.flame_raw(c['raw_seed'], c['V'], 400), c['n_shape'], c['n_exp'])
+        res['flame_verts'] = fl(sh, ex, po, ey, return_lm2d=False, return_lm3d=False)[0][:, ::c['stride']].numpy()
+        v, j = m.lbs.lbs(betas, full, assets['v_template'][None].expand(c['B'], -1, -1), assets['shapedirs'],
+                         assets['posedirs'], assets['J_regressor'], torch.tensor(assets['parents']), assets['lbs_weights'])
+        sd = m.model.get_diffusion_model(ref_shims.pinned_args(), 'cpu').state_dict()
+    else:
+        for conv in c['conventions']:
+            mats = R.euler_angles_to_matrix(i['euler'].numpy(), conv)
+            res[f'euler_angles_to_matrix_{conv}'] = mats
+            res[f'matrix_to_euler_angles_{conv}'] = R.matrix_to_euler_angles(mats, conv)
+        res['flame_verts'] = flame_lbs.flame_forward(assets, sh, ex, po, ey)[:, ::c['stride']].numpy()
+        v, j = flame_lbs.lbs(betas, full, assets['v_template'], assets['shapedirs'], assets['posedirs'],
+                             assets['J_regressor'], assets['parents'], assets['lbs_weights'])
+        sd = dropin_state_dict(1234)
+    res['lbs_verts'], res['lbs_joints'] = v[:, ::c['stride']].numpy(), j.numpy()
+    keys = sorted(k for k in sd if not k.startswith('audio_encoder.'))
+    res['state_dict_keys'] = np.array(keys)
+    res['state_dict_shapes'] = np.array([','.join(map(str, sd[k].shape)) for k in keys])
+    res['source'] = np.array('reference' if live else 'oracle')
+    np.savez_compressed(os.path.join(OUT, 'ref_modules.npz'), **res)
+    print('ref_modules.npz', res['source'], len(keys), 'state_dict keys')
+
+
 SECTIONS = dict(decode=gen_decode, denoiser_parts=gen_denoiser_parts, rot=gen_rot, flame=gen_flame, denoiser=gen_denoiser, sampler=gen_sampler, style=gen_style,
-                audio=gen_audio, infer=gen_infer, separate=gen_separate, sampler_noise=gen_sampler_noise)
+                audio=gen_audio, infer=gen_infer, separate=gen_separate, sampler_noise=gen_sampler_noise,
+                sampler_variants=gen_sampler_variants, ref_modules=gen_ref_modules)
+WITHOUT_REFERENCE = {'sampler_variants', 'ref_modules'}     # sections that can fall back to the pinned oracle
 
 
 def main(argv):
-    assert ref_shims.available(), 'needs /root/reference'
+    assert ref_shims.available() or (argv and set(argv) <= WITHOUT_REFERENCE), \
+        f'needs the unmodified reference (MSMD_REFERENCE); without it only {sorted(WITHOUT_REFERENCE)}'
     os.makedirs(OUT, exist_ok=True)
     torch.set_grad_enabled(False)
     names = argv or list(SECTIONS)

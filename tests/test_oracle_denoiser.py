@@ -9,7 +9,7 @@ import torch
 from conftest import GOLDEN, rel_l2
 from helpers import cpu_state_dict, make_msmd
 from oracle import denoiser as D, ref_shims, synth
-from oracle.make_golden import DEN_GOLD, SAMP_GOLD
+from oracle.make_golden import DEN_GOLD, SAMP_GOLD, VAR_GOLD, VARIANTS, ref_msmd, variant_kwargs
 
 
 @pytest.fixture(scope='module')
@@ -69,7 +69,8 @@ def test_cross_attention_is_step_invariant_for_motion_rows(msmd):
 
 
 def test_dropin_state_dict_layout(msmd):
-    """SURVEY App. E keys/shapes; also checked key-for-key against the reference module when it is mounted."""
+    """SURVEY App. E keys/shapes, and key for key the reference module's (stored in tests/golden/ref_modules.npz; checked
+    live too when the reference is mounted)."""
     m, args = msmd
     sd = m.state_dict()
     assert sd['denoising_net.PE'].shape == (1, 111, 512)
@@ -77,11 +78,13 @@ def test_dropin_state_dict_layout(msmd):
     assert sd['denoising_net.motion_dec.2.weight'].shape == (71, 256)
     assert sd['denoising_net.feature_proj.weight'].shape == (512, 68)
     assert sd['null_style_feat'].shape == (1, 1, 256) and sd['start_audio_feat'].shape == (1, 10, 512)
+    g = np.load(os.path.join(GOLDEN, 'ref_modules.npz'))
+    want = {k: tuple(int(n) for n in s.split(',') if n) for k, s in zip(g['state_dict_keys'], g['state_dict_shapes'])}
     if ref_shims.available():
         r = ref_shims.ref_modules()
         rm = r.model.get_diffusion_model(ref_shims.pinned_args(), 'cpu')
-        want = {k: tuple(v.shape) for k, v in rm.state_dict().items() if not k.startswith('audio_encoder.')}
-        assert {k: tuple(v.shape) for k, v in sd.items()} == want
+        assert {k: tuple(v.shape) for k, v in rm.state_dict().items() if not k.startswith('audio_encoder.')} == want
+    assert {k: tuple(v.shape) for k, v in sd.items()} == want
 
 
 def test_no_cpu_path_for_model(msmd):
@@ -109,25 +112,24 @@ def test_oracle_sampler_noise_target_matches_golden():
         assert rel_l2(nxt, gold[t - 1]) < 5e-6, t
 
 
-VARIANTS = [dict(cfg_cond=[], flexibility=0.3), dict(cfg_cond=['audio'], flexibility=0.0),
-            dict(cfg_cond=['style'], flexibility=0.5), dict(cfg_cond=['audio', 'style'], flexibility=1.0, cfg_mode='independent')]
-
-
-@pytest.mark.skipif(not ref_shims.available(), reason='needs /root/reference (build container)')
 @pytest.mark.parametrize('use_indicator', [True, False])
 def test_oracle_sampler_variants_match_reference(use_indicator):
     """Guidance sets other than the default (none / audio only / style only), sigma 'flexibility' > 0 and a model built
-    without the indicator input: the oracle against the unmodified reference, 4 sampling steps each."""
-    from oracle.make_golden import ref_msmd
-    T = 4
-    ref, args = ref_msmd(1234, n_diff_steps=T, use_indicator=use_indicator)
-    sd = {k: v.detach() for k, v in ref.state_dict().items()}
-    i = synth.sampler_inputs(2, T, 5)
+    without the indicator input, 4 sampling steps each: the oracle against the reference's outputs stored in
+    tests/golden/sampler_variants.npz (every 3rd frame; see oracle/make_golden.py for how they were made) and, when the
+    unmodified reference is mounted, against it live on every frame."""
+    c = VAR_GOLD
+    m, args = make_msmd('cpu', n_diff_steps=c['T'], use_indicator=use_indicator)
+    sd = cpu_state_dict(m)
+    gold = np.load(os.path.join(GOLDEN, 'sampler_variants.npz'))
+    i = synth.sampler_inputs(c['N'], c['T'], c['seed'])
     ind = i['indicator'] if use_indicator else None
-    for v in VARIANTS:
-        kw = dict(cfg_mode=v.get('cfg_mode', 'incremental'), cfg_cond=v['cfg_cond'], cfg_scale=[1.3, 1.6][:len(v['cfg_cond'])],
-                  flexibility=v['flexibility'])
-        with ref_shims.inject_randn_like([i['z'][t] for t in range(T, 1, -1)]):
-            want, _, _ = ref.sample(i['audio_feat'], i['shape'], i['style'], motion_at_T=i['x_T'], indicator=ind, **kw)
+    ref = ref_msmd(c['weight_seed'], n_diff_steps=c['T'], use_indicator=use_indicator)[0] if ref_shims.available() else None
+    for k, v in enumerate(VARIANTS):
+        kw = variant_kwargs(v)
         got, _, _ = D.sample(sd, args, i['audio_feat'], i['shape'], i['style'], x_T=i['x_T'], z=i['z'], indicator=ind, **kw)
-        assert rel_l2(got, want) < 5e-6, v
+        assert rel_l2(got[:, ::c['stride']], gold[f'indicator{int(use_indicator)}_variant{k}']) < 5e-6, v
+        if ref is not None:
+            with ref_shims.inject_randn_like([i['z'][t] for t in range(c['T'], 1, -1)]):
+                want, _, _ = ref.sample(i['audio_feat'], i['shape'], i['style'], motion_at_T=i['x_T'], indicator=ind, **kw)
+            assert rel_l2(got, want) < 5e-6, v

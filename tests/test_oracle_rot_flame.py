@@ -1,6 +1,6 @@
 """CPU: the oracle (oracle/rotations.py, oracle/flame_lbs.py) against the committed golden
 vectors produced from the unmodified reference (oracle/make_golden.py), and - when
-/root/reference is present - against the reference modules directly."""
+the reference is mounted (MSMD_REFERENCE) - against the reference modules directly."""
 import os
 
 import numpy as np
@@ -9,7 +9,7 @@ import torch
 
 from conftest import GOLDEN, rel_l2
 from oracle import flame_lbs, ref_shims, rotations as R, synth
-from oracle.make_golden import FLAME_GOLD, ROT_CONVENTIONS, rot_inputs
+from oracle.make_golden import FLAME_GOLD, REF_MOD_GOLD, ROT_CONVENTIONS, rot_inputs
 
 
 @pytest.fixture(scope='module')
@@ -95,27 +95,40 @@ def test_oracle_flame_known_answers():
     assert (v[0] - want).abs().max() < 1e-6
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason='reference not mounted (GPU box)')
 def test_oracle_against_reference_modules():
-    m = ref_shims.ref_modules()
-    i = rot_inputs(n=128, seed=99)
-    for conv in ('ZYX', 'YZX'):
-        want = m.rc.euler_angles_to_matrix(i['euler'], conv)
-        assert np.abs(R.euler_angles_to_matrix(i['euler'].numpy(), conv) - want.numpy()).max() < 3e-6
-        got = R.matrix_to_euler_angles(want.numpy(), conv)
-        assert np.abs(got - m.rc.matrix_to_euler_angles(want, conv).numpy()).max() < 3e-6
-    raw = synth.flame_raw(5, 300, 400)
-    fl = ref_shims.ref_flame(raw, 100, 50)
-    assets = synth.flame_assets(5, 300, 100, 50)
-    sh, ex, po, ey = synth.flame_inputs(16, 100, 50, 8)
-    with torch.no_grad():
-        want, _, _ = fl(sh, ex, po, ey, return_lm2d=False, return_lm3d=False)
-    assert rel_l2(flame_lbs.flame_forward(assets, sh, ex, po, ey), want) < 1e-6
+    """Euler conventions ZYX / YZX both ways, FLAME.forward and lbs (vertices and posed joints) on a 300-vertex model
+    with 100 + 50 betas: the oracle against the reference's outputs stored in tests/golden/ref_modules.npz (every 3rd
+    vertex; see oracle/make_golden.py for how they were made) and, when the unmodified reference is mounted, against it
+    live."""
+    c = REF_MOD_GOLD
+    g = np.load(os.path.join(GOLDEN, 'ref_modules.npz'))
+    m = ref_shims.ref_modules() if ref_shims.available() else None
+    i = rot_inputs(n=c['rot_n'], seed=c['rot_seed'])
+    for conv in c['conventions']:
+        mats = R.euler_angles_to_matrix(i['euler'].numpy(), conv)
+        assert np.abs(mats - g[f'euler_angles_to_matrix_{conv}']).max() < 3e-6
+        got = R.matrix_to_euler_angles(g[f'euler_angles_to_matrix_{conv}'], conv)
+        assert np.abs(got - g[f'matrix_to_euler_angles_{conv}']).max() < 3e-6
+        if m is not None:
+            want = m.rc.euler_angles_to_matrix(i['euler'], conv)
+            assert np.abs(mats - want.numpy()).max() < 3e-6
+            got = R.matrix_to_euler_angles(want.numpy(), conv)
+            assert np.abs(got - m.rc.matrix_to_euler_angles(want, conv).numpy()).max() < 3e-6
+    assets = synth.flame_assets(c['raw_seed'], c['V'], c['n_shape'], c['n_exp'])
+    sh, ex, po, ey = synth.flame_inputs(c['B'], c['n_shape'], c['n_exp'], c['seed'])
+    verts = flame_lbs.flame_forward(assets, sh, ex, po, ey)
+    assert rel_l2(verts[:, ::c['stride']], g['flame_verts']) < 1e-6
     # joints (lbs returns J_transformed)
-    full = flame_lbs.flame_full_pose(po, ey, 16)
+    full = flame_lbs.flame_full_pose(po, ey, c['B'])
     v2, j2 = flame_lbs.lbs(torch.cat([sh, ex], 1), full, assets['v_template'], assets['shapedirs'],
                            assets['posedirs'], assets['J_regressor'], assets['parents'], assets['lbs_weights'])
-    vr, jr = m.lbs.lbs(torch.cat([sh, ex], 1), full, assets['v_template'][None].expand(16, -1, -1),
-                       assets['shapedirs'], assets['posedirs'], assets['J_regressor'],
-                       torch.tensor(assets['parents']), assets['lbs_weights'])
-    assert rel_l2(v2, vr) < 1e-6 and rel_l2(j2, jr) < 1e-6
+    assert rel_l2(v2[:, ::c['stride']], g['lbs_verts']) < 1e-6 and rel_l2(j2, g['lbs_joints']) < 1e-6
+    if m is not None:
+        fl = ref_shims.ref_flame(synth.flame_raw(c['raw_seed'], c['V'], 400), c['n_shape'], c['n_exp'])
+        with torch.no_grad():
+            want, _, _ = fl(sh, ex, po, ey, return_lm2d=False, return_lm3d=False)
+        assert rel_l2(verts, want) < 1e-6
+        vr, jr = m.lbs.lbs(torch.cat([sh, ex], 1), full, assets['v_template'][None].expand(c['B'], -1, -1),
+                           assets['shapedirs'], assets['posedirs'], assets['J_regressor'],
+                           torch.tensor(assets['parents']), assets['lbs_weights'])
+        assert rel_l2(v2, vr) < 1e-6 and rel_l2(j2, jr) < 1e-6
