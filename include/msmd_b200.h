@@ -124,7 +124,9 @@ typedef struct {
   int n_basis;          /* 4   */
   int n_diff_steps;     /* 500 */
   int use_indicator;    /* 1   */
-  int align_mask_width; /* 1 (the only width with step-invariant cross attention; others unsupported) */
+  int align_mask_width; /* 1; >= 0.  Band of the cross-attention mask: motion token i sees memory tokens
+                         * [i-1-(w-1), i-1+(w-1)], the person token all of them; 0 = no mask.  Width 1 caches the motion
+                         * rows' cross attention per window; any other width runs the banded attention on every step */
   int target_noise;     /* 0: network predicts the sample (args.target == 'sample'), 1: the noise */
   int max_seqs;         /* capacity in sequences (E * clips); workspaces are sized for it at create */
   int precision;        /* 0: bf16 tensor-core GEMMs (fp32 accumulate, fp32 LayerNorm/softmax statistics);
@@ -147,7 +149,7 @@ int msmd_load_weights(msmd_model* m, const char* const* names, const void* const
 
 /* Per-window, step-invariant work (SURVEY section 0): memory K/V projections of every layer, the
  * cross-attention output of motion rows (== out_proj(v_proj(audio[i-1])) under the width-1 alignment
- * mask), person_proj, previous-motion projection, static-basis MLPs.
+ * mask; other widths attend on every step), person_proj, previous-motion projection, static-basis MLPs.
  * Arguments are exactly the conditioning tensors of DenoisingNetwork_MSMD.forward (model.py:914):
  *   audio [S,L,d], person [S,d_shape+d_style], style [S,d_style], prev_motion [S,Lp,dm],
  *   prev_audio [S,Lp,d], indicator [S,L] or NULL.  S = E*NX.  Everything later calls need is copied or projected

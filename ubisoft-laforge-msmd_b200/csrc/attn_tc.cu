@@ -1,5 +1,7 @@
 // Self-attention of the decoder layers on tcgen05 (nn.TransformerDecoderLayer._sa_block -> nn.MultiheadAttention,
-// no mask: DenoisingNetwork_MSMD.forward passes tgt_mask=None, model.py:951-958).
+// no mask: DenoisingNetwork_MSMD.forward passes tgt_mask=None, model.py:951-958), and, as the CROSS instantiation, the
+// banded cross-attention (_mha_block with memory_mask = alignment_mask, model.py:879-883) that every align_mask_width
+// other than 1 needs on every step: Q from its own [S*T, d] buffer, K|V from the per-window cache [S*Tk, 2d].
 //
 // One "job" = one (sequence, head): S = Q K^T (128 x 112 x 64), row softmax, O = P V (128 x 64 x 112), T <= 112
 // tokens so a sequence is a single tile and there is no online-softmax rescaling.  The legacy mma.sync path
@@ -43,6 +45,7 @@ struct AttnParams {
   CUtensorMap out_map;     // ctx rows, box {64 head dims, T rows}: a job's store covers exactly its sequence
   int S, T, H, jobs;
   unsigned long long* trace;   // -DMSMD_ATTN_TRACE builds: clock64 stamps of CTA 0, [role 0..2][job 0..15][8]
+  int Tk, width;               // CROSS: keys per sequence, alignment band (0 = no band)
 };
 
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* v) {
@@ -77,7 +80,11 @@ __device__ __forceinline__ void attn_stamp(unsigned long long* tr, int role, int
 #endif
 }
 
-template <bool TAIL16, bool F16>
+// CROSS = false: q|k|v rows of one packed [S*T, 3d] buffer, every key visible (keys >= T masked; TAIL16: T > kKeys - 16).
+// CROSS = true: q [S*T, d], k|v [S*Tk, 2d]; token 0 sees every key, token r >= 1 sees key c iff |c - (r-1)| <= width-1
+// (width 0: every key).  The 112-key tile covers Tk <= 112 keys; the rows past Tk (next sequence / TMA zero fill) are
+// masked.  TAIL16 is unused.
+template <bool TAIL16, bool F16, bool CROSS>
 __global__ void __launch_bounds__(kThreads, 1) self_attn_tc_kernel(const __grid_constant__ AttnParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -127,8 +134,13 @@ __global__ void __launch_bounds__(kThreads, 1) self_attn_tc_kernel(const __grid_
         uint8_t* sq = stage_base + st * kStageBytes;
         mbar_expect_tx(&full_bar[st], kStageBytes);
         tma_load_2d(sq, &p.q_map, &full_bar[st], h * 64, s * p.T);
-        tma_load_2d(sq + kQBytes, &p.kv_map, &full_bar[st], d + h * 64, s * p.T);
-        tma_load_2d(sq + kQBytes + kKVBytes, &p.kv_map, &full_bar[st], 2 * d + h * 64, s * p.T);
+        if constexpr (CROSS) {
+          tma_load_2d(sq + kQBytes, &p.kv_map, &full_bar[st], h * 64, s * p.Tk);
+          tma_load_2d(sq + kQBytes + kKVBytes, &p.kv_map, &full_bar[st], d + h * 64, s * p.Tk);
+        } else {
+          tma_load_2d(sq + kQBytes, &p.kv_map, &full_bar[st], d + h * 64, s * p.T);
+          tma_load_2d(sq + kQBytes + kKVBytes, &p.kv_map, &full_bar[st], 2 * d + h * 64, s * p.T);
+        }
       }
     }
     __syncwarp();
@@ -183,6 +195,18 @@ __global__ void __launch_bounds__(kThreads, 1) self_attn_tc_kernel(const __grid_
     const int swz = r & 7;
     const float kScale = 0.125f * 1.4426950408889634f;   // 1/sqrt(64) * log2(e)
     const bool issuer = (warp - 2) % 4 == 0 && lane == 0;   // one thread per group owns the group's TMA stores
+    // CROSS: visible keys of this row as a bit mask over the 112-key tile (bit c of vis[c / 32]).  Token 0, the no-band
+    // case and the tile rows past T (never stored) see all Tk keys; a motion row always sees its own column r-1 < Tk.
+    uint32_t vis[(kKeys + 31) / 32] = {};
+    if constexpr (CROSS) {
+      int lo = 0, hi = p.Tk - 1;
+      if (p.width > 0 && r >= 1 && r < p.T) { lo = max(0, r - p.width); hi = min(hi, r + p.width - 2); }
+#pragma unroll
+      for (int k = 0; k < (kKeys + 31) / 32; ++k) {
+        const int a = max(lo - 32 * k, 0), b = min(hi - 32 * k, 31);
+        vis[k] = a <= b ? (0xffffffffu >> (31 - b + a)) << a : 0u;
+      }
+    }
     for (int i = g, it = 0; i < njobs; i += 2, ++it) {
       const int job = job0 + i;
       const int s = job / p.H, h = job % p.H;
@@ -202,7 +226,10 @@ __global__ void __launch_bounds__(kThreads, 1) self_attn_tc_kernel(const __grid_
       float m = -INFINITY;
 #pragma unroll
       for (int c = 0; c < kKeys; ++c) {
-        if (c >= kKeys - 16 || !TAIL16) {   // only the last 16 key columns can lie beyond T (TAIL16: T > kKeys - 16)
+        if constexpr (CROSS) {
+          const float x = (vis[c >> 5] >> (c & 31)) & 1u ? __uint_as_float(v[c]) : -INFINITY;
+          v[c] = __float_as_uint(x);
+        } else if (c >= kKeys - 16 || !TAIL16) {   // only the last 16 key columns can lie beyond T (TAIL16: T > kKeys - 16)
           const float x = c < p.T ? __uint_as_float(v[c]) : -INFINITY;
           v[c] = __float_as_uint(x);
         }
@@ -299,16 +326,16 @@ int self_attn_tc_launch(const bf16* qkv, bf16* ctx, int S, int T, int H, int fp1
 #endif
   static bool attr = false;
   if (!attr) {
-    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
     attr = true;
   }
   ProfileScope prof("self_attn", st);
   const int grid = p.jobs < kNumSMs ? p.jobs : kNumSMs;
-  auto kern = T > kKeys - 16 ? (fp16 ? self_attn_tc_kernel<true, true> : self_attn_tc_kernel<true, false>)
-                             : (fp16 ? self_attn_tc_kernel<false, true> : self_attn_tc_kernel<false, false>);
+  auto kern = T > kKeys - 16 ? (fp16 ? self_attn_tc_kernel<true, true, false> : self_attn_tc_kernel<true, false, false>)
+                             : (fp16 ? self_attn_tc_kernel<false, true, false> : self_attn_tc_kernel<false, false, false>);
   MSMD_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kThreads), kSmemBytes, st, p));
   MSMD_CHECK_LAUNCH();
 #ifdef MSMD_ATTN_TRACE
@@ -334,6 +361,36 @@ int self_attn_tc_launch(const bf16* qkv, bf16* ctx, int S, int T, int H, int fp1
     }
   }
 #endif
+  return MSMD_OK;
+}
+
+int cross_attn_tc_launch(const bf16* q, const bf16* kv, bf16* ctx, int S, int T, int Tk, int H, int width, int fp16,
+                         cudaStream_t st) {
+  MSMD_REQUIRE(T >= 2 && T <= kKeys && Tk >= T - 1 && Tk <= kKeys,
+               "cross_attn: %d queries / %d keys exceed the %d-token tile (or a motion row has no key)", T, Tk, kKeys);
+  MSMD_REQUIRE(H >= 1 && S >= 1 && width >= 0, "cross_attn: empty problem or negative band width");
+  AttnParams p;
+  memset(&p, 0, sizeof(p));
+  const int d = H * 64;
+  int rc;
+  const auto dt16 = fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  const uint64_t rows = (uint64_t)S * T, krows = (uint64_t)S * Tk;
+  if ((rc = make_tmap_2d(&p.q_map, q, dt16, d, rows, (uint64_t)d * 2, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+  if ((rc = make_tmap_2d(&p.kv_map, kv, dt16, 2 * d, krows, (uint64_t)2 * d * 2, 64, kKeys, CU_TENSOR_MAP_SWIZZLE_128B)))
+    return rc;
+  if ((rc = make_tmap_2d(&p.out_map, ctx, dt16, d, rows, (uint64_t)d * 2, 64, T, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+  p.S = S; p.T = T; p.H = H; p.jobs = S * H; p.Tk = Tk; p.width = width;
+  static bool attr = false;
+  if (!attr) {
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_tc_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    attr = true;
+  }
+  ProfileScope prof("cross_attn", st);
+  const int grid = p.jobs < kNumSMs ? p.jobs : kNumSMs;
+  auto kern = fp16 ? self_attn_tc_kernel<true, true, true> : self_attn_tc_kernel<true, false, true>;
+  MSMD_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kThreads), kSmemBytes, st, p));
+  MSMD_CHECK_LAUNCH();
   return MSMD_OK;
 }
 

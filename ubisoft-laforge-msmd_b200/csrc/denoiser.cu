@@ -7,7 +7,7 @@
 //   qkv   [M, 3d]    bf16   packed q|k|v
 //   ctx   [M, d]     bf16   attention output
 //   h     [M, d_ff]  bf16   GELU(FF1)
-//   kv[l] [S*(T-1), 2d] bf16 and ca[l] [S, T-1, d] bf16: per-window cross-attention caches
+//   kv[l] [S*(T-1), 2d] bf16 and ca[l] [S, T-1, d] bf16: per-window cross-attention caches (ca only at align_mask_width 1)
 //   dec   [M, 80]    fp32   motion_dec output (67 dynamic + 4 alphas, row stride padded to 80)
 #include "denoiser_kernels.cuh"
 #include "gemm_tc.cuh"
@@ -186,11 +186,19 @@ int run_forward_f32(msmd_model* m, const float* xrows, cudaStream_t st) {
     if ((rc = gemm32(m, m->fx, d, w.Wqkv_h, w.Wqkv_l, d, w.bqkv, m->fqkv, 3 * d, M, 3 * d, d, 0, st))) return rc;
     if ((rc = self_attn_f32_launch(m->fqkv, m->fctx, S, T, c.n_heads, st))) return rc;
     if ((rc = gemm32(m, m->fctx, d, w.Wo_h, w.Wo_l, d, w.bo, m->fy, d, M, d, d, 0, st))) return rc;
-    if ((rc = ln_f32_launch(m->fy, m->fx, w.g1, w.be1, w.ca32, w.g2, w.be2, m->fx, m->fx0c, M, T, st))) return rc;
-    if ((rc = gemm32(m, m->fx0c, d, w.Wq0_h, w.Wq0_l, d, w.bq0, m->fq0, d, S, d, d, 0, st))) return rc;
-    if ((rc = cross_attn_row0_f32_launch(m->fq0, w.kv32, m->fctx0, S, T - 1, c.n_heads, st))) return rc;
-    if ((rc = gemm32(m, m->fctx0, d, w.Wco_h, w.Wco_l, d, w.bco, m->fy0, d, S, d, d, 0, st))) return rc;
-    if ((rc = ln_row0_f32_launch(m->fy0, m->fx0c, w.g2, w.be2, m->fx, S, T, st))) return rc;
+    if (c.align_mask_width == 1) {
+      if ((rc = ln_f32_launch(m->fy, m->fx, w.g1, w.be1, w.ca32, w.g2, w.be2, m->fx, m->fx0c, M, T, st))) return rc;
+      if ((rc = gemm32(m, m->fx0c, d, w.Wq0_h, w.Wq0_l, d, w.bq0, m->fq0, d, S, d, d, 0, st))) return rc;
+      if ((rc = cross_attn_row0_f32_launch(m->fq0, w.kv32, m->fctx0, S, T - 1, c.n_heads, st))) return rc;
+      if ((rc = gemm32(m, m->fctx0, d, w.Wco_h, w.Wco_l, d, w.bco, m->fy0, d, S, d, d, 0, st))) return rc;
+      if ((rc = ln_row0_f32_launch(m->fy0, m->fx0c, w.g2, w.be2, m->fx, S, T, st))) return rc;
+    } else {   // banded cross attention of every row (q into the free qkv workspace), out-proj, residual + norm2
+      if ((rc = ln_f32_launch(m->fy, m->fx, w.g1, w.be1, nullptr, nullptr, nullptr, m->fx, nullptr, M, T, st))) return rc;
+      if ((rc = gemm32(m, m->fx, d, w.Wq0_h, w.Wq0_l, d, w.bq0, m->fqkv, d, M, d, d, 0, st))) return rc;
+      if ((rc = cross_attn_f32_launch(m->fqkv, w.kv32, m->fctx, S, T, T - 1, c.n_heads, c.align_mask_width, st))) return rc;
+      if ((rc = gemm32(m, m->fctx, d, w.Wco_h, w.Wco_l, d, w.bco, m->fy, d, M, d, d, 0, st))) return rc;
+      if ((rc = ln_f32_launch(m->fy, m->fx, w.g2, w.be2, nullptr, nullptr, nullptr, m->fx, nullptr, M, T, st))) return rc;
+    }
     if ((rc = gemm32(m, m->fx, d, w.W1_h, w.W1_l, d, w.b1, m->fh, c.d_ff, M, c.d_ff, d, 1, st))) return rc;
     if ((rc = gemm32(m, m->fh, c.d_ff, w.W2_h, w.W2_l, c.d_ff, w.b2, m->fy, d, M, d, c.d_ff, 0, st))) return rc;
     if ((rc = ln_f32_launch(m->fy, m->fx, w.g3, w.be3, nullptr, nullptr, nullptr, m->fx, nullptr, M, T, st))) return rc;
@@ -210,6 +218,7 @@ int window_begin_f32(msmd_model* m, cudaStream_t st) {
   if ((rc = build_memory_f32(m->w_prev_audio, m->w_audio, m->fmem, S, c.n_prev_motions, c.n_motions, d, st))) return rc;
   for (auto& w : m->L) {
     if ((rc = gemm32(m, m->fmem, d, w.Wkv_h, w.Wkv_l, d, w.bkv, w.kv32, 2 * d, S * Tk, 2 * d, d, 0, st))) return rc;
+    if (c.align_mask_width != 1) continue;   // the motion rows' attention depends on the query: no ca cache
     // v half of the kv cache as a strided A operand: row stride 2d, K = d columns starting at column d
     if ((rc = split_f16(w.kv32, m->ws_hi, m->ws_lo, (int64_t)S * Tk * 2 * d, st, m->overflow))) return rc;
     GemmDesc g;
@@ -240,28 +249,42 @@ int run_forward(msmd_model* m, const float* xrows, cudaStream_t st, int fmt) {
                *Wq0 = fmt ? (const void*)w.Wq0_h : w.Wq0, *Wco = fmt ? (const void*)w.Wco_h : w.Wco,
                *W1 = fmt ? (const void*)w.W1_h : w.W1, *W2 = fmt ? (const void*)w.W2_h : w.W2;
     const bf16 *kv = fmt ? w.kvh : w.kv, *ca = fmt ? w.cah : w.ca;
-    // self-attention block (nn.TransformerDecoderLayer._sa_block) + norm1, then the cached cross-attention
+    // self-attention block (nn.TransformerDecoderLayer._sa_block) + norm1, then (width 1) the cached cross-attention
     // rows + norm2 for motion tokens
     if ((rc = gemm(fmt, m->x, d, Wqkv, d, w.bqkv, nullptr, 0, m->qkv, 3 * d, 0, M, 3 * d, d, 0, st))) return rc;
     if ((rc = self_attn_tc_launch(m->qkv, m->ctx, S, T, c.n_heads, fmt, st))) return rc;
     if ((rc = gemm(fmt, m->ctx, d, Wo, d, w.bo, nullptr, 0, m->y, d, 0, M, d, d, 0, st))) return rc;
+    static const int row0_max_s = [] { const char* e = getenv("MSMD_ROW0_FUSED_MAX_S"); return e ? atoi(e) : kRow0FusedMaxS; }();
     LnParams lp{};
     lp.resid = m->x;
     lp.y = m->y; lp.g1 = w.g1; lp.b1 = w.be1; lp.add = ca; lp.g2 = w.g2; lp.b2 = w.be2; lp.out = m->x;
     lp.x0 = m->x0c; lp.skip_tok0 = 0; lp.M = M; lp.T = T; lp.d = d; lp.fp16 = fmt;
-    if ((rc = ln_launch(lp, st))) return rc;
-    // person token (row 0): real cross attention over the memory (_mha_block) + norm2 as one cluster kernel
-    // (row0_fused.cu); the four-launch chain it replaced is kept behind MSMD_ROW0_FUSED_MAX_S for A/B runs.
-    static const int row0_max_s = [] { const char* e = getenv("MSMD_ROW0_FUSED_MAX_S"); return e ? atoi(e) : kRow0FusedMaxS; }();
-    if (S <= row0_max_s) {
-      if ((rc = row0_fused_launch(m->x0c, static_cast<const bf16*>(Wq0), w.bq0, kv, static_cast<const bf16*>(Wco), w.bco, w.g2,
-                                  w.be2, m->x, S, T, T - 1, c.n_heads, d, fmt, st)))
-        return rc;
+    if (c.align_mask_width != 1) {
+      // banded cross attention (_mha_block with the alignment mask) of every row, person token included, on every step:
+      // norm1 of all rows, q projection into the qkv workspace (free after self-attention), attention over the cached
+      // K|V, out-proj, then residual + norm2
+      lp.add = nullptr; lp.g2 = nullptr; lp.b2 = nullptr; lp.x0 = nullptr;
+      if ((rc = ln_launch(lp, st))) return rc;
+      if ((rc = gemm(fmt, m->x, d, Wq0, d, w.bq0, nullptr, 0, m->qkv, d, 0, M, d, d, 0, st))) return rc;
+      if ((rc = cross_attn_tc_launch(m->qkv, kv, m->ctx, S, T, T - 1, c.n_heads, c.align_mask_width, fmt, st))) return rc;
+      if ((rc = gemm(fmt, m->ctx, d, Wco, d, w.bco, nullptr, 0, m->y, d, 0, M, d, d, 0, st))) return rc;
+      LnParams l2 = lp;
+      l2.g1 = w.g2; l2.b1 = w.be2;
+      if ((rc = ln_launch(l2, st))) return rc;
     } else {
-      if ((rc = gemm(fmt, m->x0c, d, Wq0, d, w.bq0, nullptr, 0, m->q0, d, 0, S, d, d, 0, st))) return rc;
-      if ((rc = cross_attn_row0_launch(m->q0, kv, m->ctx0, S, T - 1, c.n_heads, fmt, st))) return rc;
-      if ((rc = gemm(fmt, m->ctx0, d, Wco, d, w.bco, nullptr, 0, m->y0, d, 0, S, d, d, 0, st))) return rc;
-      if ((rc = ln_row0_launch(m->y0, m->x0c, w.g2, w.be2, m->x, nullptr, S, T, d, fmt, st))) return rc;
+      if ((rc = ln_launch(lp, st))) return rc;
+      // person token (row 0): real cross attention over the memory (_mha_block) + norm2 as one cluster kernel
+      // (row0_fused.cu); the four-launch chain it replaced is kept behind MSMD_ROW0_FUSED_MAX_S for A/B runs.
+      if (S <= row0_max_s) {
+        if ((rc = row0_fused_launch(m->x0c, static_cast<const bf16*>(Wq0), w.bq0, kv, static_cast<const bf16*>(Wco), w.bco,
+                                    w.g2, w.be2, m->x, S, T, T - 1, c.n_heads, d, fmt, st)))
+          return rc;
+      } else {
+        if ((rc = gemm(fmt, m->x0c, d, Wq0, d, w.bq0, nullptr, 0, m->q0, d, 0, S, d, d, 0, st))) return rc;
+        if ((rc = cross_attn_row0_launch(m->q0, kv, m->ctx0, S, T - 1, c.n_heads, fmt, st))) return rc;
+        if ((rc = gemm(fmt, m->ctx0, d, Wco, d, w.bco, nullptr, 0, m->y0, d, 0, S, d, d, 0, st))) return rc;
+        if ((rc = ln_row0_launch(m->y0, m->x0c, w.g2, w.be2, m->x, nullptr, S, T, d, fmt, st))) return rc;
+      }
     }
     // feed-forward block (_ff_block) + norm3
     if ((rc = gemm(fmt, m->x, d, W1, d, w.b1, nullptr, 0, m->h, c.d_ff, 0, M, c.d_ff, d, 1, st))) return rc;
@@ -281,9 +304,10 @@ int run_forward(msmd_model* m, const float* xrows, cudaStream_t st, int fmt) {
   return MSMD_OK;
 }
 
-// per-window caches of a 16-bit path (fmt 0 bf16 / 1 fp16): memory K|V projection of every layer, then the motion rows'
-// cross-attention output out_proj(v_proj(mem)) (softmax over a single visible key is 1, so the query drops out:
-// SURVEY section 0).  Built on first use in the window: a pure-bf16 call never pays for the fp16 copies.
+// per-window caches of a 16-bit path (fmt 0 bf16 / 1 fp16): memory K|V projection of every layer, then, at
+// align_mask_width 1, the motion rows' cross-attention output out_proj(v_proj(mem)) (softmax over a single visible key
+// is 1, so the query drops out: SURVEY section 0).  Built on first use in the window: a pure-bf16 call never pays for
+// the fp16 copies.
 int window_begin_16(msmd_model* m, int fmt, cudaStream_t st) {
   const msmd_config& c = m->c;
   const int S = m->S, d = c.d_model, Tk = m->T - 1;
@@ -294,7 +318,8 @@ int window_begin_16(msmd_model* m, int fmt, cudaStream_t st) {
     bf16 *kv = fmt ? w.kvh : w.kv, *ca = fmt ? w.cah : w.ca;
     const void *Wkv = fmt ? (const void*)w.Wkv_h : w.Wkv, *Wco = fmt ? (const void*)w.Wco_h : w.Wco;
     if ((rc = gemm(fmt, mem, d, Wkv, d, w.bkv, nullptr, 0, kv, 2 * d, 0, S * Tk, 2 * d, d, 0, st))) return rc;
-    if ((rc = gemm(fmt, kv + d, 2 * d, Wco, d, w.bco, nullptr, 0, ca, d, 0, S * Tk, d, d, 0, st))) return rc;
+    if (c.align_mask_width == 1 && (rc = gemm(fmt, kv + d, 2 * d, Wco, d, w.bco, nullptr, 0, ca, d, 0, S * Tk, d, d, 0, st)))
+      return rc;
   }
   m->window16[fmt] = true;
   return MSMD_OK;
@@ -339,10 +364,8 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
                "(the released configuration is 1 + 10 + 100)", 1 + c.n_prev_motions + c.n_motions);
   MSMD_REQUIRE(c.n_layers > 0 && c.d_ff > 0 && c.d_ff % 8 == 0 && c.max_seqs > 0 && c.n_diff_steps > 0, "msmd_create: bad sizes");
   MSMD_REQUIRE(c.motion_dim > 3 && c.n_basis >= 0 && c.motion_dim + c.n_basis <= 80, "msmd_create: motion_dim + n_basis > 80");
-  if (c.align_mask_width != 1) {
-    set_error("msmd_create: align_mask_width=%d: only width 1 (step-invariant cross attention) is implemented", c.align_mask_width);
-    return MSMD_ERR_UNSUPPORTED;
-  }
+  MSMD_REQUIRE(c.align_mask_width >= 0, "msmd_create: align_mask_width=%d (0 = no alignment mask, w >= 1 = band of 2w-1 "
+               "memory tokens)", c.align_mask_width);
   MSMD_REQUIRE(c.precision >= 0 && c.precision <= 3,
                "msmd_create: precision %d (0 bf16, 1 fp32-grade, 2 hybrid: bf16 + fp16 + fp32-grade, 3 fp16)", c.precision);
   MSMD_CHECK_CUDA(cudaSetDevice(device));
@@ -365,13 +388,15 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
     A(&m->x, M * d); A(&m->qkv, M * 3 * d); A(&m->ctx, M * d); A(&m->h, M * c.d_ff); A(&m->dec1, M * d / 2);
     A(&m->x0c, S * d); A(&m->q0, S * d); A(&m->ctx0, S * d); A(&m->y, M * d); A(&m->y0, S * d);
   }
+  // the step-invariant cross-attention rows (ca / cah / ca32) exist only at align_mask_width 1
+  const bool want_ca = c.align_mask_width == 1;
   if (has_bf16(c)) {
     A(&m->mem, S * (T - 1) * d);
-    for (auto& w : m->L) { A(&w.kv, S * (T - 1) * 2 * d); A(&w.ca, S * (T - 1) * d); }
+    for (auto& w : m->L) { A(&w.kv, S * (T - 1) * 2 * d); if (want_ca) A(&w.ca, S * (T - 1) * d); }
   }
   if (has_fp16(c)) {
     A(&m->memh, S * (T - 1) * d);
-    for (auto& w : m->L) { A(&w.kvh, S * (T - 1) * 2 * d); A(&w.cah, S * (T - 1) * d); }
+    for (auto& w : m->L) { A(&w.kvh, S * (T - 1) * 2 * d); if (want_ca) A(&w.cah, S * (T - 1) * d); }
   }
   if (has_f32(c)) {
     A(&m->fx, M * d); A(&m->fqkv, M * 3 * d); A(&m->fctx, M * d); A(&m->fh, M * c.d_ff); A(&m->fy, M * d);
@@ -380,7 +405,7 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
     // split scratch of the current A operand: the widest is FF2's [M, d_ff] or the window pass's kv cache [S*Tk, 2d]
     const size_t ws = std::max(M * (size_t)c.d_ff, S * (T - 1) * 2 * d);
     A(&m->ws_hi, ws); A(&m->ws_lo, ws); A(&m->overflow, 1);
-    for (auto& w : m->L) { A(&w.kv32, S * (T - 1) * 2 * d); A(&w.ca32, S * (T - 1) * d); }
+    for (auto& w : m->L) { A(&w.kv32, S * (T - 1) * 2 * d); if (want_ca) A(&w.ca32, S * (T - 1) * d); }
   }
   if (!rc && cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking) != cudaSuccess) rc = MSMD_ERR_CUDA;
   if (!rc && m->overflow) {

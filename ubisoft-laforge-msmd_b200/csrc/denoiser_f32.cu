@@ -138,32 +138,38 @@ int ln_row0_f32_launch(const float* y0, const float* r0, const float* g, const f
 }
 
 // ---------------------------------------------------------------------------------------- attention (fp32, SIMT)
-// one CTA per (sequence, head); thread = query row; K and V rows broadcast from shared memory; online softmax
-__global__ void __launch_bounds__(128) self_attn_f32_kernel(const float* __restrict__ qkv, float* __restrict__ ctx, int T,
-                                                            int H) {
-  extern __shared__ float sm[];  // K [T][64], V [T][64]
+// one CTA per (sequence, head); thread = query row; K and V rows broadcast from shared memory; online softmax.
+// q rows s*T.. (row stride ldq), k|v rows s*Tk.. (row stride ldkv, K at column h*64, V at d + h*64).  width 0: every key
+// visible (self-attention); width >= 1: the alignment band of the cross attention (token 0 sees every key, token i >= 1
+// the keys j with |j - (i-1)| <= width-1).
+__global__ void __launch_bounds__(128) attn_f32_kernel(const float* __restrict__ q_src, int ldq, const float* __restrict__ kv,
+                                                       int ldkv, float* __restrict__ ctx, int T, int Tk, int H, int width) {
+  extern __shared__ float sm[];  // K [Tk][64], V [Tk][64]
   const int h = blockIdx.x, s = blockIdx.y, d = H * 64;
   float* sK = sm;
-  float* sV = sm + T * 64;
-  const float* base = qkv + (int64_t)s * T * 3 * d + h * 64;
-  for (int i = threadIdx.x; i < T * 16; i += blockDim.x) {
+  float* sV = sm + Tk * 64;
+  const float* kbase = kv + (int64_t)s * Tk * ldkv + h * 64;
+  for (int i = threadIdx.x; i < Tk * 16; i += blockDim.x) {
     const int r = i >> 4, c4 = i & 15;
-    *reinterpret_cast<float4*>(sK + r * 64 + c4 * 4) = *reinterpret_cast<const float4*>(base + (int64_t)r * 3 * d + d + c4 * 4);
-    *reinterpret_cast<float4*>(sV + r * 64 + c4 * 4) = *reinterpret_cast<const float4*>(base + (int64_t)r * 3 * d + 2 * d + c4 * 4);
+    *reinterpret_cast<float4*>(sK + r * 64 + c4 * 4) = *reinterpret_cast<const float4*>(kbase + (int64_t)r * ldkv + c4 * 4);
+    *reinterpret_cast<float4*>(sV + r * 64 + c4 * 4) = *reinterpret_cast<const float4*>(kbase + (int64_t)r * ldkv + d + c4 * 4);
   }
   __syncthreads();
   const int i = threadIdx.x;
   if (i >= T) return;
+  int j0 = 0, j1 = Tk - 1;
+  if (width > 0 && i > 0) { j0 = max(0, i - width); j1 = min(Tk - 1, i + width - 2); }
+  const float* qrow = q_src + ((int64_t)s * T + i) * ldq + h * 64;
   float q[64], o[64];
 #pragma unroll
   for (int c4 = 0; c4 < 16; ++c4) {
-    const float4 t = *reinterpret_cast<const float4*>(base + (int64_t)i * 3 * d + c4 * 4);
+    const float4 t = *reinterpret_cast<const float4*>(qrow + c4 * 4);
     q[4 * c4] = t.x * 0.125f; q[4 * c4 + 1] = t.y * 0.125f; q[4 * c4 + 2] = t.z * 0.125f; q[4 * c4 + 3] = t.w * 0.125f;
   }
 #pragma unroll
   for (int c = 0; c < 64; ++c) o[c] = 0.f;
   float m = -INFINITY, l = 0.f;
-  for (int j = 0; j < T; ++j) {
+  for (int j = j0; j <= j1; ++j) {
     float sc = 0.f;
 #pragma unroll
     for (int c = 0; c < 64; ++c) sc = fmaf(q[c], sK[j * 64 + c], sc);
@@ -185,18 +191,30 @@ __global__ void __launch_bounds__(128) self_attn_f32_kernel(const float* __restr
   for (int c4 = 0; c4 < 16; ++c4)
     *reinterpret_cast<float4*>(dst + c4 * 4) = make_float4(o[4 * c4] * inv, o[4 * c4 + 1] * inv, o[4 * c4 + 2] * inv, o[4 * c4 + 3] * inv);
 }
-int self_attn_f32_launch(const float* qkv, float* ctx, int S, int T, int H, cudaStream_t st) {
-  const int smem = 2 * T * 64 * (int)sizeof(float);
+namespace {
+int attn_f32_launch(const float* q, int ldq, const float* kv, int ldkv, float* ctx, int S, int T, int Tk, int H, int width,
+                    const char* name, cudaStream_t st) {
   static bool attr = false;
   if (!attr) {
-    MSMD_CHECK_CUDA(cudaFuncSetAttribute(self_attn_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 128 * 64 * 4));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(attn_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 128 * 64 * 4));
     attr = true;
   }
-  MSMD_REQUIRE(T <= 128, "self_attn_f32: T %d > 128", T);
-  ProfileScope prof("self_attn_f32", st);
-  self_attn_f32_kernel<<<dim3(H, S), 128, smem, st>>>(qkv, ctx, T, H);
+  MSMD_REQUIRE(T <= 128 && Tk <= 128, "%s: %d queries / %d keys > 128", name, T, Tk);
+  ProfileScope prof(name, st);
+  attn_f32_kernel<<<dim3(H, S), 128, 2 * Tk * 64 * (int)sizeof(float), st>>>(q, ldq, kv, ldkv, ctx, T, Tk, H, width);
   MSMD_CHECK_LAUNCH();
   return MSMD_OK;
+}
+}  // namespace
+int self_attn_f32_launch(const float* qkv, float* ctx, int S, int T, int H, cudaStream_t st) {
+  const int d = H * 64;
+  return attn_f32_launch(qkv, 3 * d, qkv + d, 3 * d, ctx, S, T, T, H, 0, "self_attn_f32", st);
+}
+int cross_attn_f32_launch(const float* q, const float* kv, float* ctx, int S, int T, int Tk, int H, int width,
+                          cudaStream_t st) {
+  MSMD_REQUIRE(T >= 2 && Tk >= T - 1 && width >= 0, "cross_attn_f32: %d queries / %d keys / width %d", T, Tk, width);
+  const int d = H * 64;
+  return attn_f32_launch(q, d, kv, 2 * d, ctx, S, T, Tk, H, width, "cross_attn_f32", st);
 }
 
 // person-token cross attention, fp32: one warp per (sequence, head); lane = output dims 2*lane, 2*lane+1

@@ -111,6 +111,10 @@ int split_parts_launch(const float* dec, const float* stat, float* dyn, float* s
 
 // tcgen05 self-attention (attn_tc.cu) over T <= 112 tokens, head dim 64: qkv [S*T, 3*d] (q|k|v) -> ctx [S*T, d], 16-bit storage
 int self_attn_tc_launch(const bf16* qkv, bf16* ctx, int S, int T, int H, int fp16, cudaStream_t st);
+// the same kernel in its cross-attention mode: q [S*T, d], kv [S*Tk, 2d] (k|v, the per-window cache) -> ctx [S*T, d] under
+// the alignment band of `width` (token 0 sees every key; token r >= 1 the keys c with |c - (r-1)| <= width-1; 0 = no band)
+int cross_attn_tc_launch(const bf16* q, const bf16* kv, bf16* ctx, int S, int T, int Tk, int H, int width, int fp16,
+                         cudaStream_t st);
 
 // ---- fp32-grade variants (denoiser_f32.cu) ----
 int embed_f32_launch(const EmbedParams& p, float* out, cudaStream_t st);
@@ -119,6 +123,8 @@ int ln_f32_launch(const float* y, const float* resid, const float* g1, const flo
 int ln_row0_f32_launch(const float* y0, const float* r0, const float* g, const float* b, float* out, int S, int T,
                        cudaStream_t st);
 int self_attn_f32_launch(const float* qkv, float* ctx, int S, int T, int H, cudaStream_t st);
+int cross_attn_f32_launch(const float* q, const float* kv, float* ctx, int S, int T, int Tk, int H, int width,
+                          cudaStream_t st);
 int cross_attn_row0_f32_launch(const float* q0, const float* kv, float* ctx0, int S, int Tk, int H, cudaStream_t st);
 int build_memory_f32(const float* prev_audio, const float* audio, float* mem, int S, int Lp, int L, int d, cudaStream_t st);
 int split_tf32(const float* x, float* hi, float* lo, int64_t n, cudaStream_t st);   // gemm_tc.cu

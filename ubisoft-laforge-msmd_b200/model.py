@@ -76,6 +76,23 @@ def _engine_cfg(net, n_diff_steps, target, max_seqs, precision='bf16'):
                 target_noise=int(target == 'noise'), max_seqs=max_seqs, precision=PRECISIONS[precision])
 
 
+def _check_alignment_mask(net):
+    """The engine builds the cross-attention band from ``align_mask_width`` and never reads the bool
+    ``alignment_mask`` buffer (only floating-point entries are packed).  A buffer that disagrees with the width, e.g. one
+    overwritten by a checkpoint loaded with ``strict=True``, would be silently ignored, so it raises instead."""
+    w = net.align_mask_width
+    got = getattr(net, 'alignment_mask', None)
+    if w <= 0:
+        if got is not None:
+            raise _lib.MsmdError(f'alignment_mask is set but align_mask_width={w} means no cross-attention mask')
+        return
+    n = net.n_prev_motions + net.n_motions
+    want = torch.nn.functional.pad(enc_dec_mask(n, n, 1, w - 1, device='cpu'), (0, 0, 1, 0), value=False)
+    if got is None or tuple(got.shape) != tuple(want.shape) or not torch.equal(got.detach().cpu().bool(), want):
+        raise _lib.MsmdError(f'alignment_mask does not match align_mask_width={w}: the engine applies the band of the '
+                             'width, so the module buffer must equal enc_dec_mask(n, n, 1, w-1) with an all-visible row 0')
+
+
 class _EngineOwner:
     """Mixin: lazily creates / grows the CUDA engine and keeps its packed weights in sync with the module.
 
@@ -110,6 +127,7 @@ class _EngineOwner:
         sd = sd_fn()
         key = tuple((k, v.data_ptr(), v._version) for k, v in sd.items())
         if eng.weights_key != key:
+            _check_alignment_mask(getattr(self, 'denoising_net', self))   # MSMD holds the network, which owns the buffer
             eng.load_state_dict(sd)
             eng.weights_key = key
         return eng
