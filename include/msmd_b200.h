@@ -206,6 +206,11 @@ typedef struct {
   int64_t noise_clip_offset; /* in-kernel Philox noise (z == NULL) is keyed by (seed, t, GLOBAL element index): clip n of
                            * this call draws the noise of global clip noise_clip_offset + n, so a clip's codes do not
                            * depend on how the clips are partitioned over calls / GPUs (SURVEY 8(e)). */
+  const int64_t* noise_keys;  /* device [NX][2] or NULL: clip n of this call draws the in-kernel Philox noise of
+                               * (seed = noise_keys[n][0], global clip id = noise_keys[n][1]) instead of
+                               * (seed, noise_clip_offset + n), so one call can mix clips of different windows / seeds.
+                               * Copied into the handle in stream order (the caller may free it when the call returns);
+                               * not allowed together with z. */
 } msmd_sample_extras;
 
 int msmd_sample_window_ex(msmd_model* m, const float* x_T, const float* z, uint64_t seed, int cfg_independent,

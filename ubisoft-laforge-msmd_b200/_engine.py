@@ -16,7 +16,8 @@ class MsmdConfig(C.Structure):
 class SampleExtras(C.Structure):
     _fields_ = [('use_dynamic_threshold', C.c_int), ('dt_ratio', C.c_float), ('dt_min', C.c_float), ('dt_max', C.c_float),
                 ('target_dynamic', C.c_void_p), ('cumulative_static', C.c_void_p), ('alpha_traj', C.c_void_p),
-                ('precise_last_steps', C.c_int), ('fp16_last_steps', C.c_int), ('noise_clip_offset', C.c_int64)]
+                ('precise_last_steps', C.c_int), ('fp16_last_steps', C.c_int), ('noise_clip_offset', C.c_int64),
+                ('noise_keys', C.c_void_p)]
 
 
 PRECISIONS = {'bf16': 0, 'fp32': 1, 'hybrid': 2, 'fp16': 3}
@@ -112,7 +113,9 @@ class DenoiserEngine:
 
     def sample_window(self, x_T, z=None, seed=0, cfg_independent=False, scale0=0.0, scale1=0.0, flexibility=0.0,
                       t_start=None, n_steps=None, want_traj=False, dynamic_threshold=None, separate=False,
-                      precise_last_steps=0, fp16_last_steps=0, noise_clip_offset=0):
+                      precise_last_steps=0, fp16_last_steps=0, noise_clip_offset=0, noise_keys=None):
+        """noise_keys: int64 [N, 2] (seed, global clip id) per clip, keying each clip's in-kernel noise on its own
+        (``seed`` and ``noise_clip_offset`` are then unused).  The library rejects it together with ``z``."""
         c = self.cfg
         x_T = x_T.detach().to(self.device, torch.float32).contiguous()
         t_start = c.n_diff_steps if t_start is None else t_start
@@ -121,12 +124,18 @@ class DenoiserEngine:
             z = z.detach().to(self.device, torch.float32).contiguous()
             if tuple(z.shape) != (c.n_diff_steps + 1,) + tuple(x_T.shape):
                 raise ValueError(f'noise must be [T+1, N, L, d] = {(c.n_diff_steps + 1,) + tuple(x_T.shape)}, got {tuple(z.shape)}')
+        if noise_keys is not None:
+            if noise_keys.dtype != torch.int64 or tuple(noise_keys.shape) != (x_T.shape[0], 2):
+                raise ValueError(f'noise_keys must be int64 [N, 2] = {(x_T.shape[0], 2)}, got {noise_keys.dtype} '
+                                 f'{tuple(noise_keys.shape)}')
+            noise_keys = noise_keys.to(self.device).contiguous()
         out = torch.empty_like(x_T)
         traj = torch.zeros((c.n_diff_steps + 1,) + tuple(x_T.shape), device=self.device) if want_traj else None
         ex = SampleExtras()
         ex.precise_last_steps = int(precise_last_steps)
         ex.fp16_last_steps = int(fp16_last_steps)
         ex.noise_clip_offset = int(noise_clip_offset)
+        ex.noise_keys = _lib.dev_ptr(noise_keys, torch.int64, 'noise_keys').value
         sep = None
         if dynamic_threshold:
             ex.use_dynamic_threshold = 1

@@ -92,6 +92,7 @@ struct msmd_model {
   // window / call of the same shape; the capture stream is created once here.
   UpdateParams* d_up = nullptr;
   unsigned int* d_done = nullptr;   // block-completion counter of the update kernel
+  long long* d_keys = nullptr;      // [max_seqs][2] per-clip Philox keys of the current call (msmd_sample_extras.noise_keys)
   cudaStream_t cap_stream = nullptr;
   typedef std::tuple<int, int, int, int, int, float, float, float> GraphKey;
   std::map<GraphKey, cudaGraphExec_t> graphs;
@@ -383,7 +384,7 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
   A(&m->thr, S);
   A(&m->xbuf, S * c.n_motions * c.motion_dim); A(&m->mixed, S * (T - 1) * c.motion_dim); A(&m->steps, S);
   A(&m->w_audio, S * c.n_motions * d); A(&m->w_prev_audio, S * c.n_prev_motions * d); A(&m->w_ind, S * c.n_motions);
-  A(&m->d_up, 1); A(&m->d_done, 1);
+  A(&m->d_up, 1); A(&m->d_done, 1); A(&m->d_keys, S * 2);
   if (has_bf16(c) || has_fp16(c)) {
     A(&m->x, M * d); A(&m->qkv, M * 3 * d); A(&m->ctx, M * d); A(&m->h, M * c.d_ff); A(&m->dec1, M * d / 2);
     A(&m->x0c, S * d); A(&m->q0, S * d); A(&m->ctx0, S * d); A(&m->y, M * d); A(&m->y0, S * d);
@@ -694,6 +695,8 @@ extern "C" int msmd_sample_window_ex(msmd_model* m, const float* x_T, const floa
   MSMD_REQUIRE(t_start >= 1 && t_start <= c.n_diff_steps && n_steps >= 1 && n_steps <= t_start,
                "msmd_sample_window: steps %d..%d outside 1..%d", t_start, t_start - n_steps + 1, c.n_diff_steps);
   MSMD_REQUIRE(flexibility >= 0.f && flexibility <= 1.f, "msmd_sample_window: flexibility outside [0,1]");
+  MSMD_REQUIRE(!(ex && ex->noise_keys && z),
+               "msmd_sample_window: noise_keys key the in-kernel noise and cannot be combined with an external z");
   int rc;
   if ((rc = poll_overflow(m, "msmd_sample_window"))) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -732,6 +735,12 @@ extern "C" int msmd_sample_window_ex(msmd_model* m, const float* x_T, const floa
     if (use_dt) up.thr = m->thr;
     up.tgt_dyn = ex->target_dynamic; up.cum_static = ex->cumulative_static; up.alpha_traj = ex->alpha_traj;
     up.noise_offset = (long long)ex->noise_clip_offset * c.n_motions * c.motion_dim;
+    if (ex->noise_keys) {
+      // copied into the handle: the step graph reads only engine-owned memory, and the caller may free its keys on return
+      MSMD_CHECK_CUDA(cudaMemcpyAsync(m->d_keys, ex->noise_keys, (size_t)m->NX * 2 * sizeof(int64_t),
+                                      cudaMemcpyDeviceToDevice, st));
+      up.noise_keys = m->d_keys;
+    }
     if (up.cum_static) MSMD_CHECK_CUDA(cudaMemsetAsync(up.cum_static, 0, n_el * 4, st));
   }
   if ((rc = update_params_set(m->d_up, up, st))) return rc;

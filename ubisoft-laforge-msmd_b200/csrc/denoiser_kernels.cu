@@ -764,10 +764,11 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
   // alias the shared-memory parameter block, so every p.field in the loop was re-read after each store
   struct Loc {
     const float *dec, *stat, *z, *thr; float *x, *traj, *tgt_dyn, *cum_static, *alpha_traj; const int* overflow;
+    const long long* keys;
     float scale0, scale1; unsigned long long seed; long long noise_offset;
     int NX, E, T, L, Lp, dm, nb, ldd, cfg_independent, target_noise, t_start;
   };
-  const Loc q = {p.dec, p.stat, p.z, p.thr, p.x, p.traj, p.tgt_dyn, p.cum_static, p.alpha_traj, p.overflow,
+  const Loc q = {p.dec, p.stat, p.z, p.thr, p.x, p.traj, p.tgt_dyn, p.cum_static, p.alpha_traj, p.overflow, p.noise_keys,
                  p.scale0, p.scale1, p.seed, p.noise_offset,
                  p.NX, p.E, p.T, p.L, p.Lp, p.dm, p.nb, p.ldd, p.cfg_independent, p.target_noise, p.t_start};
   const bool sep = q.tgt_dyn != nullptr || q.cum_static != nullptr;
@@ -789,6 +790,14 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
       thv[e] = q.thr ? q.thr[sq] : 0.f;
 #pragma unroll
       for (int b = 0; b < 4; ++b) al[e][b] = b < q.nb ? rowp[e][q.dm + b] : 0.f;
+    }
+    // Philox key of the row: element index (global clip id * L + l) * dm + c under the clip's seed.  Without per-clip keys
+    // the global clip id is noise_clip_offset + n, i.e. the index is i + noise_offset (32-bit wrap-around either way)
+    unsigned long long nseed = q.seed;
+    long long nbase = (long long)row * q.dm + q.noise_offset;
+    if (q.keys != nullptr) {
+      nseed = (unsigned long long)q.keys[2 * n];
+      nbase = (long long)l * q.dm + q.keys[2 * n + 1] * q.L * q.dm;
     }
    for (int c = lane; c < q.dm; c += 32) {
     const int64_t i = (int64_t)row * q.dm + c;
@@ -823,7 +832,7 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
       prev = r; pd = dyn; psv = sta;
     }
     float zt = 0.f;
-    if (t > 1) zt = q.z ? q.z[(int64_t)t * n_el + i] : philox_normal(q.seed, (uint32_t)t, (uint32_t)(i + q.noise_offset));
+    if (t > 1) zt = q.z ? q.z[(int64_t)t * n_el + i] : philox_normal(nseed, (uint32_t)t, (uint32_t)(nbase + c));
     const float xo = q.x[i];
     float xn = q.target_noise ? (c0 * (xo - c1 * tgt) + sigma * zt) : (c0 * xo + c1 * tgt + sigma * zt);
     // fp32-grade steps: an activation left the fp16 range of the operand split -> poison the state instead of

@@ -88,6 +88,7 @@ struct UpdateParams {
   int S;
   long long noise_offset; // added to the element index that keys the in-kernel Philox noise (= global clip id * L * dm)
   const int* overflow;    // fp32-grade steps: device flag raised by the operand split; non-zero poisons x with NaN
+  const long long* noise_keys;  // [NX][2] (seed, global clip id) per clip, or null (-> seed, noise_offset); engine-owned
 };
 // per-sequence threshold s = clamp(quantile(|x0_hat[:, -L:]|, ratio), lo, hi) -> thr[S] (torch.quantile 'linear')
 int threshold_launch(const float* dec, const float* stat, float* thr, int S, int T, int L, int Lp, int dm, int nb, int ldd,

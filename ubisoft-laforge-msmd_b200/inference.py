@@ -7,6 +7,10 @@ of ``n_motions`` frames are sampled sequentially, each conditioned on the previo
 
 ``infer_coeffs_batched`` is the same loop over a batch of independent clips (the reference handles one
 clip per call; clips never interact, so they are simply stacked along the batch dimension).
+
+``infer_coeffs_queue`` / ``infer_coeffs_many`` sample clips of different lengths with a clip queue: every sampler call
+keeps up to ``max_clips`` clips in flight, whatever window each of them is on, and each clip's step noise is keyed by
+its own (seed + window, global clip id).
 """
 import math
 
@@ -52,24 +56,175 @@ def infer_coeffs_batched(model, args, audio_feat, shape_coef, style_feats=None, 
     return torch.cat(coef_list, dim=1)
 
 
+def plan_clip(n_samples, args, audio_unit):
+    """Windowing of one clip of ``n_samples`` 16 kHz samples (inference.py:39-45): (n_subdivision, samples after zero
+    padding, clip_len = frames kept).  The clip is padded up to n_subdivision windows of audio, never truncated."""
+    clip_len = int(n_samples / 16000 * args.fps)
+    n_audio_samples = round(audio_unit * args.n_motions)
+    n_subdivision = 1 if clip_len <= args.n_motions else math.ceil(clip_len / args.n_motions)
+    n_padding_audio_samples = n_audio_samples * n_subdivision - n_samples
+    n_padding_frames = math.ceil(n_padding_audio_samples / audio_unit)
+    padded = n_samples + max(n_padding_audio_samples, 0)
+    return n_subdivision, padded, args.n_motions * n_subdivision - max(n_padding_frames, 0)
+
+
 @torch.no_grad()
 def infer_coeffs(model, args, audio, shape_coef, audio_unit, style_feats=None, n_repetitions: int = 1, cfg_mode=None,
                  cfg_cond=None, cfg_scale: float = 1.15, include_shape: bool = False, dynamic_threshold=(0, 1, 4)):
     """inference.py:34-75 (one clip, 1-D 16 kHz audio)."""
-    clip_len = int(len(audio) / 16000 * args.fps)
-    n_audio_samples = round(audio_unit * args.n_motions)
-    n_subdivision = 1 if clip_len <= args.n_motions else math.ceil(clip_len / args.n_motions)
-    n_padding_audio_samples = n_audio_samples * n_subdivision - len(audio)
-    n_padding_frames = math.ceil(n_padding_audio_samples / audio_unit)
-    if n_padding_audio_samples > 0:
-        audio = F.pad(audio, (0, n_padding_audio_samples), value=0)
+    n_subdivision, padded, clip_len = plan_clip(len(audio), args, audio_unit)
+    if padded > len(audio):
+        audio = F.pad(audio, (0, padded - len(audio)), value=0)
     audio_feat = model.extract_audio_feature(audio.unsqueeze(0), args.n_motions * n_subdivision)
-    total = args.n_motions * n_subdivision
     rep = lambda t: t if t is None else t.expand(n_repetitions, *t.shape[1:])
     style = [rep(s) for s in style_feats] if isinstance(style_feats, list) else rep(style_feats)
     return infer_coeffs_batched(model, args, audio_feat.expand(n_repetitions, -1, -1), rep(shape_coef), style,
-                                clip_len=total - max(n_padding_frames, 0), cfg_mode=cfg_mode, cfg_cond=cfg_cond,
+                                clip_len=clip_len, cfg_mode=cfg_mode, cfg_cond=cfg_cond,
                                 cfg_scale=cfg_scale, dynamic_threshold=dynamic_threshold)
+
+
+def queue_schedule(n_windows, max_clips):
+    """Sampler calls of the clip queue: a list of calls, each a list of (clip, window) in slot order.  At most
+    ``max_clips`` clips are in flight; clips are admitted in order; a clip that has run its last window hands its
+    slot to the next queued clip at the next window boundary (slots left without a clip close up)."""
+    if max_clips < 1:
+        raise ValueError(f'max_clips must be >= 1, got {max_clips}')
+    if any(n < 1 for n in n_windows):
+        raise ValueError('every clip needs at least one window')
+    slots, calls, nxt = [], [], 0
+    while nxt < len(n_windows) and len(slots) < max_clips:
+        slots.append([nxt, 0])
+        nxt += 1
+    while slots:
+        calls.append([(k, w) for k, w in slots])
+        kept = []
+        for k, w in slots:
+            if w + 1 < n_windows[k]:
+                kept.append([k, w + 1])
+            elif nxt < len(n_windows):
+                kept.append([nxt, 0])
+                nxt += 1
+        slots = kept
+    return calls
+
+
+@torch.no_grad()
+def infer_coeffs_queue(model, args, audio_feats, shape_coefs, style_feats, clip_lens, x_T, max_clips=64, clip_ids=None,
+                       noise_seed=0, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, dynamic_threshold=None):
+    """``infer_coeffs_batched`` over clips of different lengths, keeping up to ``max_clips`` clips in every sampler call.
+
+    Per clip k: audio_feats[k] [n_sub_k * n_motions, d] (already extracted), shape_coefs[k] [100] / [1, 100],
+    style_feats[k] [d_style] (or style_feats None), clip_lens[k] frames to keep, x_T[k] [n_motions, 67] (re-used by every
+    window, like infer_coeffs_batched).  One call mixes clips that are on different windows (queue_schedule); the step
+    noise of clip k's window w is keyed by (noise_seed + w, clip_ids[k]) (default clip_ids: 0..K-1), so clip k's codes
+    are those of infer_coeffs_batched on that clip alone with noise_seed and clip_offset = clip_ids[k].
+    The schedule depends on the lengths only: nothing is read back from the device between windows.
+    Returns (codes [K, max_k clip_lens[k], 67], zero beyond each clip's length; lengths [K] int64)."""
+    K = len(audio_feats)
+    if K == 0:
+        raise ValueError('infer_coeffs_queue: no clips')
+    clip_ids = list(range(K)) if clip_ids is None else [int(i) for i in clip_ids]
+    others = dict(shape_coefs=shape_coefs, clip_lens=clip_lens, x_T=x_T, clip_ids=clip_ids)
+    if style_feats is not None:
+        others['style_feats'] = style_feats
+    bad = {k: len(v) for k, v in others.items() if len(v) != K}
+    if bad:
+        raise ValueError(f'infer_coeffs_queue: {K} audio feature tensors but {bad}')
+    L, Lp = args.n_motions, args.n_prev_motions
+    n_sub = []
+    for k, (f, n) in enumerate(zip(audio_feats, clip_lens)):
+        if f.ndim != 2 or f.shape[0] % L or f.shape[0] == 0:
+            raise ValueError(f'clip {k}: audio features must be [n_sub * {L}, d], got {tuple(f.shape)}')
+        if not (f.shape[0] - L <= int(n) <= f.shape[0]):
+            raise ValueError(f'clip {k}: clip_len {int(n)} outside its last window ({f.shape[0] - L}, {f.shape[0]}]')
+        n_sub.append(f.shape[0] // L)
+    calls = queue_schedule(n_sub, max_clips)
+    dev = model.device
+    W = max(n_sub)
+    # the small per-clip inputs are stacked once and each call gathers its rows with index tensors planned (and uploaded)
+    # up front; the audio features stay in the caller's per-clip tensors (a dense [K, W*L, d] copy would grow with
+    # K x the longest clip) and each call stacks its windows' slices (views) with one copy
+    feats = [f.to(dev) for f in audio_feats]
+    start_audio = model.start_audio_feat.detach()[0]
+    shape = torch.stack([s.reshape(1, -1) for s in shape_coefs]).to(dev)
+    style = None if style_feats is None else torch.stack([s.reshape(-1) for s in style_feats]).to(dev)
+    xT = torch.stack([x.reshape(L, -1) for x in x_T]).to(dev)
+    prev_motion = model.start_motion_feat.detach().expand(K, -1, -1).clone()
+    codes = torch.zeros((K, W * L, xT.shape[-1]), device=dev)
+    plan = []                                    # per call: clip, window, valid frames, seed, global clip id
+    for call in calls:
+        for k, w in call:
+            valid = int(clip_lens[k]) - w * L if w == n_sub[k] - 1 else L
+            plan.append((k, w, valid, int(noise_seed) + w, clip_ids[k]))
+    plan = torch.tensor(plan, dtype=torch.int64)
+    plan = (plan.pin_memory() if dev.type == 'cuda' else plan).to(dev, non_blocking=True)
+    frames = torch.arange(L, device=dev)
+    pos = 0
+    for call in calls:
+        n = len(call)
+        p = plan[pos:pos + n]
+        pos += n
+        idx, win = p[:, 0], p[:, 1]
+        rows = win[:, None] * L + frames                                  # [n, L] frames of this window
+        audio_in = torch.stack([feats[k][w * L:(w + 1) * L] for k, w in call])
+        # window w > 0 is conditioned on the last Lp INPUT frames of window w - 1, window 0 on the learnt start rows
+        prev_audio = torch.stack([feats[k][w * L - Lp:w * L] if w > 0 else start_audio for k, w in call])
+        indicator = (frames < p[:, 2:3]).float() if args.use_indicator else None
+        out, _, _ = model.sample(audio_in, shape[idx], None if style is None else style[idx], prev_motion[idx], prev_audio,
+                                 xT[idx], indicator=indicator, cfg_mode=cfg_mode, cfg_cond=cfg_cond, cfg_scale=cfg_scale,
+                                 dynamic_threshold=dynamic_threshold, noise_keys=p[:, 3:5].contiguous())
+        prev_motion[idx] = out[:, -Lp:]
+        codes[idx[:, None], rows] = out
+    lengths = torch.tensor([int(n) for n in clip_lens], dtype=torch.int64)
+    T_max = int(lengths.max())
+    codes = codes[:, :T_max]
+    keep = torch.arange(T_max, device=dev)[None, :] < lengths.to(dev)[:, None]
+    return torch.where(keep[..., None], codes, torch.zeros((), device=dev)), lengths
+
+
+# audio encoder batch of infer_coeffs_many: 64 clips x 10 s, the encoder batch of the configs[2] benchmark
+AUDIO_BATCH_SAMPLES = 64 * 160000
+
+
+@torch.no_grad()
+def extract_clip_features(model, args, audios, audio_unit=640.0):
+    """Audio features of many 1-D 16 kHz clips, each planned and zero-padded exactly as infer_coeffs does (plan_clip).
+    The encoder runs once per group of clips with the same padded length, in batches of one clip count for every group,
+    chosen so that clips x the longest padded clip stays within AUDIO_BATCH_SAMPLES: the encoder's workspace grows to
+    (largest batch seen) x (longest clip seen), so a per-group count (many short clips, few long ones) would size it
+    for the product of both maxima.  Returns (features: list of [n_sub_k * n_motions, d], clip_lens: list of frames to keep)."""
+    plans = [plan_clip(len(a), args, audio_unit) for a in audios]
+    groups = {}
+    for k, (n_sub, padded, _) in enumerate(plans):
+        groups.setdefault((n_sub, padded), []).append(k)
+    feats = [None] * len(audios)
+    step = max(1, AUDIO_BATCH_SAMPLES // max((p[1] for p in plans), default=1))
+    for (n_sub, padded), ks in groups.items():
+        for a in range(0, len(ks), step):
+            chunk = ks[a:a + step]
+            wav = torch.stack([F.pad(audios[k], (0, padded - len(audios[k])), value=0) for k in chunk])
+            f = model.extract_audio_feature(wav, args.n_motions * n_sub)
+            for j, k in enumerate(chunk):
+                feats[k] = f[j]
+    return feats, [p[2] for p in plans]
+
+
+@torch.no_grad()
+def infer_coeffs_many(model, args, audios, shape_coefs, style_feats, audio_unit=640.0, **queue_kwargs):
+    """``infer_coeffs`` for many 1-D 16 kHz clips of any lengths: features from extract_clip_features, then
+    infer_coeffs_queue.  queue_kwargs: x_T ([K, n_motions, 67] or a list; default drawn from torch's generator),
+    max_clips, clip_ids, noise_seed, cfg_mode, cfg_cond, cfg_scale, dynamic_threshold (default (0, 1, 4), infer_coeffs's
+    default; None turns dynamic thresholding off).
+    Returns (codes [K, max clip_len, 67], zero beyond each clip's length; lengths [K])."""
+    K = len(audios)
+    if K == 0:
+        raise ValueError('infer_coeffs_many: no clips')
+    feats, clip_lens = extract_clip_features(model, args, audios, audio_unit)
+    queue_kwargs.setdefault('dynamic_threshold', (0, 1, 4))
+    x_T = queue_kwargs.pop('x_T', None)
+    if x_T is None:       # drawn on the CPU like MSMD.sample's default x_T (model.py:337)
+        x_T = torch.randn((K, args.n_motions, 67)).to(model.device)
+    return infer_coeffs_queue(model, args, feats, shape_coefs, style_feats, clip_lens, x_T, **queue_kwargs)
 
 
 def load_model(model_root: str, model_name: str, iter_num: str, device='cuda'):

@@ -327,7 +327,7 @@ class MSMD(nn.Module, _EngineOwner):
     def sample(self, audio_or_feat, shape_feat, style_feat=None, prev_motion_feat=None, prev_audio_feat=None,
                motion_at_T=None, indicator=None, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, flexibility=0,
                dynamic_threshold=None, ret_traj=False, noise=None, n_steps=None, t_start=None, _separate=False,
-               precise_last_steps=None, fp16_last_steps=None, noise_seed=None, clip_offset=0):
+               precise_last_steps=None, fp16_last_steps=None, noise_seed=None, clip_offset=0, noise_keys=None):
         """model.py:282-440.  Extra keyword arguments (not in the reference): ``noise`` = externally supplied
         z tensor [T+1, N, L, 67] indexed by step t (default: in-kernel Philox seeded from torch's generator);
         ``t_start`` / ``n_steps`` = start at step t_start (motion_at_T is then x_{t_start}) and run n steps
@@ -336,8 +336,16 @@ class MSMD(nn.Module, _EngineOwner):
         fp16 arithmetic (defaults: the attributes of the same names, 'auto'); ``noise_seed`` / ``clip_offset`` = key of the
         in-kernel Philox step noise (used when ``noise`` is None): clip n draws the stream of global clip clip_offset + n
         under ``noise_seed`` (default: a seed drawn from torch's generator), so clip-sharded runs reproduce the
-        single-GPU codes (SURVEY 8(e))."""
+        single-GPU codes (SURVEY 8(e)); ``noise_keys`` = int64 [N, 2] of (seed, global clip id) per clip, instead of
+        ``noise_seed`` / ``clip_offset``, so one call can carry clips of different windows (inference.infer_coeffs_queue)."""
         N = audio_or_feat.shape[0]
+        if noise_keys is not None:
+            if not isinstance(noise_keys, torch.Tensor) or noise_keys.dtype != torch.int64 or \
+                    tuple(noise_keys.shape) != (N, 2):
+                raise ValueError(f'noise_keys must be an int64 tensor [N, 2] = [{N}, 2], got '
+                                 f'{getattr(noise_keys, "dtype", type(noise_keys))} {tuple(getattr(noise_keys, "shape", ()))}')
+            if noise is not None or noise_seed is not None or clip_offset != 0:
+                raise ValueError('noise_keys replace noise_seed / clip_offset and exclude an external noise tensor')
         dev = self.device
         cfg_mode = self.cfg_mode if cfg_mode is None else cfg_mode
         cfg_cond = self.guiding_conditions if cfg_cond is None else cfg_cond
@@ -397,7 +405,7 @@ class MSMD(nn.Module, _EngineOwner):
         eng.window_begin(torch.cat(audio_in, 0), torch.cat(person_in, 0).reshape(N * E, -1),
                          rep(style_feat).reshape(N * E, -1), rep(prev_motion_feat), rep(prev_audio_feat),
                          rep(indicator) if indicator is not None else None, NX=N, E=E)
-        if noise is not None:
+        if noise is not None or noise_keys is not None:
             seed = 0
         elif noise_seed is not None:
             seed = int(noise_seed)
@@ -410,7 +418,8 @@ class MSMD(nn.Module, _EngineOwner):
                                 t_start=T, n_steps=n_steps, want_traj=ret_traj, dynamic_threshold=dynamic_threshold,
                                 separate=_separate,
                                 precise_last_steps=self._precise_steps(precise_last_steps),
-                                fp16_last_steps=self._fp16_steps(fp16_last_steps), noise_clip_offset=clip_offset)
+                                fp16_last_steps=self._fp16_steps(fp16_last_steps), noise_clip_offset=clip_offset,
+                                noise_keys=noise_keys)
         x0, traj = res[0], res[1]
         if _separate and not ret_traj:
             return x0, motion_at_T, audio_feat, res[2]
