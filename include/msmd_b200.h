@@ -217,6 +217,30 @@ int msmd_sample_window_ex(msmd_model* m, const float* x_T, const float* z, uint6
                           float scale0, float scale1, float flexibility, int t_start, int n_steps,
                           float* x_out, float* traj, const msmd_sample_extras* extras, void* stream);
 
+/* Respaced (DDIM) schedule of the sampling loop: the strictly decreasing HOST list of visited timesteps
+ * t_1 > ... > t_K in [1, n_diff_steps], and eta in [0, 1].  With s the successor of t in the list (0 after the last
+ * entry), A = alpha_bars[t], B = alpha_bars[s] (alpha_bars[0] = 1) and
+ *   sigma = eta sqrt((1 - B) / (1 - A)) sqrt(1 - A / B),  r = sqrt(max(0, 1 - B - sigma^2)),
+ * a step is x_s = k x_t + (sqrt(B) - sqrt(A) k) x0_hat + sigma z_t with k = r / sqrt(1 - A)       (target 'sample')
+ *        or x_s = sqrt(B / A) x_t + (r - sqrt(B) sqrt(1 - A) / sqrt(A)) eps_hat + sigma z_t           (target 'noise').
+ * z_t is the noise of step t of the default loop (z[t], or the in-kernel Philox stream keyed by t) and is drawn only
+ * when s > 0.  The list is read on the host during the call and may be freed on return. */
+typedef struct {
+  const int32_t* timesteps;
+  int n_timesteps;
+  float eta;
+} msmd_sample_schedule;
+
+/* msmd_sample_window_ex on a respaced schedule (sched = NULL: the default loop t = t_start .. t_start - n_steps + 1).
+ * t_start must be an entry of the list and n_steps counts list entries from there.  flexibility must be 0.  traj
+ * receives x_s at index s; extras->alpha_traj row i is the i-th executed step; extras->cumulative_static sums the
+ * output coefficient times the static part.  The hybrid precision schedule keeps its meaning in t: visited steps with
+ * t <= precise_last_steps run fp32-grade, t <= fp16_last_steps fp16.  Step graphs are shared with the default loop. */
+int msmd_sample_window_sched(msmd_model* m, const float* x_T, const float* z, uint64_t seed, int cfg_independent,
+                             float scale0, float scale1, float flexibility, int t_start, int n_steps,
+                             float* x_out, float* traj, const msmd_sample_extras* extras,
+                             const msmd_sample_schedule* sched, void* stream);
+
 /* Synchronise `stream` and report a pending fp32-grade operand-split overflow of an earlier call on this handle. */
 int msmd_check(msmd_model* m, void* stream);
 

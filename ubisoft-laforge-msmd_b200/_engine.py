@@ -20,6 +20,11 @@ class SampleExtras(C.Structure):
                 ('noise_keys', C.c_void_p)]
 
 
+class SampleSchedule(C.Structure):
+    """msmd_sample_schedule: a HOST int32 list of visited timesteps (strictly decreasing) and eta."""
+    _fields_ = [('timesteps', C.POINTER(C.c_int32)), ('n_timesteps', C.c_int), ('eta', C.c_float)]
+
+
 PRECISIONS = {'bf16': 0, 'fp32': 1, 'hybrid': 2, 'fp16': 3}
 PATHS = {'bf16': 0, 'fp32': 1, 'fp16': 2}          # msmd_denoise_ex's `precise` argument
 
@@ -113,11 +118,23 @@ class DenoiserEngine:
 
     def sample_window(self, x_T, z=None, seed=0, cfg_independent=False, scale0=0.0, scale1=0.0, flexibility=0.0,
                       t_start=None, n_steps=None, want_traj=False, dynamic_threshold=None, separate=False,
-                      precise_last_steps=0, fp16_last_steps=0, noise_clip_offset=0, noise_keys=None):
+                      precise_last_steps=0, fp16_last_steps=0, noise_clip_offset=0, noise_keys=None, timesteps=None,
+                      eta=0.0):
         """noise_keys: int64 [N, 2] (seed, global clip id) per clip, keying each clip's in-kernel noise on its own
-        (``seed`` and ``noise_clip_offset`` are then unused).  The library rejects it together with ``z``."""
+        (``seed`` and ``noise_clip_offset`` are then unused).  The library rejects it together with ``z``.
+        timesteps: strictly decreasing visited steps of a respaced (DDIM) schedule with ``eta`` in [0, 1], or None for
+        the default loop t_start, t_start - 1, ...  On a schedule t_start defaults to its first entry and n_steps to the
+        entries from t_start on; ``traj`` then holds x_s at each visited successor s."""
         c = self.cfg
         x_T = x_T.detach().to(self.device, torch.float32).contiguous()
+        sched = ts = None
+        if timesteps is not None:
+            ts = (C.c_int32 * len(timesteps))(*[int(t) for t in timesteps])
+            sched = SampleSchedule(ts, len(timesteps), float(eta))
+            t_start = int(timesteps[0]) if t_start is None else t_start
+            if n_steps is None:
+                later = [i for i, t in enumerate(timesteps) if int(t) == t_start]
+                n_steps = len(timesteps) - later[0] if later else 1   # t_start off the list: the library rejects it
         t_start = c.n_diff_steps if t_start is None else t_start
         n_steps = t_start if n_steps is None else n_steps
         if z is not None:
@@ -145,11 +162,11 @@ class DenoiserEngine:
                    torch.empty((n_steps,) + tuple(x_T.shape[:2]) + (c.n_basis,), device=self.device))
             ex.target_dynamic, ex.cumulative_static, ex.alpha_traj = [t.data_ptr() for t in sep]
         with torch.cuda.device(self.device):
-            _lib.check(_lib.lib().msmd_sample_window_ex(self._h, _lib.dev_ptr(x_T), _lib.dev_ptr(z), C.c_uint64(seed),
-                                                        int(cfg_independent), float(scale0), float(scale1),
-                                                        float(flexibility), int(t_start), int(n_steps),
-                                                        _lib.dev_ptr(out), _lib.dev_ptr(traj), C.byref(ex),
-                                                        _lib.stream_ptr()))
+            _lib.check(_lib.lib().msmd_sample_window_sched(self._h, _lib.dev_ptr(x_T), _lib.dev_ptr(z), C.c_uint64(seed),
+                                                           int(cfg_independent), float(scale0), float(scale1),
+                                                           float(flexibility), int(t_start), int(n_steps),
+                                                           _lib.dev_ptr(out), _lib.dev_ptr(traj), C.byref(ex),
+                                                           None if sched is None else C.byref(sched), _lib.stream_ptr()))
         return (out, traj, sep) if separate else (out, traj)
 
     def __del__(self):

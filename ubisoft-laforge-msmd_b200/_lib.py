@@ -46,6 +46,8 @@ SIGNATURES = {
     'msmd_audio_normalize': (_i, [_vp, _vp, _i, _i64, _vp]),
     'msmd_resample_linear': (_i, [_vp, _vp, _i, _i, _i, _vp]),
     'msmd_sample_window_ex': (_i, [_vp, _vp, _vp, C.c_uint64, _i, C.c_float, C.c_float, C.c_float, _i, _i, _vp, _vp, _vp, _vp]),
+    'msmd_sample_window_sched': (_i, [_vp, _vp, _vp, C.c_uint64, _i, C.c_float, C.c_float, C.c_float, _i, _i, _vp, _vp, _vp,
+                                      _vp, _vp]),
     'msmd_flame_create': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, C.POINTER(_vp)]),
     'msmd_flame_decode': (_i, [_vp, _vp, _vp, _i, _i64, _vp, _vp, _i, _vp]),
     'msmd_flame_destroy': (None, [_vp]),

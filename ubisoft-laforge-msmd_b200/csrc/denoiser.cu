@@ -13,6 +13,8 @@
 #include "gemm_tc.cuh"
 #include "profile.cuh"
 #include <cuda_fp16.h>
+#include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <map>
@@ -93,6 +95,8 @@ struct msmd_model {
   UpdateParams* d_up = nullptr;
   unsigned int* d_done = nullptr;   // block-completion counter of the update kernel
   long long* d_keys = nullptr;      // [max_seqs][2] per-clip Philox keys of the current call (msmd_sample_extras.noise_keys)
+  SchedStep* d_sched = nullptr;     // [n_diff_steps + 1] respaced-step table of the current call, indexed by t
+  std::vector<double> h_alpha_bars; // host copy of diffusion_sched.alpha_bars: the respaced coefficients are planned on the host
   cudaStream_t cap_stream = nullptr;
   typedef std::tuple<int, int, int, int, int, float, float, float> GraphKey;
   std::map<GraphKey, cudaGraphExec_t> graphs;
@@ -384,7 +388,7 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
   A(&m->thr, S);
   A(&m->xbuf, S * c.n_motions * c.motion_dim); A(&m->mixed, S * (T - 1) * c.motion_dim); A(&m->steps, S);
   A(&m->w_audio, S * c.n_motions * d); A(&m->w_prev_audio, S * c.n_prev_motions * d); A(&m->w_ind, S * c.n_motions);
-  A(&m->d_up, 1); A(&m->d_done, 1); A(&m->d_keys, S * 2);
+  A(&m->d_up, 1); A(&m->d_done, 1); A(&m->d_keys, S * 2); A(&m->d_sched, (size_t)c.n_diff_steps + 1);
   if (has_bf16(c) || has_fp16(c)) {
     A(&m->x, M * d); A(&m->qkv, M * 3 * d); A(&m->ctx, M * d); A(&m->h, M * c.d_ff); A(&m->dec1, M * d / 2);
     A(&m->x0c, S * d); A(&m->q0, S * d); A(&m->ctx0, S * d); A(&m->y, M * d); A(&m->y0, S * d);
@@ -554,7 +558,10 @@ extern "C" int msmd_load_weights(msmd_model* m, const char* const* names, const 
   F32(P + "diff_step_map.2.weight", d * d, &w2); F32(P + "diff_step_map.2.bias", d, &b2);
   // schedule (model.py:20-71): copied, not recomputed (SURVEY 8(a) a6)
   F32("diffusion_sched.alphas", nt, &m->alphas);
-  F32("diffusion_sched.alpha_bars", nt, &m->alpha_bars);
+  if (!rc && fetch("diffusion_sched.alpha_bars", nt, h)) {
+    rc = up_f32(m, &m->alpha_bars, h);
+    m->h_alpha_bars.assign(h.begin(), h.end());
+  }
   F32("diffusion_sched.sigmas_flex", nt, &m->sig_flex);
   F32("diffusion_sched.sigmas_inflex", nt, &m->sig_inflex);
   if (rc) return rc;
@@ -689,12 +696,72 @@ extern "C" int msmd_sample_window(msmd_model* m, const float* x_T, const float* 
 extern "C" int msmd_sample_window_ex(msmd_model* m, const float* x_T, const float* z, uint64_t seed, int cfg_independent,
                                      float scale0, float scale1, float flexibility, int t_start, int n_steps,
                                      float* x_out, float* traj, const msmd_sample_extras* ex, void* stream) {
+  return msmd_sample_window_sched(m, x_T, z, seed, cfg_independent, scale0, scale1, flexibility, t_start, n_steps, x_out,
+                                  traj, ex, nullptr, stream);
+}
+
+namespace {
+// The visited steps of a respaced call (t_start and the n_steps list entries from it) and their update coefficients,
+// planned in double from the loaded alpha_bars (include/msmd_b200.h, msmd_sample_schedule)
+int plan_respaced(const msmd_model* m, const msmd_sample_schedule& sc, float flexibility, int t_start, int n_steps,
+                  std::vector<SchedStep>& out) {
+  const msmd_config& c = m->c;
+  MSMD_REQUIRE(sc.timesteps && sc.n_timesteps >= 1, "msmd_sample_window: empty timestep list");
+  MSMD_REQUIRE(sc.eta >= 0.f && sc.eta <= 1.f, "msmd_sample_window: eta %g outside [0, 1]", (double)sc.eta);
+  MSMD_REQUIRE(flexibility == 0.f, "msmd_sample_window: flexibility %g has no meaning on a respaced schedule (must be 0)",
+               (double)flexibility);
+  const int K = sc.n_timesteps;
+  const int32_t* ts = sc.timesteps;
+  int pos = -1;
+  for (int i = 0; i < K; ++i) {
+    MSMD_REQUIRE(ts[i] >= 1 && ts[i] <= c.n_diff_steps, "msmd_sample_window: timesteps[%d] = %d outside [1, %d]", i, ts[i],
+                 c.n_diff_steps);
+    MSMD_REQUIRE(i == 0 || ts[i] < ts[i - 1], "msmd_sample_window: timesteps not strictly decreasing at index %d (%d after %d)",
+                 i, ts[i], i ? ts[i - 1] : 0);
+    if (ts[i] == t_start) pos = i;
+  }
+  MSMD_REQUIRE(pos >= 0, "msmd_sample_window: t_start %d is not an entry of the timestep list", t_start);
+  MSMD_REQUIRE(n_steps >= 1 && pos + n_steps <= K, "msmd_sample_window: n_steps %d outside [1, %d] list entries from t_start %d",
+               n_steps, K - pos, t_start);
+  const std::vector<double>& ab = m->h_alpha_bars;
+  const double eta = sc.eta;
+  out.resize(n_steps);
+  for (int i = 0; i < n_steps; ++i) {
+    const int t = ts[pos + i], s = pos + i + 1 < K ? ts[pos + i + 1] : 0;
+    const double A = ab[t], B = s > 0 ? ab[s] : 1.0;
+    MSMD_REQUIRE(A < 1.0 && A > 0.0, "msmd_sample_window: alpha_bars[%d] = %g outside (0, 1)", t, A);
+    const double sigma = eta * std::sqrt((1.0 - B) / (1.0 - A)) * std::sqrt(std::max(0.0, 1.0 - A / B));
+    const double r = std::sqrt(std::max(0.0, 1.0 - B - sigma * sigma));
+    double c0, c1;
+    if (c.target_noise) {
+      c0 = std::sqrt(B / A);
+      c1 = r - std::sqrt(B) * std::sqrt(1.0 - A) / std::sqrt(A);
+    } else {
+      c0 = r / std::sqrt(1.0 - A);
+      c1 = std::sqrt(B) - std::sqrt(A) * c0;
+    }
+    out[i] = SchedStep{(float)c0, (float)c1, (float)sigma, t, s, i};
+  }
+  return MSMD_OK;
+}
+}  // namespace
+
+extern "C" int msmd_sample_window_sched(msmd_model* m, const float* x_T, const float* z, uint64_t seed, int cfg_independent,
+                                        float scale0, float scale1, float flexibility, int t_start, int n_steps,
+                                        float* x_out, float* traj, const msmd_sample_extras* ex,
+                                        const msmd_sample_schedule* sched, void* stream) {
   MSMD_REQUIRE(m && x_T && x_out, "msmd_sample_window: null argument");
   if (!m->window) { set_error("msmd_sample_window: call msmd_window_begin first"); return MSMD_ERR_STATE; }
   const msmd_config& c = m->c;
-  MSMD_REQUIRE(t_start >= 1 && t_start <= c.n_diff_steps && n_steps >= 1 && n_steps <= t_start,
-               "msmd_sample_window: steps %d..%d outside 1..%d", t_start, t_start - n_steps + 1, c.n_diff_steps);
-  MSMD_REQUIRE(flexibility >= 0.f && flexibility <= 1.f, "msmd_sample_window: flexibility outside [0,1]");
+  std::vector<SchedStep> plan;   // respaced calls: the visited steps, in order
+  if (sched) {
+    int r = plan_respaced(m, *sched, flexibility, t_start, n_steps, plan);
+    if (r) return r;
+  } else {
+    MSMD_REQUIRE(t_start >= 1 && t_start <= c.n_diff_steps && n_steps >= 1 && n_steps <= t_start,
+                 "msmd_sample_window: steps %d..%d outside 1..%d", t_start, t_start - n_steps + 1, c.n_diff_steps);
+    MSMD_REQUIRE(flexibility >= 0.f && flexibility <= 1.f, "msmd_sample_window: flexibility outside [0,1]");
+  }
   MSMD_REQUIRE(!(ex && ex->noise_keys && z),
                "msmd_sample_window: noise_keys key the in-kernel noise and cannot be combined with an external z");
   int rc;
@@ -742,6 +809,12 @@ extern "C" int msmd_sample_window_ex(msmd_model* m, const float* x_T, const floa
       up.noise_keys = m->d_keys;
     }
     if (up.cum_static) MSMD_CHECK_CUDA(cudaMemsetAsync(up.cum_static, 0, n_el * 4, st));
+  }
+  if (sched) {
+    // the visited steps' entries go into the engine-owned table (stream order, by value): the step graphs keep reading only
+    // engine memory, so respaced and default calls of one shape share them
+    if ((rc = sched_table_set(m->d_sched, plan.data(), (int)plan.size(), st))) return rc;
+    up.sched = m->d_sched;
   }
   if ((rc = update_params_set(m->d_up, up, st))) return rc;
 
@@ -798,9 +871,16 @@ extern "C" int msmd_sample_window_ex(msmd_model* m, const float* x_T, const floa
     return MSMD_OK;
   };
 
-  // executed steps are t = t_start .. t_end
+  // executed steps are t = t_start .. t_end, or the visited entries of a respaced call; the segments are counted in t
   const int t_end = t_start - n_steps + 1;
-  auto count = [&](int hi, int lo) { hi = std::min(hi, t_start); lo = std::max(lo, t_end); return hi >= lo ? hi - lo + 1 : 0; };
+  auto count = [&](int hi, int lo) {
+    if (sched) {
+      int n = 0;
+      for (const SchedStep& e : plan) n += e.t <= hi && e.t >= lo;
+      return n;
+    }
+    hi = std::min(hi, t_start); lo = std::max(lo, t_end); return hi >= lo ? hi - lo + 1 : 0;
+  };
   const int n_main = count(c.n_diff_steps, k16 + 1), n_f16 = count(k16, k32 + 1), n_hi = count(k32, 1);
   if ((rc = run_16(has_bf16(c) ? 0 : 2, n_main))) return rc;
   if ((rc = run_16(2, n_f16))) return rc;

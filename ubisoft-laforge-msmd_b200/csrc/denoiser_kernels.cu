@@ -749,16 +749,22 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
   const UpdateParams& p = *reinterpret_cast<const UpdateParams*>(p_raw);
   const int64_t n_el = (int64_t)p.NX * p.L * p.dm;
   const int t = p.steps[0];
-  // model.py:383-386, :421-428 - 0-dim fp32 tensor arithmetic, same operation order
-  const float alpha = p.alphas[t], ab = p.alpha_bars[t], abp = p.alpha_bars[t - 1];
-  const float sigma = p.sig_flex[t] * p.flexibility + p.sig_inflex[t] * (1.0f - p.flexibility);
-  float c0, c1;
-  if (p.target_noise) {
-    c0 = 1.0f / sqrtf(alpha);
-    c1 = (1.0f - alpha) / sqrtf(1.0f - ab);
+  float sigma, c0, c1;
+  int t_next = t - 1, ord = p.t_start - t;
+  if (p.sched != nullptr) {   // respaced schedule: host-computed coefficients of x_s = c0 x_t + c1 out + sigma z
+    const SchedStep e = p.sched[t];
+    c0 = e.c0; c1 = e.c1; sigma = e.sigma; t_next = e.next; ord = e.ord;
   } else {
-    c0 = (1.0f - abp) * sqrtf(alpha) / (1.0f - ab);
-    c1 = (1.0f - alpha) * sqrtf(abp) / (1.0f - ab);
+    // model.py:383-386, :421-428 - 0-dim fp32 tensor arithmetic, same operation order
+    const float alpha = p.alphas[t], ab = p.alpha_bars[t], abp = p.alpha_bars[t - 1];
+    sigma = p.sig_flex[t] * p.flexibility + p.sig_inflex[t] * (1.0f - p.flexibility);
+    if (p.target_noise) {
+      c0 = 1.0f / sqrtf(alpha);
+      c1 = (1.0f - alpha) / sqrtf(1.0f - ab);
+    } else {
+      c0 = (1.0f - abp) * sqrtf(alpha) / (1.0f - ab);
+      c1 = (1.0f - alpha) * sqrtf(abp) / (1.0f - ab);
+    }
   }
   // loop-invariant fields in registers: the stores below go through generic pointers that the compiler must assume may
   // alias the shared-memory parameter block, so every p.field in the loop was re-read after each store
@@ -766,11 +772,13 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
     const float *dec, *stat, *z, *thr; float *x, *traj, *tgt_dyn, *cum_static, *alpha_traj; const int* overflow;
     const long long* keys;
     float scale0, scale1; unsigned long long seed; long long noise_offset;
-    int NX, E, T, L, Lp, dm, nb, ldd, cfg_independent, target_noise, t_start;
+    int NX, E, T, L, Lp, dm, nb, ldd, cfg_independent, target_noise;
   };
+  // target_noise here selects the posterior's form x_{t-1} = c0 (x_t - c1 eps_hat); a respaced step is affine in both
+  // targets
   const Loc q = {p.dec, p.stat, p.z, p.thr, p.x, p.traj, p.tgt_dyn, p.cum_static, p.alpha_traj, p.overflow, p.noise_keys,
                  p.scale0, p.scale1, p.seed, p.noise_offset,
-                 p.NX, p.E, p.T, p.L, p.Lp, p.dm, p.nb, p.ldd, p.cfg_independent, p.target_noise, p.t_start};
+                 p.NX, p.E, p.T, p.L, p.Lp, p.dm, p.nb, p.ldd, p.cfg_independent, p.target_noise && p.sched == nullptr};
   const bool sep = q.tgt_dyn != nullptr || q.cum_static != nullptr;
   // warp = one (clip, frame) row of dm codes, lane = column c (+32, +64): no 64-bit index arithmetic per element (three
   // int64 divisions per element made this kernel instruction-bound: 600 instructions per element, 23 us per step)
@@ -832,14 +840,14 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
       prev = r; pd = dyn; psv = sta;
     }
     float zt = 0.f;
-    if (t > 1) zt = q.z ? q.z[(int64_t)t * n_el + i] : philox_normal(nseed, (uint32_t)t, (uint32_t)(nbase + c));
+    if (t_next > 0) zt = q.z ? q.z[(int64_t)t * n_el + i] : philox_normal(nseed, (uint32_t)t, (uint32_t)(nbase + c));
     const float xo = q.x[i];
     float xn = q.target_noise ? (c0 * (xo - c1 * tgt) + sigma * zt) : (c0 * xo + c1 * tgt + sigma * zt);
     // fp32-grade steps: an activation left the fp16 range of the operand split -> poison the state instead of
     // returning a silently wrong sample (the host reports it at the next call, without synchronising this one)
     if (q.overflow != nullptr && *q.overflow != 0) xn = __int_as_float(0x7fc00000);
     q.x[i] = xn;
-    if (q.traj) q.traj[(int64_t)(t - 1) * n_el + i] = xn;
+    if (q.traj) q.traj[(int64_t)t_next * n_el + i] = xn;
     if (q.tgt_dyn) q.tgt_dyn[i] = td;
     if (q.cum_static) q.cum_static[i] += c1 * ts;
     if (q.alpha_traj && c < q.nb) {   // alphas: columns dm..dm+nb-1 of the decoder output, same CFG recursion
@@ -850,11 +858,11 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
         else ta = ta + ((e == 1) ? q.scale0 : q.scale1) * (a - ((q.cfg_independent || e == 1) ? ta : pa));
         pa = a;
       }
-      q.alpha_traj[(((int64_t)(q.t_start - t) * q.NX + n) * q.L + l) * q.nb + c] = ta;
+      q.alpha_traj[(((int64_t)ord * q.NX + n) * q.L + l) * q.nb + c] = ta;
     }
    }
   }
-  // step index t -> t - 1 for the next step, by the LAST block to finish (every block has read t by then): the separate
+  // step index t -> t_next for the next step, by the LAST block to finish (every block has read t by then): the separate
   // one-thread-block "advance" launch of round 1 is gone
   if (p.done != nullptr) {
     __shared__ bool last;
@@ -865,7 +873,7 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
     }
     __syncthreads();
     if (last) {
-      for (int i = threadIdx.x; i < p.S; i += blockDim.x) p.steps_rw[i] = t - 1;
+      for (int i = threadIdx.x; i < p.S; i += blockDim.x) p.steps_rw[i] = t_next;
       if (threadIdx.x == 0) *p.done = 0u;
     }
   }
@@ -946,6 +954,26 @@ int update_launch(const UpdateParams* d_p, int NX, int L, int dm, cudaStream_t s
   // (parameter block -> step index -> schedule coefficients, ~2 us); the 4-wave grid of round 1 paid it four times
   MSMD_CHECK_CUDA(launch_pdl(update_kernel, dim3(std::min(cdiv(NX * L, 8), kNumSMs * 2)), dim3(256), 0, st, d_p));
   MSMD_CHECK_LAUNCH();
+  return MSMD_OK;
+}
+
+// 512 entries = 12 KB of kernel parameters (the limit is 32 KB): one launch for any schedule of the 500-step models
+constexpr int kSchedChunk = 512;
+struct SchedChunk {
+  int n;
+  SchedStep e[kSchedChunk];
+};
+__global__ void sched_table_set_kernel(SchedStep* table, const SchedChunk c) {
+  for (int i = threadIdx.x; i < c.n; i += blockDim.x) table[c.e[i].t] = c.e[i];
+}
+int sched_table_set(SchedStep* table, const SchedStep* h, int n, cudaStream_t st) {
+  for (int a = 0; a < n; a += kSchedChunk) {
+    SchedChunk c;
+    c.n = std::min(kSchedChunk, n - a);
+    memcpy(c.e, h + a, c.n * sizeof(SchedStep));
+    sched_table_set_kernel<<<1, 256, 0, st>>>(table, c);
+    MSMD_CHECK_LAUNCH();
+  }
   return MSMD_OK;
 }
 

@@ -64,6 +64,13 @@ int ln_row0_launch(const bf16* y0, const bf16* resid0, const float* g, const flo
 int cross_attn_row0_launch(const bf16* q0, const bf16* kv, bf16* ctx0, int S, int Tk, int H, int fp16, cudaStream_t st);
 
 
+// One visited step t of a respaced schedule (msmd_sample_window_sched): x_s = c0 x_t + c1 out + sigma z_t, where out is
+// the network output (x0_hat or eps_hat), s = next (0 after the last entry) and ord = position from the call's t_start
+struct SchedStep {
+  float c0, c1, sigma;
+  int t, next, ord;
+};
+
 struct UpdateParams {
   const float* dec;       // [S, T, ldd] fp32: motion_dec output (dm dynamic + nb alphas)
   const float* stat;      // [S, nb, dm]
@@ -89,6 +96,10 @@ struct UpdateParams {
   long long noise_offset; // added to the element index that keys the in-kernel Philox noise (= global clip id * L * dm)
   const int* overflow;    // fp32-grade steps: device flag raised by the operand split; non-zero poisons x with NaN
   const long long* noise_keys;  // [NX][2] (seed, global clip id) per clip, or null (-> seed, noise_offset); engine-owned
+  // respaced schedule: [n_diff_steps + 1] indexed by t (engine-owned), or null (-> the posterior step t -> t - 1).  When
+  // set, the step takes its coefficients from sched[t], draws noise iff next > 0, writes traj at next and alpha_traj at
+  // ord, and advances steps_rw to next
+  const SchedStep* sched;
 };
 // per-sequence threshold s = clamp(quantile(|x0_hat[:, -L:]|, ratio), lo, hi) -> thr[S] (torch.quantile 'linear')
 int threshold_launch(const float* dec, const float* stat, float* thr, int S, int T, int L, int Lp, int dm, int nb, int ldd,
@@ -96,6 +107,9 @@ int threshold_launch(const float* dec, const float* stat, float* thr, int S, int
 // the parameter block is read from DEVICE memory (d_p), written by update_params_set in stream order
 int update_params_set(UpdateParams* d_dst, const UpdateParams& p, cudaStream_t st);
 int update_launch(const UpdateParams* d_p, int NX, int L, int dm, cudaStream_t st);
+// scatter n host entries into table[entry.t], in stream order (by-value kernel arguments: the host array may be freed on
+// return, and nothing synchronises)
+int sched_table_set(SchedStep* table, const SchedStep* h, int n, cudaStream_t st);
 int steps_set(int* steps, int S, int value, cudaStream_t st);
 
 // out[S, T-1... ] : x̂0 per sequence (module-level parity): dyn + static mix for ALL Lp+L rows -> [S, T-1, dm]

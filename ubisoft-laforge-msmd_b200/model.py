@@ -7,6 +7,8 @@ only HOLD parameters - every forward runs in the CUDA engine behind the C ABI (c
 csrc/gemm_tc.cuh).  Training-only code paths of the reference (MSMD.forward's noising / CFG dropout,
 model.py:146-248) are out of scope and raise.
 """
+from fractions import Fraction
+
 import torch
 import torch.nn as nn
 
@@ -63,6 +65,35 @@ class DiffusionSchedule(nn.Module):
     def get_sigmas(self, t, flexibility=0):
         assert 0 <= flexibility <= 1
         return self.sigmas_flex[t] * flexibility + self.sigmas_inflex[t] * (1 - flexibility)
+
+
+def respaced_timesteps(n_diff_steps, k):
+    """The uniform 'trailing' respacing of a T-step schedule: round(i T / k) for i = k .. 1 (round half to even), a
+    strictly decreasing list of k steps that starts at T.  k = T gives T, T - 1, ..., 1."""
+    T, k = int(n_diff_steps), int(k)
+    if not 1 <= k <= T:
+        raise ValueError(f'k must be in [1, n_diff_steps = {T}], got {k}')
+    return [round(Fraction(i * T, k)) for i in range(k, 0, -1)]
+
+
+def respaced_coefficients(alpha_bars, timesteps, eta, target):
+    """float64 (c0, c1, sigma) per visited step of a respaced schedule: x_s = c0 x_t + c1 out + sigma z with out the
+    network output (x0_hat for target 'sample', eps_hat for 'noise'); s is the next entry (0 after the last, alpha_bars[0]
+    = 1).  The engine plans the same coefficients on the host (include/msmd_b200.h, msmd_sample_schedule)."""
+    ab = torch.as_tensor(alpha_bars).double().cpu()
+    t = torch.tensor([int(v) for v in timesteps])
+    s = torch.cat([t[1:], torch.zeros(1, dtype=t.dtype)])
+    A = ab[t]
+    B = torch.where(s > 0, ab[s], torch.ones_like(A))
+    sigma = eta * torch.sqrt((1 - B) / (1 - A)) * torch.sqrt(torch.clamp(1 - A / B, min=0))
+    r = torch.sqrt(torch.clamp(1 - B - sigma ** 2, min=0))
+    if target == 'noise':
+        c0 = torch.sqrt(B / A)
+        c1 = r - torch.sqrt(B) * torch.sqrt(1 - A) / torch.sqrt(A)
+    else:
+        c0 = r / torch.sqrt(1 - A)
+        c1 = torch.sqrt(B) - torch.sqrt(A) * c0
+    return c0, c1, sigma
 
 
 def _engine_cfg(net, n_diff_steps, target, max_seqs, precision='bf16'):
@@ -287,11 +318,17 @@ class MSMD(nn.Module, _EngineOwner):
     BF16_ERR_BOUND = 1.0e-2
     FP16_ERR_BOUND = 2.0e-3
 
-    def auto_steps(self, err, tol=1e-3):
+    def auto_steps(self, err, tol=1e-3, timesteps=None, eta=None):
         """Number of final sampling steps on which a network-output error of ``err`` could exceed ``tol`` in x_{t-1}:
         x_{t-1} = c0 x_t + c1(t) x0_hat + sigma z carries the error scaled by c1(t), which decreases with t
-        (c1(1) = 1, c1(2) = 0.52, c1(16) = 0.10 for the 500-step cosine schedule)."""
+        (c1(1) = 1, c1(2) = 0.52, c1(16) = 0.10 for the 500-step cosine schedule).  On a respaced schedule
+        (``timesteps``, ``eta``): the largest visited t whose |output coefficient| x err exceeds tol, or 0; the
+        hybrid rule 't <= bound' then selects the same visited steps."""
         sch = self.diffusion_sched
+        if timesteps is not None:
+            _, c1, _ = respaced_coefficients(sch.alpha_bars, timesteps, float(eta or 0.0), self.target)
+            over = [int(t) for t, c in zip(timesteps, c1.abs().tolist()) if c * err > tol]
+            return max(over) if over else 0
         a, ab = sch.alphas.double().cpu(), sch.alpha_bars.double().cpu()
         t = torch.arange(1, sch.num_steps + 1)
         if self.target == 'noise':
@@ -304,18 +341,19 @@ class MSMD(nn.Module, _EngineOwner):
     def auto_precise_steps(self, tol=1e-3):
         return self.auto_steps(self.FP16_ERR_BOUND, tol)
 
-    def _precise_steps(self, override=None):
-        """(fp32-grade last steps, fp16 last steps) of the hybrid schedule; (0, 0) for the single-arithmetic engines."""
+    def _precise_steps(self, override=None, timesteps=None, eta=None):
+        """(fp32-grade last steps, fp16 last steps) of the hybrid schedule; (0, 0) for the single-arithmetic engines.
+        Both are bounds in t: visited steps with t <= bound run the more precise arithmetic."""
         if self.precision != 'hybrid':
             return 0
         k = self.precise_last_steps if override is None else override
-        return self.auto_steps(self.FP16_ERR_BOUND) if k == 'auto' else int(k)
+        return self.auto_steps(self.FP16_ERR_BOUND, timesteps=timesteps, eta=eta) if k == 'auto' else int(k)
 
-    def _fp16_steps(self, override=None):
+    def _fp16_steps(self, override=None, timesteps=None, eta=None):
         if self.precision != 'hybrid':
             return 0
         k = self.fp16_last_steps if override is None else override
-        return self.auto_steps(self.BF16_ERR_BOUND) if k == 'auto' else int(k)
+        return self.auto_steps(self.BF16_ERR_BOUND, timesteps=timesteps, eta=eta) if k == 'auto' else int(k)
 
     @torch.no_grad()
     def extract_audio_feature(self, audio, frame_num=None):
@@ -327,7 +365,8 @@ class MSMD(nn.Module, _EngineOwner):
     def sample(self, audio_or_feat, shape_feat, style_feat=None, prev_motion_feat=None, prev_audio_feat=None,
                motion_at_T=None, indicator=None, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, flexibility=0,
                dynamic_threshold=None, ret_traj=False, noise=None, n_steps=None, t_start=None, _separate=False,
-               precise_last_steps=None, fp16_last_steps=None, noise_seed=None, clip_offset=0, noise_keys=None):
+               precise_last_steps=None, fp16_last_steps=None, noise_seed=None, clip_offset=0, noise_keys=None,
+               timesteps=None, eta=None):
         """model.py:282-440.  Extra keyword arguments (not in the reference): ``noise`` = externally supplied
         z tensor [T+1, N, L, 67] indexed by step t (default: in-kernel Philox seeded from torch's generator);
         ``t_start`` / ``n_steps`` = start at step t_start (motion_at_T is then x_{t_start}) and run n steps
@@ -337,8 +376,30 @@ class MSMD(nn.Module, _EngineOwner):
         in-kernel Philox step noise (used when ``noise`` is None): clip n draws the stream of global clip clip_offset + n
         under ``noise_seed`` (default: a seed drawn from torch's generator), so clip-sharded runs reproduce the
         single-GPU codes (SURVEY 8(e)); ``noise_keys`` = int64 [N, 2] of (seed, global clip id) per clip, instead of
-        ``noise_seed`` / ``clip_offset``, so one call can carry clips of different windows (inference.infer_coeffs_queue)."""
+        ``noise_seed`` / ``clip_offset``, so one call can carry clips of different windows (inference.infer_coeffs_queue);
+        ``timesteps`` / ``eta`` = sample on a respaced (DDIM) schedule: a strictly decreasing list of visited steps in
+        [1, T] (e.g. respaced_timesteps(T, 50)) and eta in [0, 1] (default 0, deterministic), with ``flexibility`` 0.
+        ``t_start`` must then be an entry of the list and ``n_steps`` counts list entries; ``ret_traj`` returns x_t
+        over the visited t and 0."""
         N = audio_or_feat.shape[0]
+        if timesteps is None:
+            if eta is not None:
+                raise ValueError('eta applies to a respaced schedule: pass timesteps too')
+        else:
+            if isinstance(timesteps, torch.Tensor):
+                timesteps = timesteps.reshape(-1).tolist()
+            timesteps = [int(t) for t in timesteps]
+            T_all = self.diffusion_sched.num_steps
+            if not timesteps or any(not 1 <= t <= T_all for t in timesteps) or \
+                    any(b >= a for a, b in zip(timesteps, timesteps[1:])):
+                raise ValueError(f'timesteps must be a non-empty, strictly decreasing list in [1, {T_all}]')
+            eta = 0.0 if eta is None else float(eta)
+            if not 0.0 <= eta <= 1.0:
+                raise ValueError(f'eta must be in [0, 1], got {eta}')
+            if flexibility != 0:
+                raise ValueError('flexibility has no meaning on a respaced schedule: it must be 0 with timesteps')
+            if t_start is not None and t_start not in timesteps:
+                raise ValueError(f't_start {t_start} is not an entry of timesteps')
         if noise_keys is not None:
             if not isinstance(noise_keys, torch.Tensor) or noise_keys.dtype != torch.int64 or \
                     tuple(noise_keys.shape) != (N, 2):
@@ -413,16 +474,28 @@ class MSMD(nn.Module, _EngineOwner):
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
         s0 = float(cfg_scale[0]) if E > 1 else 0.0
         s1 = float(cfg_scale[1]) if E > 2 else 0.0
-        T = t_start or self.diffusion_sched.num_steps
+        T = t_start or (timesteps[0] if timesteps is not None else self.diffusion_sched.num_steps)
+        visited = None
+        if timesteps is not None:
+            visited = timesteps[timesteps.index(T):]
+            n_steps = n_steps or len(visited)
+            visited = visited[:n_steps]
         res = eng.sample_window(motion_at_T, noise, seed, cfg_mode == 'independent', s0, s1, flexibility,
                                 t_start=T, n_steps=n_steps, want_traj=ret_traj, dynamic_threshold=dynamic_threshold,
                                 separate=_separate,
-                                precise_last_steps=self._precise_steps(precise_last_steps),
-                                fp16_last_steps=self._fp16_steps(fp16_last_steps), noise_clip_offset=clip_offset,
-                                noise_keys=noise_keys)
+                                precise_last_steps=self._precise_steps(precise_last_steps, timesteps, eta),
+                                fp16_last_steps=self._fp16_steps(fp16_last_steps, timesteps, eta),
+                                noise_clip_offset=clip_offset, noise_keys=noise_keys, timesteps=timesteps, eta=eta)
         x0, traj = res[0], res[1]
         if _separate and not ret_traj:
             return x0, motion_at_T, audio_feat, res[2]
+        if ret_traj and visited is not None:
+            # x_s at each visited step's successor s (the list's next entry, 0 after the last)
+            nxt = timesteps[timesteps.index(visited[-1]) + 1] if visited[-1] != timesteps[-1] else 0
+            out = {T: motion_at_T.cpu()}
+            out.update({t: traj[t].cpu() for t in visited[1:]})
+            out[nxt] = traj[nxt]
+            return out, motion_at_T, audio_feat
         if ret_traj:
             last = T - (n_steps or T)
             out = {T: motion_at_T.cpu()}
@@ -435,16 +508,17 @@ class MSMD(nn.Module, _EngineOwner):
 def _sample_separate(self, audio_or_feat, shape_feat, style_feat=None, prev_motion_feat=None, prev_audio_feat=None,
                      motion_at_T=None, indicator=None, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, flexibility=0,
                      dynamic_threshold=None, ret_traj=False, alpah_t_modification=None, return_all_alpha=False,
-                     noise=None, n_steps=None):
+                     noise=None, n_steps=None, timesteps=None, eta=None):
     """model.py:442-651.  Same loop as ``sample`` plus the decomposition outputs:
     (x0, x_T, audio_feat, target_dynamic, cumulative_static, alpha) with alpha = all steps concatenated along
     dim 0 (return_all_alpha) or the last step's [N, L, n_basis].  ``alpah_t_modification`` (a Python callback on
-    the alphas of every step) cannot run inside the fused loop and must be None."""
+    the alphas of every step) cannot run inside the fused loop and must be None.  ``timesteps`` / ``eta``: a respaced
+    schedule as in ``MSMD.sample``; alpha then has one entry per visited step."""
     if alpah_t_modification is not None:
         raise _lib.MsmdError('msmd_b200: alpah_t_modification callbacks are not supported by the fused sampler')
     out = self.sample(audio_or_feat, shape_feat, style_feat, prev_motion_feat, prev_audio_feat, motion_at_T, indicator,
                       cfg_mode, cfg_cond, cfg_scale, flexibility, dynamic_threshold, ret_traj, noise=noise,
-                      n_steps=n_steps, _separate=True)
+                      n_steps=n_steps, _separate=True, timesteps=timesteps, eta=eta)
     if ret_traj:
         return out
     x0, x_T, audio_feat, (tgt_dyn, cum_static, alpha_traj) = out
