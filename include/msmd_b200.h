@@ -224,11 +224,28 @@ int msmd_sample_window_ex(msmd_model* m, const float* x_T, const float* z, uint6
  * a step is x_s = k x_t + (sqrt(B) - sqrt(A) k) x0_hat + sigma z_t with k = r / sqrt(1 - A)       (target 'sample')
  *        or x_s = sqrt(B / A) x_t + (r - sqrt(B) sqrt(1 - A) / sqrt(A)) eps_hat + sigma z_t           (target 'noise').
  * z_t is the noise of step t of the default loop (z[t], or the in-kernel Philox stream keyed by t) and is drawn only
- * when s > 0.  The list is read on the host during the call and may be freed on return. */
+ * when s > 0.  The list is read on the host during the call and may be freed on return.
+ *
+ * solver 1 is DPM-Solver++(2M) (its SDE variant for eta > 0; this eta is not DDIM's).  With alpha = sqrt(alpha_bar),
+ * sigma = sqrt(1 - alpha_bar), lambda = log(alpha / sigma), p the entry executed before t, h = lambda_s - lambda_t and
+ * r = (lambda_t - lambda_p) / h, a step is
+ *   D   = x0_t + (x0_t - x0_p) / (2 r)    (D = x0_t when there is no p, and on the step to s = 0)
+ *   x_s = (sigma_s / sigma_t) e^{-eta h} x_t + alpha_s (1 - e^{-(1 + eta) h}) D + sigma_s sqrt(1 - e^{-2 eta h}) z_t
+ * where x0 is the CFG-combined, thresholded data prediction (x0 = (x_t - sigma_t eps_hat) / alpha_t for target
+ * 'noise'); z_t is drawn as for solver 0.  A first-order step has DDIM's coefficients at eta = 0 and at eta = 1.
+ * The engine keeps x0 of the last executed step per row; a call starts without one, so its first step is first
+ * order unless x0_prev is given.
+ *   solver:  0 = DDIM (zero-initialised callers), 1 = DPM-Solver++(2M); anything else is MSMD_ERR_INVALID.
+ *   x0_prev: device [NX, L, dm] or NULL: x0 of the list entry before t_start, so a call that starts mid-list takes its
+ *            first step at second order.  Copied into the handle in stream order (the caller may free it on return).
+ *            MSMD_ERR_INVALID with solver 0 and when t_start is the list's first entry.
+ * Solver 1 together with extras->cumulative_static is MSMD_ERR_INVALID. */
 typedef struct {
   const int32_t* timesteps;
   int n_timesteps;
   float eta;
+  int solver;
+  const float* x0_prev;
 } msmd_sample_schedule;
 
 /* msmd_sample_window_ex on a respaced schedule (sched = NULL: the default loop t = t_start .. t_start - n_steps + 1).

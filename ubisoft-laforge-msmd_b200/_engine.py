@@ -21,8 +21,13 @@ class SampleExtras(C.Structure):
 
 
 class SampleSchedule(C.Structure):
-    """msmd_sample_schedule: a HOST int32 list of visited timesteps (strictly decreasing) and eta."""
-    _fields_ = [('timesteps', C.POINTER(C.c_int32)), ('n_timesteps', C.c_int), ('eta', C.c_float)]
+    """msmd_sample_schedule: a HOST int32 list of visited timesteps (strictly decreasing), eta, the solver (0 DDIM,
+    1 DPM-Solver++(2M)) and an optional device x0_prev."""
+    _fields_ = [('timesteps', C.POINTER(C.c_int32)), ('n_timesteps', C.c_int), ('eta', C.c_float), ('solver', C.c_int),
+                ('x0_prev', C.c_void_p)]
+
+
+SOLVERS = {'ddim': 0, 'dpmpp_2m': 1}
 
 
 PRECISIONS = {'bf16': 0, 'fp32': 1, 'hybrid': 2, 'fp16': 3}
@@ -119,18 +124,27 @@ class DenoiserEngine:
     def sample_window(self, x_T, z=None, seed=0, cfg_independent=False, scale0=0.0, scale1=0.0, flexibility=0.0,
                       t_start=None, n_steps=None, want_traj=False, dynamic_threshold=None, separate=False,
                       precise_last_steps=0, fp16_last_steps=0, noise_clip_offset=0, noise_keys=None, timesteps=None,
-                      eta=0.0):
+                      eta=0.0, solver='ddim', x0_prev=None):
         """noise_keys: int64 [N, 2] (seed, global clip id) per clip, keying each clip's in-kernel noise on its own
         (``seed`` and ``noise_clip_offset`` are then unused).  The library rejects it together with ``z``.
         timesteps: strictly decreasing visited steps of a respaced (DDIM) schedule with ``eta`` in [0, 1], or None for
         the default loop t_start, t_start - 1, ...  On a schedule t_start defaults to its first entry and n_steps to the
-        entries from t_start on; ``traj`` then holds x_s at each visited successor s."""
+        entries from t_start on; ``traj`` then holds x_s at each visited successor s.  solver: 'ddim' or 'dpmpp_2m'
+        (needs timesteps); x0_prev: [N, L, dm] data prediction of the list entry before t_start ('dpmpp_2m')."""
         c = self.cfg
         x_T = x_T.detach().to(self.device, torch.float32).contiguous()
         sched = ts = None
+        if solver not in SOLVERS:
+            raise ValueError(f'solver must be one of {sorted(SOLVERS)}, got {solver!r}')
+        if x0_prev is not None:
+            x0_prev = x0_prev.detach().to(self.device, torch.float32).contiguous()
+            if x0_prev.shape != x_T.shape:
+                raise ValueError(f'x0_prev must be [N, L, d] = {tuple(x_T.shape)}, got {tuple(x0_prev.shape)}')
+        if timesteps is None and (solver != 'ddim' or x0_prev is not None):
+            raise ValueError("solver='dpmpp_2m' and x0_prev need a respaced schedule: pass timesteps")
         if timesteps is not None:
             ts = (C.c_int32 * len(timesteps))(*[int(t) for t in timesteps])
-            sched = SampleSchedule(ts, len(timesteps), float(eta))
+            sched = SampleSchedule(ts, len(timesteps), float(eta), SOLVERS[solver], _lib.dev_ptr(x0_prev).value)
             t_start = int(timesteps[0]) if t_start is None else t_start
             if n_steps is None:
                 later = [i for i, t in enumerate(timesteps) if int(t) == t_start]

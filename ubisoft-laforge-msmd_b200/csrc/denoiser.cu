@@ -96,6 +96,7 @@ struct msmd_model {
   unsigned int* d_done = nullptr;   // block-completion counter of the update kernel
   long long* d_keys = nullptr;      // [max_seqs][2] per-clip Philox keys of the current call (msmd_sample_extras.noise_keys)
   SchedStep* d_sched = nullptr;     // [n_diff_steps + 1] respaced-step table of the current call, indexed by t
+  float* d_hist = nullptr;          // [max_seqs, L, dm] data prediction of the last executed DPM-Solver++(2M) step, per row
   std::vector<double> h_alpha_bars; // host copy of diffusion_sched.alpha_bars: the respaced coefficients are planned on the host
   cudaStream_t cap_stream = nullptr;
   typedef std::tuple<int, int, int, int, int, float, float, float> GraphKey;
@@ -389,6 +390,7 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
   A(&m->xbuf, S * c.n_motions * c.motion_dim); A(&m->mixed, S * (T - 1) * c.motion_dim); A(&m->steps, S);
   A(&m->w_audio, S * c.n_motions * d); A(&m->w_prev_audio, S * c.n_prev_motions * d); A(&m->w_ind, S * c.n_motions);
   A(&m->d_up, 1); A(&m->d_done, 1); A(&m->d_keys, S * 2); A(&m->d_sched, (size_t)c.n_diff_steps + 1);
+  A(&m->d_hist, S * c.n_motions * c.motion_dim);
   if (has_bf16(c) || has_fp16(c)) {
     A(&m->x, M * d); A(&m->qkv, M * 3 * d); A(&m->ctx, M * d); A(&m->h, M * c.d_ff); A(&m->dec1, M * d / 2);
     A(&m->x0c, S * d); A(&m->q0, S * d); A(&m->ctx0, S * d); A(&m->y, M * d); A(&m->y0, S * d);
@@ -708,6 +710,8 @@ int plan_respaced(const msmd_model* m, const msmd_sample_schedule& sc, float fle
   const msmd_config& c = m->c;
   MSMD_REQUIRE(sc.timesteps && sc.n_timesteps >= 1, "msmd_sample_window: empty timestep list");
   MSMD_REQUIRE(sc.eta >= 0.f && sc.eta <= 1.f, "msmd_sample_window: eta %g outside [0, 1]", (double)sc.eta);
+  MSMD_REQUIRE(sc.solver == 0 || sc.solver == 1, "msmd_sample_window: solver %d (0 DDIM, 1 DPM-Solver++(2M))", sc.solver);
+  MSMD_REQUIRE(!sc.x0_prev || sc.solver == 1, "msmd_sample_window: x0_prev needs solver 1 (DPM-Solver++(2M))");
   MSMD_REQUIRE(flexibility == 0.f, "msmd_sample_window: flexibility %g has no meaning on a respaced schedule (must be 0)",
                (double)flexibility);
   const int K = sc.n_timesteps;
@@ -723,6 +727,7 @@ int plan_respaced(const msmd_model* m, const msmd_sample_schedule& sc, float fle
   MSMD_REQUIRE(pos >= 0, "msmd_sample_window: t_start %d is not an entry of the timestep list", t_start);
   MSMD_REQUIRE(n_steps >= 1 && pos + n_steps <= K, "msmd_sample_window: n_steps %d outside [1, %d] list entries from t_start %d",
                n_steps, K - pos, t_start);
+  MSMD_REQUIRE(!sc.x0_prev || pos > 0, "msmd_sample_window: x0_prev given but t_start %d is the list's first entry", t_start);
   const std::vector<double>& ab = m->h_alpha_bars;
   const double eta = sc.eta;
   out.resize(n_steps);
@@ -730,6 +735,34 @@ int plan_respaced(const msmd_model* m, const msmd_sample_schedule& sc, float fle
     const int t = ts[pos + i], s = pos + i + 1 < K ? ts[pos + i + 1] : 0;
     const double A = ab[t], B = s > 0 ? ab[s] : 1.0;
     MSMD_REQUIRE(A < 1.0 && A > 0.0, "msmd_sample_window: alpha_bars[%d] = %g outside (0, 1)", t, A);
+    if (sc.solver == 1) {
+      // DPM-Solver++(2M) in the lambda form (include/msmd_b200.h); second order when the call has a predecessor p
+      // (an earlier step of this call, or x0_prev) and s > 0
+      const double al_t = std::sqrt(A), sg_t = std::sqrt(1.0 - A), lam_t = std::log(al_t / sg_t);
+      double k = 0.0, M = 1.0, sigma = 0.0;   // s = 0: x_0 = D
+      if (s > 0) {
+        MSMD_REQUIRE(B < 1.0 && B > A, "msmd_sample_window: alpha_bars[%d] = %g outside (alpha_bars[%d], 1)", s, B, t);
+        const double al_s = std::sqrt(B), sg_s = std::sqrt(1.0 - B), h = std::log(al_s / sg_s) - lam_t;
+        k = sg_s / sg_t * std::exp(-eta * h);
+        M = al_s * -std::expm1(-(1.0 + eta) * h);
+        sigma = sg_s * std::sqrt(-std::expm1(-2.0 * eta * h));
+      }
+      double w1 = 1.0, w2 = 0.0;   // D = w1 x0_t + w2 x0_p
+      if (s > 0 && (i > 0 || sc.x0_prev)) {
+        const double Ap = ab[ts[pos + i - 1]];
+        const double lam_p = std::log(std::sqrt(Ap) / std::sqrt(1.0 - Ap));
+        const double h = std::log(std::sqrt(B) / std::sqrt(1.0 - B)) - lam_t, r = (lam_t - lam_p) / h;
+        w1 = 1.0 + 0.5 / r;
+        w2 = -0.5 / r;
+      }
+      // x0_t = a x_t + b out: out itself for target 'sample', (x_t - sigma_t eps_hat) / alpha_t for 'noise'
+      const double a = c.target_noise ? 1.0 / al_t : 0.0, b = c.target_noise ? -sg_t / al_t : 1.0;
+      // the history is written only where the next step of this call reads it
+      const bool keep = i + 1 < n_steps && pos + i + 2 < K;
+      out[i] = SchedStep{(float)(k + M * w1 * a), (float)(M * w1 * b), (float)sigma, (float)(M * w2),
+                         keep ? (float)a : 0.f, keep ? (float)b : 0.f, t, s, i};
+      continue;
+    }
     const double sigma = eta * std::sqrt((1.0 - B) / (1.0 - A)) * std::sqrt(std::max(0.0, 1.0 - A / B));
     const double r = std::sqrt(std::max(0.0, 1.0 - B - sigma * sigma));
     double c0, c1;
@@ -740,7 +773,7 @@ int plan_respaced(const msmd_model* m, const msmd_sample_schedule& sc, float fle
       c0 = r / std::sqrt(1.0 - A);
       c1 = std::sqrt(B) - std::sqrt(A) * c0;
     }
-    out[i] = SchedStep{(float)c0, (float)c1, (float)sigma, t, s, i};
+    out[i] = SchedStep{(float)c0, (float)c1, (float)sigma, 0.f, 0.f, 0.f, t, s, i};
   }
   return MSMD_OK;
 }
@@ -764,6 +797,8 @@ extern "C" int msmd_sample_window_sched(msmd_model* m, const float* x_T, const f
   }
   MSMD_REQUIRE(!(ex && ex->noise_keys && z),
                "msmd_sample_window: noise_keys key the in-kernel noise and cannot be combined with an external z");
+  MSMD_REQUIRE(!(sched && sched->solver == 1 && ex && ex->cumulative_static),
+               "msmd_sample_window: cumulative_static is not available with solver 1 (DPM-Solver++(2M))");
   int rc;
   if ((rc = poll_overflow(m, "msmd_sample_window"))) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -815,6 +850,9 @@ extern "C" int msmd_sample_window_sched(msmd_model* m, const float* x_T, const f
     // engine memory, so respaced and default calls of one shape share them
     if ((rc = sched_table_set(m->d_sched, plan.data(), (int)plan.size(), st))) return rc;
     up.sched = m->d_sched;
+    up.hist = m->d_hist;
+    // copied into the handle like noise_keys: the step graph reads only engine-owned memory
+    if (sched->x0_prev) MSMD_CHECK_CUDA(cudaMemcpyAsync(m->d_hist, sched->x0_prev, n_el * 4, cudaMemcpyDeviceToDevice, st));
   }
   if ((rc = update_params_set(m->d_up, up, st))) return rc;
 

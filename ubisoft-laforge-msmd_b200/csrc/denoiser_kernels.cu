@@ -749,11 +749,11 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
   const UpdateParams& p = *reinterpret_cast<const UpdateParams*>(p_raw);
   const int64_t n_el = (int64_t)p.NX * p.L * p.dm;
   const int t = p.steps[0];
-  float sigma, c0, c1;
+  float sigma, c0, c1, c2 = 0.f, ha = 0.f, hb = 0.f;
   int t_next = t - 1, ord = p.t_start - t;
-  if (p.sched != nullptr) {   // respaced schedule: host-computed coefficients of x_s = c0 x_t + c1 out + sigma z
+  if (p.sched != nullptr) {   // respaced schedule: host-computed coefficients of x_s = c0 x_t + c1 out + c2 h_p + sigma z
     const SchedStep e = p.sched[t];
-    c0 = e.c0; c1 = e.c1; sigma = e.sigma; t_next = e.next; ord = e.ord;
+    c0 = e.c0; c1 = e.c1; sigma = e.sigma; c2 = e.c2; ha = e.a; hb = e.b; t_next = e.next; ord = e.ord;
   } else {
     // model.py:383-386, :421-428 - 0-dim fp32 tensor arithmetic, same operation order
     const float alpha = p.alphas[t], ab = p.alpha_bars[t], abp = p.alpha_bars[t - 1];
@@ -769,14 +769,15 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
   // loop-invariant fields in registers: the stores below go through generic pointers that the compiler must assume may
   // alias the shared-memory parameter block, so every p.field in the loop was re-read after each store
   struct Loc {
-    const float *dec, *stat, *z, *thr; float *x, *traj, *tgt_dyn, *cum_static, *alpha_traj; const int* overflow;
+    const float *dec, *stat, *z, *thr; float *x, *traj, *tgt_dyn, *cum_static, *alpha_traj, *hist; const int* overflow;
     const long long* keys;
     float scale0, scale1; unsigned long long seed; long long noise_offset;
     int NX, E, T, L, Lp, dm, nb, ldd, cfg_independent, target_noise;
   };
   // target_noise here selects the posterior's form x_{t-1} = c0 (x_t - c1 eps_hat); a respaced step is affine in both
   // targets
-  const Loc q = {p.dec, p.stat, p.z, p.thr, p.x, p.traj, p.tgt_dyn, p.cum_static, p.alpha_traj, p.overflow, p.noise_keys,
+  const Loc q = {p.dec, p.stat, p.z, p.thr, p.x, p.traj, p.tgt_dyn, p.cum_static, p.alpha_traj, p.hist, p.overflow,
+                 p.noise_keys,
                  p.scale0, p.scale1, p.seed, p.noise_offset,
                  p.NX, p.E, p.T, p.L, p.Lp, p.dm, p.nb, p.ldd, p.cfg_independent, p.target_noise && p.sched == nullptr};
   const bool sep = q.tgt_dyn != nullptr || q.cum_static != nullptr;
@@ -842,7 +843,12 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restr
     float zt = 0.f;
     if (t_next > 0) zt = q.z ? q.z[(int64_t)t * n_el + i] : philox_normal(nseed, (uint32_t)t, (uint32_t)(nbase + c));
     const float xo = q.x[i];
-    float xn = q.target_noise ? (c0 * (xo - c1 * tgt) + sigma * zt) : (c0 * xo + c1 * tgt + sigma * zt);
+    // DPM-Solver++(2M) steps read the previous step's data prediction and leave their own for the next step; DDIM
+    // steps and the default loop keep their expression (c2 = b = 0, uniform over the grid)
+    float xn;
+    if (c2 != 0.f) xn = c0 * xo + c1 * tgt + c2 * q.hist[i] + sigma * zt;
+    else xn = q.target_noise ? (c0 * (xo - c1 * tgt) + sigma * zt) : (c0 * xo + c1 * tgt + sigma * zt);
+    if (hb != 0.f) q.hist[i] = ha * xo + hb * tgt;
     // fp32-grade steps: an activation left the fp16 range of the operand split -> poison the state instead of
     // returning a silently wrong sample (the host reports it at the next call, without synchronising this one)
     if (q.overflow != nullptr && *q.overflow != 0) xn = __int_as_float(0x7fc00000);
@@ -957,12 +963,13 @@ int update_launch(const UpdateParams* d_p, int NX, int L, int dm, cudaStream_t s
   return MSMD_OK;
 }
 
-// 512 entries = 12 KB of kernel parameters (the limit is 32 KB): one launch for any schedule of the 500-step models
+// 512 entries = 18 KB of kernel parameters (the limit is 32 KB): one launch for any schedule of the 500-step models
 constexpr int kSchedChunk = 512;
 struct SchedChunk {
   int n;
   SchedStep e[kSchedChunk];
 };
+static_assert(sizeof(SchedChunk) <= 32764, "sched_table_set: a chunk must fit the kernel-parameter limit");
 __global__ void sched_table_set_kernel(SchedStep* table, const SchedChunk c) {
   for (int i = threadIdx.x; i < c.n; i += blockDim.x) table[c.e[i].t] = c.e[i];
 }

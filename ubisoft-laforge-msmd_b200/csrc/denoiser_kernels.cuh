@@ -64,10 +64,12 @@ int ln_row0_launch(const bf16* y0, const bf16* resid0, const float* g, const flo
 int cross_attn_row0_launch(const bf16* q0, const bf16* kv, bf16* ctx0, int S, int Tk, int H, int fp16, cudaStream_t st);
 
 
-// One visited step t of a respaced schedule (msmd_sample_window_sched): x_s = c0 x_t + c1 out + sigma z_t, where out is
-// the network output (x0_hat or eps_hat), s = next (0 after the last entry) and ord = position from the call's t_start
+// One visited step t of a respaced schedule (msmd_sample_window_sched): x_s = c0 x_t + c1 out + c2 h_p + sigma z_t,
+// where out is the network output (x0_hat or eps_hat), h_p the data prediction of the previous step (history buffer;
+// c2 = 0: not read), s = next (0 after the last entry) and ord = position from the call's t_start.  b != 0: the step
+// writes its own data prediction h_t = a x_t + b out to the history for the next step.  DDIM steps have c2 = a = b = 0.
 struct SchedStep {
-  float c0, c1, sigma;
+  float c0, c1, sigma, c2, a, b;
   int t, next, ord;
 };
 
@@ -100,6 +102,9 @@ struct UpdateParams {
   // set, the step takes its coefficients from sched[t], draws noise iff next > 0, writes traj at next and alpha_traj at
   // ord, and advances steps_rw to next
   const SchedStep* sched;
+  // [NX, L, dm] data prediction of the last executed step (engine-owned), read where sched[t].c2 != 0 and written where
+  // sched[t].b != 0, element by element by the same thread
+  float* hist;
 };
 // per-sequence threshold s = clamp(quantile(|x0_hat[:, -L:]|, ratio), lo, hi) -> thr[S] (torch.quantile 'linear')
 int threshold_launch(const float* dec, const float* stat, float* thr, int S, int T, int L, int Lp, int dm, int nb, int ldd,

@@ -21,13 +21,13 @@ import torch.nn.functional as F
 @torch.no_grad()
 def infer_coeffs_batched(model, args, audio_feat, shape_coef, style_feats=None, clip_len=None, cfg_mode=None,
                          cfg_cond=None, cfg_scale=1.15, dynamic_threshold=None, x_T=None, noise=None, noise_seed=None,
-                         clip_offset=0, timesteps=None, eta=None):
+                         clip_offset=0, timesteps=None, eta=None, solver='ddim'):
     """audio_feat [N, n_sub*n_motions, d] (already extracted); shape_coef [N,1,100] or [N,100];
     style_feats [N,d_style] (or a list per window); clip_len = frames to keep (<= n_sub*n_motions).
     x_T [N,n_motions,67] / noise ([T+1,N,L,67] or a list per window) are optional fixed inputs; without ``noise`` the
     step noise is the in-kernel Philox stream keyed by (noise_seed + window, global clip id = clip_offset + n), so the
-    codes of a clip do not depend on which batch / GPU it was sampled in.  ``timesteps`` / ``eta``: sample every window on
-    a respaced schedule (MSMD.sample).
+    codes of a clip do not depend on which batch / GPU it was sampled in.  ``timesteps`` / ``eta`` / ``solver``: sample
+    every window on a respaced schedule (MSMD.sample).
     Returns [N, clip_len, 67]."""
     N, total = audio_feat.shape[:2]
     L = args.n_motions
@@ -49,7 +49,7 @@ def infer_coeffs_batched(model, args, audio_feat, shape_coef, style_feats=None, 
             audio_in, shape_coef, style_feat, prev_motion_feat, prev_audio_feat, noise_T, indicator=indicator,
             cfg_mode=cfg_mode, cfg_cond=cfg_cond, cfg_scale=cfg_scale, dynamic_threshold=dynamic_threshold, noise=z,
             noise_seed=None if noise_seed is None else int(noise_seed) + i, clip_offset=clip_offset, timesteps=timesteps,
-            eta=eta)
+            eta=eta, solver=solver)
         prev_motion_feat = motion_feat[:, -args.n_prev_motions:].clone()
         prev_audio_feat = used_audio[:, -args.n_prev_motions:]
         if i == n_sub - 1 and n_padding_frames > 0:
@@ -73,8 +73,9 @@ def plan_clip(n_samples, args, audio_unit):
 @torch.no_grad()
 def infer_coeffs(model, args, audio, shape_coef, audio_unit, style_feats=None, n_repetitions: int = 1, cfg_mode=None,
                  cfg_cond=None, cfg_scale: float = 1.15, include_shape: bool = False, dynamic_threshold=(0, 1, 4),
-                 timesteps=None, eta=None):
-    """inference.py:34-75 (one clip, 1-D 16 kHz audio).  ``timesteps`` / ``eta``: a respaced schedule (MSMD.sample)."""
+                 timesteps=None, eta=None, solver='ddim'):
+    """inference.py:34-75 (one clip, 1-D 16 kHz audio).  ``timesteps`` / ``eta`` / ``solver``: a respaced schedule
+    (MSMD.sample)."""
     n_subdivision, padded, clip_len = plan_clip(len(audio), args, audio_unit)
     if padded > len(audio):
         audio = F.pad(audio, (0, padded - len(audio)), value=0)
@@ -83,7 +84,8 @@ def infer_coeffs(model, args, audio, shape_coef, audio_unit, style_feats=None, n
     style = [rep(s) for s in style_feats] if isinstance(style_feats, list) else rep(style_feats)
     return infer_coeffs_batched(model, args, audio_feat.expand(n_repetitions, -1, -1), rep(shape_coef), style,
                                 clip_len=clip_len, cfg_mode=cfg_mode, cfg_cond=cfg_cond,
-                                cfg_scale=cfg_scale, dynamic_threshold=dynamic_threshold, timesteps=timesteps, eta=eta)
+                                cfg_scale=cfg_scale, dynamic_threshold=dynamic_threshold, timesteps=timesteps, eta=eta,
+                                solver=solver)
 
 
 def queue_schedule(n_windows, max_clips):
@@ -114,7 +116,7 @@ def queue_schedule(n_windows, max_clips):
 @torch.no_grad()
 def infer_coeffs_queue(model, args, audio_feats, shape_coefs, style_feats, clip_lens, x_T, max_clips=64, clip_ids=None,
                        noise_seed=0, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, dynamic_threshold=None, timesteps=None,
-                       eta=None):
+                       eta=None, solver='ddim'):
     """``infer_coeffs_batched`` over clips of different lengths, keeping up to ``max_clips`` clips in every sampler call.
 
     Per clip k: audio_feats[k] [n_sub_k * n_motions, d] (already extracted), shape_coefs[k] [100] / [1, 100],
@@ -123,7 +125,8 @@ def infer_coeffs_queue(model, args, audio_feats, shape_coefs, style_feats, clip_
     noise of clip k's window w is keyed by (noise_seed + w, clip_ids[k]) (default clip_ids: 0..K-1), so clip k's codes
     are those of infer_coeffs_batched on that clip alone with noise_seed and clip_offset = clip_ids[k].
     The schedule depends on the lengths only: nothing is read back from the device between windows.  ``timesteps`` /
-    ``eta``: every call samples on this one respaced schedule (the clips of a call share the step index).
+    ``eta`` / ``solver``: every call samples on this one respaced schedule (the clips of a call share the step index;
+    every call runs a whole window, so a 2M call starts first order).
     Returns (codes [K, max_k clip_lens[k], 67], zero beyond each clip's length; lengths [K] int64)."""
     K = len(audio_feats)
     if K == 0:
@@ -178,7 +181,7 @@ def infer_coeffs_queue(model, args, audio_feats, shape_coefs, style_feats, clip_
         out, _, _ = model.sample(audio_in, shape[idx], None if style is None else style[idx], prev_motion[idx], prev_audio,
                                  xT[idx], indicator=indicator, cfg_mode=cfg_mode, cfg_cond=cfg_cond, cfg_scale=cfg_scale,
                                  dynamic_threshold=dynamic_threshold, noise_keys=p[:, 3:5].contiguous(), timesteps=timesteps,
-                                 eta=eta)
+                                 eta=eta, solver=solver)
         prev_motion[idx] = out[:, -Lp:]
         codes[idx[:, None], rows] = out
     lengths = torch.tensor([int(n) for n in clip_lens], dtype=torch.int64)
@@ -220,7 +223,7 @@ def infer_coeffs_many(model, args, audios, shape_coefs, style_feats, audio_unit=
     """``infer_coeffs`` for many 1-D 16 kHz clips of any lengths: features from extract_clip_features, then
     infer_coeffs_queue.  queue_kwargs: x_T ([K, n_motions, 67] or a list; default drawn from torch's generator),
     max_clips, clip_ids, noise_seed, cfg_mode, cfg_cond, cfg_scale, dynamic_threshold (default (0, 1, 4), infer_coeffs's
-    default; None turns dynamic thresholding off), timesteps, eta (a respaced schedule for every clip).
+    default; None turns dynamic thresholding off), timesteps, eta, solver (a respaced schedule for every clip).
     Returns (codes [K, max clip_len, 67], zero beyond each clip's length; lengths [K])."""
     K = len(audios)
     if K == 0:

@@ -7,6 +7,7 @@ only HOLD parameters - every forward runs in the CUDA engine behind the C ABI (c
 csrc/gemm_tc.cuh).  Training-only code paths of the reference (MSMD.forward's noising / CFG dropout,
 model.py:146-248) are out of scope and raise.
 """
+import math
 from fractions import Fraction
 
 import torch
@@ -94,6 +95,58 @@ def respaced_coefficients(alpha_bars, timesteps, eta, target):
         c0 = r / torch.sqrt(1 - A)
         c1 = torch.sqrt(B) - torch.sqrt(A) * c0
     return c0, c1, sigma
+
+
+def dpmpp_2m_coefficients(alpha_bars, timesteps, eta, target, start=0, first=True):
+    """float64 (c0, c1, c2, sigma, a, b) per step of DPM-Solver++(2M) on a respaced schedule, for a call that runs
+    timesteps[start:]: x_s = c0 x_t + c1 out + c2 x0_p + sigma z with out the network output, x0_p the data prediction
+    of the previous step and x0_t = a x_t + b out this step's (a = 0, b = 1 for target 'sample').  The first step is
+    first order when ``first`` (no predecessor: a call without x0_prev), else its predecessor is timesteps[start - 1]
+    (x0_prev); the step to s = 0 is first order.  A call of fewer steps uses a prefix of the rows.  The engine plans
+    the same coefficients on the host (include/msmd_b200.h, msmd_sample_schedule)."""
+    ab = torch.as_tensor(alpha_bars).double().cpu().tolist()
+    ts = [int(v) for v in timesteps]
+    if not first and start == 0:
+        raise ValueError('first=False needs a predecessor: start must be > 0')
+    lam = lambda A: math.log(math.sqrt(A) / math.sqrt(1 - A))
+    rows = []
+    for i in range(start, len(ts)):
+        t, s = ts[i], (ts[i + 1] if i + 1 < len(ts) else 0)
+        al_t, sg_t = math.sqrt(ab[t]), math.sqrt(1 - ab[t])
+        k, M, sigma, w1, w2 = 0.0, 1.0, 0.0, 1.0, 0.0      # s = 0: x_0 = x0_t
+        if s > 0:
+            al_s, sg_s = math.sqrt(ab[s]), math.sqrt(1 - ab[s])
+            h = lam(ab[s]) - lam(ab[t])
+            k = sg_s / sg_t * math.exp(-eta * h)
+            M = -al_s * math.expm1(-(1 + eta) * h)
+            sigma = sg_s * math.sqrt(-math.expm1(-2 * eta * h))
+            if i > start or not first:
+                r = (lam(ab[t]) - lam(ab[ts[i - 1]])) / h
+                w1, w2 = 1 + 0.5 / r, -0.5 / r
+        a, b = (1 / al_t, -sg_t / al_t) if target == 'noise' else (0.0, 1.0)
+        rows.append([k + M * w1 * a, M * w1 * b, M * w2, sigma, a, b])
+    return tuple(torch.tensor(rows, dtype=torch.float64).T)
+
+
+def hybrid_bounds(timesteps, w1, w2, tol, err16, err_main, k32=None):
+    """Segment bounds (k32, k16) of the hybrid arithmetic on a visited-step list: steps with t <= k32 run fp32-grade
+    (error 0), t <= k16 fp16 (err16), the others the main 16-bit arithmetic (err_main).  Step j carries
+    w1[j] err(t_j) + w2[j] err(t_{j-1}): its own output's error and that of the previous step's output, which a
+    multistep solver reuses.  k32 (unless given) is the smallest bound, 0 or a visited t, with every step within tol
+    when k16 = T; then k16 is the smallest bound >= k32 that keeps every step within tol.  Feasibility is monotone in
+    both bounds, so each is the largest of the per-step minima."""
+    ts = [int(t) for t in timesteps]
+    w1, w2 = [float(v) for v in w1], [float(v) for v in w2]
+
+    def ok(j, b32, b16):
+        e = lambda t: 0.0 if t <= b32 else (err16 if t <= b16 else err_main)
+        return w1[j] * e(ts[j]) + (w2[j] * e(ts[j - 1]) if j else 0.0) <= tol
+
+    prev = lambda j: ts[j - 1] if j else ts[j]
+    if k32 is None:
+        k32 = max(next((b for b in (0, ts[j]) if ok(j, b, ts[0])), prev(j)) for j in range(len(ts)))
+    k16 = max(next((b for b in (k32, max(k32, ts[j])) if ok(j, k32, b)), max(k32, prev(j))) for j in range(len(ts)))
+    return k32, k16
 
 
 def _engine_cfg(net, n_diff_steps, target, max_seqs, precision='bf16'):
@@ -318,17 +371,26 @@ class MSMD(nn.Module, _EngineOwner):
     BF16_ERR_BOUND = 1.0e-2
     FP16_ERR_BOUND = 2.0e-3
 
-    def auto_steps(self, err, tol=1e-3, timesteps=None, eta=None):
+    def _output_weights(self, timesteps, eta, solver):
+        """Per visited step: |coefficient| of this step's network output and of the previous step's output."""
+        ab = self.diffusion_sched.alpha_bars
+        if solver == 'dpmpp_2m':
+            _, c1, c2, _, _, b = dpmpp_2m_coefficients(ab, timesteps, eta, self.target)
+            return c1.abs().tolist(), [0.0] + (c2[1:] * b[:-1]).abs().tolist()
+        _, c1, _ = respaced_coefficients(ab, timesteps, eta, self.target)
+        return c1.abs().tolist(), [0.0] * len(c1)
+
+    def auto_steps(self, err, tol=1e-3, timesteps=None, eta=None, solver='ddim'):
         """Number of final sampling steps on which a network-output error of ``err`` could exceed ``tol`` in x_{t-1}:
         x_{t-1} = c0 x_t + c1(t) x0_hat + sigma z carries the error scaled by c1(t), which decreases with t
         (c1(1) = 1, c1(2) = 0.52, c1(16) = 0.10 for the 500-step cosine schedule).  On a respaced schedule
-        (``timesteps``, ``eta``): the largest visited t whose |output coefficient| x err exceeds tol, or 0; the
-        hybrid rule 't <= bound' then selects the same visited steps."""
+        (``timesteps``, ``eta``, ``solver``): the smallest bound, 0 or a visited t, such that running the steps above
+        it with error ``err`` keeps every step within tol (hybrid_bounds); for DDIM, the largest visited t whose
+        |output coefficient| x err exceeds tol."""
         sch = self.diffusion_sched
         if timesteps is not None:
-            _, c1, _ = respaced_coefficients(sch.alpha_bars, timesteps, float(eta or 0.0), self.target)
-            over = [int(t) for t, c in zip(timesteps, c1.abs().tolist()) if c * err > tol]
-            return max(over) if over else 0
+            w1, w2 = self._output_weights(timesteps, float(eta or 0.0), solver)
+            return hybrid_bounds(timesteps, w1, w2, tol, err, err)[0]
         a, ab = sch.alphas.double().cpu(), sch.alpha_bars.double().cpu()
         t = torch.arange(1, sch.num_steps + 1)
         if self.target == 'noise':
@@ -341,19 +403,26 @@ class MSMD(nn.Module, _EngineOwner):
     def auto_precise_steps(self, tol=1e-3):
         return self.auto_steps(self.FP16_ERR_BOUND, tol)
 
-    def _precise_steps(self, override=None, timesteps=None, eta=None):
+    def _precise_steps(self, override=None, timesteps=None, eta=None, solver='ddim'):
         """(fp32-grade last steps, fp16 last steps) of the hybrid schedule; (0, 0) for the single-arithmetic engines.
-        Both are bounds in t: visited steps with t <= bound run the more precise arithmetic."""
+        Both are bounds in t: visited steps with t <= bound run the more precise arithmetic.  On a respaced schedule
+        both come from hybrid_bounds."""
         if self.precision != 'hybrid':
             return 0
         k = self.precise_last_steps if override is None else override
-        return self.auto_steps(self.FP16_ERR_BOUND, timesteps=timesteps, eta=eta) if k == 'auto' else int(k)
+        return self.auto_steps(self.FP16_ERR_BOUND, timesteps=timesteps, eta=eta, solver=solver) if k == 'auto' else int(k)
 
-    def _fp16_steps(self, override=None, timesteps=None, eta=None):
+    def _fp16_steps(self, override=None, timesteps=None, eta=None, solver='ddim', precise_override=None):
         if self.precision != 'hybrid':
             return 0
         k = self.fp16_last_steps if override is None else override
-        return self.auto_steps(self.BF16_ERR_BOUND, timesteps=timesteps, eta=eta) if k == 'auto' else int(k)
+        if k != 'auto':
+            return int(k)
+        if timesteps is None:
+            return self.auto_steps(self.BF16_ERR_BOUND)
+        w1, w2 = self._output_weights(timesteps, float(eta or 0.0), solver)
+        k32 = self._precise_steps(precise_override, timesteps, eta, solver)
+        return hybrid_bounds(timesteps, w1, w2, 1e-3, self.FP16_ERR_BOUND, self.BF16_ERR_BOUND, k32=k32)[1]
 
     @torch.no_grad()
     def extract_audio_feature(self, audio, frame_num=None):
@@ -366,7 +435,7 @@ class MSMD(nn.Module, _EngineOwner):
                motion_at_T=None, indicator=None, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, flexibility=0,
                dynamic_threshold=None, ret_traj=False, noise=None, n_steps=None, t_start=None, _separate=False,
                precise_last_steps=None, fp16_last_steps=None, noise_seed=None, clip_offset=0, noise_keys=None,
-               timesteps=None, eta=None):
+               timesteps=None, eta=None, solver='ddim', x0_prev=None):
         """model.py:282-440.  Extra keyword arguments (not in the reference): ``noise`` = externally supplied
         z tensor [T+1, N, L, 67] indexed by step t (default: in-kernel Philox seeded from torch's generator);
         ``t_start`` / ``n_steps`` = start at step t_start (motion_at_T is then x_{t_start}) and run n steps
@@ -380,11 +449,25 @@ class MSMD(nn.Module, _EngineOwner):
         ``timesteps`` / ``eta`` = sample on a respaced (DDIM) schedule: a strictly decreasing list of visited steps in
         [1, T] (e.g. respaced_timesteps(T, 50)) and eta in [0, 1] (default 0, deterministic), with ``flexibility`` 0.
         ``t_start`` must then be an entry of the list and ``n_steps`` counts list entries; ``ret_traj`` returns x_t
-        over the visited t and 0."""
+        over the visited t and 0.  ``solver`` = 'ddim' or 'dpmpp_2m' (DPM-Solver++(2M), second order with one network
+        evaluation per step; its SDE variant for eta > 0), which needs ``timesteps``; ``x0_prev`` = [N, L, 67] CUDA
+        tensor, the data prediction of the list entry before ``t_start`` (2M only), so a call that starts mid-list takes
+        its first step at second order (without it the first step of a call is first order)."""
         N = audio_or_feat.shape[0]
+        if solver not in ('ddim', 'dpmpp_2m'):
+            raise ValueError(f"solver must be 'ddim' or 'dpmpp_2m', got {solver!r}")
+        if x0_prev is not None:
+            if solver != 'dpmpp_2m':
+                raise ValueError("x0_prev applies to solver='dpmpp_2m'")
+            if not isinstance(x0_prev, torch.Tensor) or not x0_prev.is_cuda or \
+                    tuple(x0_prev.shape) != (N, self.n_motions, self.motion_feat_dim):
+                raise ValueError(f'x0_prev must be a CUDA tensor [N, L, d] = [{N}, {self.n_motions}, '
+                                 f'{self.motion_feat_dim}], got {tuple(getattr(x0_prev, "shape", ()))}')
         if timesteps is None:
             if eta is not None:
                 raise ValueError('eta applies to a respaced schedule: pass timesteps too')
+            if solver != 'ddim':
+                raise ValueError("solver='dpmpp_2m' needs a respaced schedule: pass timesteps")
         else:
             if isinstance(timesteps, torch.Tensor):
                 timesteps = timesteps.reshape(-1).tolist()
@@ -400,6 +483,8 @@ class MSMD(nn.Module, _EngineOwner):
                 raise ValueError('flexibility has no meaning on a respaced schedule: it must be 0 with timesteps')
             if t_start is not None and t_start not in timesteps:
                 raise ValueError(f't_start {t_start} is not an entry of timesteps')
+            if x0_prev is not None and (t_start or timesteps[0]) == timesteps[0]:
+                raise ValueError("x0_prev needs a predecessor: t_start must not be timesteps' first entry")
         if noise_keys is not None:
             if not isinstance(noise_keys, torch.Tensor) or noise_keys.dtype != torch.int64 or \
                     tuple(noise_keys.shape) != (N, 2):
@@ -483,9 +568,11 @@ class MSMD(nn.Module, _EngineOwner):
         res = eng.sample_window(motion_at_T, noise, seed, cfg_mode == 'independent', s0, s1, flexibility,
                                 t_start=T, n_steps=n_steps, want_traj=ret_traj, dynamic_threshold=dynamic_threshold,
                                 separate=_separate,
-                                precise_last_steps=self._precise_steps(precise_last_steps, timesteps, eta),
-                                fp16_last_steps=self._fp16_steps(fp16_last_steps, timesteps, eta),
-                                noise_clip_offset=clip_offset, noise_keys=noise_keys, timesteps=timesteps, eta=eta)
+                                precise_last_steps=self._precise_steps(precise_last_steps, timesteps, eta, solver),
+                                fp16_last_steps=self._fp16_steps(fp16_last_steps, timesteps, eta, solver,
+                                                                 precise_last_steps),
+                                noise_clip_offset=clip_offset, noise_keys=noise_keys, timesteps=timesteps, eta=eta,
+                                solver=solver, x0_prev=x0_prev)
         x0, traj = res[0], res[1]
         if _separate and not ret_traj:
             return x0, motion_at_T, audio_feat, res[2]
@@ -508,12 +595,15 @@ class MSMD(nn.Module, _EngineOwner):
 def _sample_separate(self, audio_or_feat, shape_feat, style_feat=None, prev_motion_feat=None, prev_audio_feat=None,
                      motion_at_T=None, indicator=None, cfg_mode=None, cfg_cond=None, cfg_scale=1.15, flexibility=0,
                      dynamic_threshold=None, ret_traj=False, alpah_t_modification=None, return_all_alpha=False,
-                     noise=None, n_steps=None, timesteps=None, eta=None):
+                     noise=None, n_steps=None, timesteps=None, eta=None, solver='ddim'):
     """model.py:442-651.  Same loop as ``sample`` plus the decomposition outputs:
     (x0, x_T, audio_feat, target_dynamic, cumulative_static, alpha) with alpha = all steps concatenated along
     dim 0 (return_all_alpha) or the last step's [N, L, n_basis].  ``alpah_t_modification`` (a Python callback on
     the alphas of every step) cannot run inside the fused loop and must be None.  ``timesteps`` / ``eta``: a respaced
-    schedule as in ``MSMD.sample``; alpha then has one entry per visited step."""
+    schedule as in ``MSMD.sample``; alpha then has one entry per visited step.  Only ``solver='ddim'``: the
+    cumulative static part of DPM-Solver++(2M) would need a second history buffer."""
+    if solver != 'ddim':
+        raise ValueError(f"sample_separate supports solver='ddim' only, got {solver!r}")
     if alpah_t_modification is not None:
         raise _lib.MsmdError('msmd_b200: alpah_t_modification callbacks are not supported by the fused sampler')
     out = self.sample(audio_or_feat, shape_feat, style_feat, prev_motion_feat, prev_audio_feat, motion_at_T, indicator,
