@@ -61,6 +61,18 @@ def test_flame_ragged_batches_vs_oracle(built_lib, impl, B):
     assert rel_l2(got2, want) < TOL
 
 
+@pytest.mark.parametrize('impl', [0, 1])
+def test_flame_odd_coefficient_count_vs_oracle(built_lib, impl):
+    """101 + 50 coefficients: the tensor-core pose kernel reads them in pairs and needs an even count, so an odd
+    count runs the CUDA-core pose kernel."""
+    assets = synth.flame_assets(0, synth.FLAME_V, 101, 50)
+    fl = make_flame(synth.FLAME_V, 101, 50, impl=impl)
+    sh, ex, po, ey = synth.flame_inputs(130, 101, 50, seed=5)
+    want = flame_lbs.flame_forward(assets, sh, ex, po, ey)
+    got, _, _ = fl(sh.cuda(), ex.cuda(), po.cuda(), ey.cuda(), return_lm2d=False, return_lm3d=False)
+    assert rel_l2(got, want) < TOL
+
+
 def test_flame_small_mesh_and_lbs_function(built_lib):
     """lbs() drop-in (verts AND posed joints) on a mesh whose 3V is not a tile multiple."""
     from msmd_b200.utils.lbs import lbs

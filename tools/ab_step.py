@@ -1,5 +1,5 @@
 """A/B helper: graph-replay time of a sampling step + per-class eager times for chosen kernel classes.
-python tools/ab_step.py [class ...]   (run the same command under different MSMD_* env toggles in ONE gpurun call)"""
+python tools/ab_step.py [class ...]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

@@ -1,4 +1,4 @@
-"""Pair vs single-CTA tiles of the GEMM core on the denoiser's shapes (MSMD_GEMM_CTA2=0 disables the pair).
+"""The GEMM core on the denoiser's shapes.
 Build with -DMSMD_GEMM_TRACE and set MSMD_GEMM_TRACE=1 for the per-role clock64 timeline of CTAs 0, 1, 77."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -99,7 +99,6 @@ __global__ void __launch_bounds__(kThreads, 1) self_attn_tc_kernel(const __grid_
   uint64_t* aempty_bar = ofull_bar + 2;       // [2]  S_g / O_g read out: the group's TMEM slice may be overwritten
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(aempty_bar + 2);
 
-  griddep_launch();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int d = p.H * 64;
   // contiguous job range of this CTA
@@ -121,7 +120,6 @@ __global__ void __launch_bounds__(kThreads, 1) self_attn_tc_kernel(const __grid_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  griddep_wait();
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer
@@ -336,7 +334,7 @@ int self_attn_tc_launch(const bf16* qkv, bf16* ctx, int S, int T, int H, int fp1
   const int grid = p.jobs < kNumSMs ? p.jobs : kNumSMs;
   auto kern = T > kKeys - 16 ? (fp16 ? self_attn_tc_kernel<true, true, false> : self_attn_tc_kernel<true, false, false>)
                              : (fp16 ? self_attn_tc_kernel<false, true, false> : self_attn_tc_kernel<false, false, false>);
-  MSMD_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kThreads), kSmemBytes, st, p));
+  kern<<<grid, kThreads, kSmemBytes, st>>>(p);
   MSMD_CHECK_LAUNCH();
 #ifdef MSMD_ATTN_TRACE
   {
@@ -389,7 +387,7 @@ int cross_attn_tc_launch(const bf16* q, const bf16* kv, bf16* ctx, int S, int T,
   ProfileScope prof("cross_attn", st);
   const int grid = p.jobs < kNumSMs ? p.jobs : kNumSMs;
   auto kern = fp16 ? self_attn_tc_kernel<true, true, true> : self_attn_tc_kernel<true, false, true>;
-  MSMD_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kThreads), kSmemBytes, st, p));
+  kern<<<grid, kThreads, kSmemBytes, st>>>(p);
   MSMD_CHECK_LAUNCH();
   return MSMD_OK;
 }

@@ -26,8 +26,6 @@ using namespace msmd;
 
 namespace {
 
-constexpr int kRow0FusedMaxS = 1 << 30;   // every batch size (MSMD_ROW0_FUSED_MAX_S=n: the four-launch chain above n sequences)
-
 struct LayerW {
   bf16 *Wqkv = nullptr, *Wo = nullptr, *Wq0 = nullptr, *Wkv = nullptr, *Wco = nullptr, *W1 = nullptr, *W2 = nullptr;
   float *bqkv = nullptr, *bo = nullptr, *bq0 = nullptr, *bkv = nullptr, *bco = nullptr, *b1 = nullptr, *b2 = nullptr;
@@ -69,9 +67,8 @@ struct msmd_model {
   float *bd1 = nullptr, *bd2 = nullptr;
   float *alphas = nullptr, *alpha_bars = nullptr, *sig_flex = nullptr, *sig_inflex = nullptr;
   // workspaces
-  bf16 *x = nullptr, *qkv = nullptr, *ctx = nullptr, *h = nullptr, *dec1 = nullptr, *mem = nullptr, *x0c = nullptr,
-       *q0 = nullptr, *ctx0 = nullptr;
-  bf16 *y = nullptr, *y0 = nullptr, *memh = nullptr;
+  bf16 *x = nullptr, *qkv = nullptr, *ctx = nullptr, *h = nullptr, *dec1 = nullptr, *mem = nullptr, *x0c = nullptr;
+  bf16 *y = nullptr, *memh = nullptr;
   float *dec2 = nullptr, *pp = nullptr, *pmproj = nullptr, *stat = nullptr,
         *hid = nullptr, *xbuf = nullptr, *mixed = nullptr, *thr = nullptr;
   int* steps = nullptr;
@@ -260,11 +257,10 @@ int run_forward(msmd_model* m, const float* xrows, cudaStream_t st, int fmt) {
     if ((rc = gemm(fmt, m->x, d, Wqkv, d, w.bqkv, nullptr, 0, m->qkv, 3 * d, 0, M, 3 * d, d, 0, st))) return rc;
     if ((rc = self_attn_tc_launch(m->qkv, m->ctx, S, T, c.n_heads, fmt, st))) return rc;
     if ((rc = gemm(fmt, m->ctx, d, Wo, d, w.bo, nullptr, 0, m->y, d, 0, M, d, d, 0, st))) return rc;
-    static const int row0_max_s = [] { const char* e = getenv("MSMD_ROW0_FUSED_MAX_S"); return e ? atoi(e) : kRow0FusedMaxS; }();
     LnParams lp{};
     lp.resid = m->x;
     lp.y = m->y; lp.g1 = w.g1; lp.b1 = w.be1; lp.add = ca; lp.g2 = w.g2; lp.b2 = w.be2; lp.out = m->x;
-    lp.x0 = m->x0c; lp.skip_tok0 = 0; lp.M = M; lp.T = T; lp.d = d; lp.fp16 = fmt;
+    lp.x0 = m->x0c; lp.M = M; lp.T = T; lp.d = d; lp.fp16 = fmt;
     if (c.align_mask_width != 1) {
       // banded cross attention (_mha_block with the alignment mask) of every row, person token included, on every step:
       // norm1 of all rows, q projection into the qkv workspace (free after self-attention), attention over the cached
@@ -280,17 +276,10 @@ int run_forward(msmd_model* m, const float* xrows, cudaStream_t st, int fmt) {
     } else {
       if ((rc = ln_launch(lp, st))) return rc;
       // person token (row 0): real cross attention over the memory (_mha_block) + norm2 as one cluster kernel
-      // (row0_fused.cu); the four-launch chain it replaced is kept behind MSMD_ROW0_FUSED_MAX_S for A/B runs.
-      if (S <= row0_max_s) {
-        if ((rc = row0_fused_launch(m->x0c, static_cast<const bf16*>(Wq0), w.bq0, kv, static_cast<const bf16*>(Wco), w.bco,
-                                    w.g2, w.be2, m->x, S, T, T - 1, c.n_heads, d, fmt, st)))
-          return rc;
-      } else {
-        if ((rc = gemm(fmt, m->x0c, d, Wq0, d, w.bq0, nullptr, 0, m->q0, d, 0, S, d, d, 0, st))) return rc;
-        if ((rc = cross_attn_row0_launch(m->q0, kv, m->ctx0, S, T - 1, c.n_heads, fmt, st))) return rc;
-        if ((rc = gemm(fmt, m->ctx0, d, Wco, d, w.bco, nullptr, 0, m->y0, d, 0, S, d, d, 0, st))) return rc;
-        if ((rc = ln_row0_launch(m->y0, m->x0c, w.g2, w.be2, m->x, nullptr, S, T, d, fmt, st))) return rc;
-      }
+      // (row0_fused.cu)
+      if ((rc = row0_fused_launch(m->x0c, static_cast<const bf16*>(Wq0), w.bq0, kv, static_cast<const bf16*>(Wco), w.bco,
+                                  w.g2, w.be2, m->x, S, T, T - 1, c.n_heads, d, fmt, st)))
+        return rc;
     }
     // feed-forward block (_ff_block) + norm3
     if ((rc = gemm(fmt, m->x, d, W1, d, w.b1, nullptr, 0, m->h, c.d_ff, 0, M, c.d_ff, d, 1, st))) return rc;
@@ -298,7 +287,7 @@ int run_forward(msmd_model* m, const float* xrows, cudaStream_t st, int fmt) {
     LnParams l3{};
     l3.resid = m->x;
     l3.y = m->y; l3.g1 = w.g3; l3.b1 = w.be3; l3.add = nullptr; l3.g2 = nullptr; l3.b2 = nullptr; l3.out = m->x;
-    l3.x0 = nullptr; l3.skip_tok0 = 0; l3.M = M; l3.T = T; l3.d = d; l3.fp16 = fmt;
+    l3.x0 = nullptr; l3.M = M; l3.T = T; l3.d = d; l3.fp16 = fmt;
     if ((rc = ln_launch(l3, st))) return rc;
   }
   // motion_dec (model.py:961): Linear(d, d/2) + GELU + Linear(d/2, dm + n_basis)
@@ -393,7 +382,7 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
   A(&m->d_hist, S * c.n_motions * c.motion_dim);
   if (has_bf16(c) || has_fp16(c)) {
     A(&m->x, M * d); A(&m->qkv, M * 3 * d); A(&m->ctx, M * d); A(&m->h, M * c.d_ff); A(&m->dec1, M * d / 2);
-    A(&m->x0c, S * d); A(&m->q0, S * d); A(&m->ctx0, S * d); A(&m->y, M * d); A(&m->y0, S * d);
+    A(&m->x0c, S * d); A(&m->y, M * d);
   }
   // the step-invariant cross-attention rows (ca / cah / ca32) exist only at align_mask_width 1
   const bool want_ca = c.align_mask_width == 1;
@@ -525,7 +514,7 @@ extern "C" int msmd_load_weights(msmd_model* m, const char* const* names, const 
     for (size_t cc = 0; cc < d; ++cc)
       for (size_t k = 0; k < fin; ++k) t[k * d + cc] = h[cc * fin + k];
     if (!rc) rc = up_f32(m, &m->WfT, t);
-    if (!rc && dm <= 80) {   // fp16 two-term split of the motion columns, [n][k] with K zero-padded to 80 (embed_x_mma_kernel)
+    if (!rc) {   // fp16 two-term split of the motion columns, [n][k] with K zero-padded to 80 (embed_x_mma_kernel)
       std::vector<__half> w16(2 * d * 80, __float2half_rn(0.f));
       for (size_t cc = 0; cc < d; ++cc)
         for (size_t k = 0; k < dm; ++k) {

@@ -1,8 +1,7 @@
 // Non-GEMM kernels of the denoiser / sampler: embeddings (model.py:931-949), LayerNorm chains of the
-// post-LN decoder layers, self-attention over the 111-token sequence, the person-token (row 0) cross
-// attention, and the fused CFG-combine + static-basis mix + DDPM posterior step (model.py:404-430,
-// :964-995).  All HBM-bound elementwise / small-tile work: coalesced float4 / bf16x4 accesses,
-// warp-shuffle reductions, fp32 statistics.
+// post-LN decoder layers, self-attention over the 111-token sequence, and the fused CFG-combine +
+// static-basis mix + DDPM posterior step (model.py:404-430, :964-995).  All HBM-bound elementwise /
+// small-tile work: coalesced float4 / bf16x4 accesses, warp-shuffle reductions, fp32 statistics.
 #include "denoiser_kernels.cuh"
 #include "profile.cuh"
 #include <cuda_fp16.h>
@@ -131,88 +130,11 @@ __device__ __forceinline__ void embed_ctx_rows(const EmbedParams& p, int row) {
     store_h1<F16>(p.out + ((int64_t)s * T + i) * p.d + c, v);
   }
 }
-// rows Lp+1..: feature_proj([x_t, indicator]) + PE, computed once per x row and written to its E sequences.
-// CTA = 25 frames x 512 features; the x rows sit in shared memory k-major ([k][28]) so one 128-bit broadcast
-// load feeds 4 frames' FMAs (the scalar-load version was LDS-bound at 65 us; this one is FMA-issue-bound).
-constexpr int kEmbedRows = 25, kEmbedPitch = 28;
-template <bool F16>
-__global__ void __launch_bounds__(256, 2) embed_x_kernel(EmbedParams p) {
-  griddep_launch();
-  griddep_wait();
-  extern __shared__ __align__(16) float xs[];  // [dm][kEmbedPitch] x values (frame-minor), then [E][kEmbedPitch] indicators
-  const int T = 1 + p.Lp + p.L;
-  const int blocks_per_x = (p.L + kEmbedRows - 1) / kEmbedRows;
-  if ((int)blockIdx.x >= p.NX * blocks_per_x) {      // context rows ride in the same launch (one launch fewer per step)
-    embed_ctx_rows<F16>(p, (int)blockIdx.x - p.NX * blocks_per_x);
-    return;
-  }
-  const int n = blockIdx.x / blocks_per_x;
-  const int l0 = (blockIdx.x % blocks_per_x) * kEmbedRows;
-  const int nr = min(kEmbedRows, p.L - l0);
-  float* inds = xs + p.dm * kEmbedPitch;
-  for (int i = threadIdx.x; i < kEmbedPitch * p.dm; i += blockDim.x) {
-    const int r = i / p.dm, k = i % p.dm;      // coalesced global read, transposed shared write
-    xs[k * kEmbedPitch + r] = r < nr ? p.x[((int64_t)n * p.L + l0 + r) * p.dm + k] : 0.f;
-  }
-  for (int i = threadIdx.x; i < p.E * kEmbedPitch; i += blockDim.x) {
-    const int e = i / kEmbedPitch, r = i % kEmbedPitch;
-    inds[i] = (p.indicator && r < nr) ? p.indicator[(int64_t)(e * p.NX + n) * p.L + l0 + r] : 0.f;
-  }
-  __syncthreads();
-  for (int c = 2 * threadIdx.x; c < p.d; c += 2 * blockDim.x) {
-    // accumulators start from bias + positional encoding: those 25 independent loads overlap the staging above
-    // instead of sitting, one latency each, between the stores of the epilogue
-    float a0[kEmbedPitch], a1[kEmbedPitch];
-    const float2 bc = *reinterpret_cast<const float2*>(p.bf + c);
-#pragma unroll
-    for (int r = 0; r < kEmbedPitch; ++r) {
-      float2 pe = make_float2(0.f, 0.f);
-      if (r < nr) pe = __ldg(reinterpret_cast<const float2*>(p.PE + (int64_t)(1 + p.Lp + l0 + r) * p.d + c));
-      a0[r] = bc.x + pe.x;
-      a1[r] = bc.y + pe.y;
-    }
-    // weights for 4 k at a time: the 4 loads are issued together, so their (L1/L2) latency is paid once per 224 FMAs
-    const float* wcol = p.WfT + c;
-    for (int k0 = 0; k0 < p.dm; k0 += 4) {
-      float2 w[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-        w[u] = k0 + u < p.dm ? __ldg(reinterpret_cast<const float2*>(wcol + (int64_t)(k0 + u) * p.d)) : make_float2(0.f, 0.f);
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        if (k0 + u < p.dm) {
-          const float4* xr = reinterpret_cast<const float4*>(xs + (k0 + u) * kEmbedPitch);
-#pragma unroll
-          for (int q = 0; q < kEmbedPitch / 4; ++q) {
-            const float4 xv = xr[q];
-            a0[4 * q + 0] = fmaf(xv.x, w[u].x, a0[4 * q + 0]); a1[4 * q + 0] = fmaf(xv.x, w[u].y, a1[4 * q + 0]);
-            a0[4 * q + 1] = fmaf(xv.y, w[u].x, a0[4 * q + 1]); a1[4 * q + 1] = fmaf(xv.y, w[u].y, a1[4 * q + 1]);
-            a0[4 * q + 2] = fmaf(xv.z, w[u].x, a0[4 * q + 2]); a1[4 * q + 2] = fmaf(xv.z, w[u].y, a1[4 * q + 2]);
-            a0[4 * q + 3] = fmaf(xv.w, w[u].x, a0[4 * q + 3]); a1[4 * q + 3] = fmaf(xv.w, w[u].y, a1[4 * q + 3]);
-          }
-        }
-      }
-    }
-    const float2 wi = *reinterpret_cast<const float2*>(p.WfT + (int64_t)p.dm * p.d + c);
-#pragma unroll
-    for (int r = 0; r < kEmbedRows; ++r) {
-      if (r < nr) {
-        const int l = l0 + r;
-        for (int e = 0; e < p.E; ++e) {
-          const float ind = inds[e * kEmbedPitch + r];
-          const int s = e * p.NX + n;
-          *reinterpret_cast<uint32_t*>(p.out + ((int64_t)s * T + 1 + p.Lp + l) * p.d + c) =
-              pack_h<F16>(fmaf(ind, wi.x, a0[r]), fmaf(ind, wi.y, a1[r]));
-        }
-      }
-    }
-  }
-}
-
-// The same rows on the tensor cores.  feature_proj is a [rows, dm] x [dm, 512] product with fp32 inputs (x_t is the
-// sampler state) and a 16-bit output: three mma.sync passes over fp16 two-term splits (x = hi + lo, W = hi + lo:
-// hi*hi + lo*hi + hi*lo, 22 mantissa bits - the result rounds to the same 16-bit value as the fp32 FMA chain except
-// for rare last-bit ties) cost 240 MMAs per warp instead of 3800 FFMAs + 480 shared-memory loads per thread.
+// rows Lp+1..: feature_proj([x_t, indicator]) + PE, computed once per x row and written to its E sequences, on the
+// tensor cores.  feature_proj is a [rows, dm] x [dm, 512] product with fp32 inputs (x_t is the sampler state) and a
+// 16-bit output: three mma.sync passes over fp16 two-term splits (x = hi + lo, W = hi + lo: hi*hi + lo*hi + hi*lo,
+// 22 mantissa bits - the result rounds to the same 16-bit value as the fp32 FMA chain except for rare last-bit ties)
+// cost 240 MMAs per warp where the FMA chain costs 3800 FFMAs + 480 shared-memory loads per thread.
 //   CTA   = 32 consecutive x rows (clip boundaries may fall inside a tile) x 512 features, 8 warps x 64 features
 //   A     = the rows' hi / lo halves in shared memory (pitch 88: ldmatrix conflict-free), K zero-padded to 80
 //   B     = Wf16 [n][k] fragments straight from global memory (164 KB in all: L1 / L2 resident)
@@ -231,8 +153,6 @@ __device__ __forceinline__ void em_mma(float (&d)[4], const uint32_t (&a)[4], ui
 }
 template <bool F16>
 __global__ void __launch_bounds__(256, 2) embed_x_mma_kernel(EmbedParams p) {
-  griddep_launch();
-  griddep_wait();
   extern __shared__ __align__(16) uint8_t esm[];
   const int T = 1 + p.Lp + p.L;
   const int rows_total = p.NX * p.L;
@@ -353,23 +273,19 @@ __global__ void __launch_bounds__(256, 2) embed_x_mma_kernel(EmbedParams p) {
   }
 }
 int embed_launch(const EmbedParams& p, cudaStream_t st) {
+  MSMD_REQUIRE(p.Wf16 != nullptr && p.d == 512 && p.dm <= kEmK && p.E <= 3,
+               "embed: built for d_model = 512, motion_dim + n_basis <= %d and <= 3 guidance entries (got %d, %d, %d)",
+               kEmK, p.d, p.dm, p.E);
   ProfileScope prof("embed", st);
-  static const bool use_mma = [] { const char* e = getenv("MSMD_EMBED_MMA"); return e ? atoi(e) != 0 : true; }();
-  if (use_mma && p.Wf16 != nullptr && p.d == 512 && p.dm <= kEmK && p.E <= 3) {
-    static bool attr = false;
-    if (!attr) {
-      MSMD_CHECK_CUDA(cudaFuncSetAttribute(embed_x_mma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEmSmem));
-      MSMD_CHECK_CUDA(cudaFuncSetAttribute(embed_x_mma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEmSmem));
-      attr = true;
-    }
-    const int blocks = cdiv(p.NX * p.L, kEmRows) + p.S * (p.Lp + 1);
-    MSMD_CHECK_CUDA(launch_pdl(p.fp16 ? embed_x_mma_kernel<true> : embed_x_mma_kernel<false>, dim3(blocks), dim3(256), kEmSmem, st, p));
-    MSMD_CHECK_LAUNCH();
-    return MSMD_OK;
+  static bool attr = false;
+  if (!attr) {
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(embed_x_mma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEmSmem));
+    MSMD_CHECK_CUDA(cudaFuncSetAttribute(embed_x_mma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEmSmem));
+    attr = true;
   }
-  const int blocks = p.NX * ((p.L + kEmbedRows - 1) / kEmbedRows) + p.S * (p.Lp + 1);
-  MSMD_CHECK_CUDA(launch_pdl(p.fp16 ? embed_x_kernel<true> : embed_x_kernel<false>, dim3(blocks), dim3(256),
-                             (p.dm + 3) * kEmbedPitch * sizeof(float), st, p));
+  const int blocks = cdiv(p.NX * p.L, kEmRows) + p.S * (p.Lp + 1);
+  if (p.fp16) embed_x_mma_kernel<true><<<blocks, 256, kEmSmem, st>>>(p);
+  else embed_x_mma_kernel<false><<<blocks, 256, kEmSmem, st>>>(p);
   MSMD_CHECK_LAUNCH();
   return MSMD_OK;
 }
@@ -414,108 +330,13 @@ __device__ __forceinline__ void load_h4(const bf16* src, float* v) {
   else { v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y; }
 }
 
-// LayerNorm chain of the post-LN layers: out = LN2(LN1(y + resid) + add) (LN3: out = LN(y + resid)).  Inside the replayed
-// step y and the residual stream come out of L2 (ncu --cache-control none: 90% L2 hits, 2.5 MB of DRAM traffic), so the
-// kernel is bound by instruction issue and load latency, not by HBM.  Hence: a warp owns kLnRows consecutive rows;
-// a lane owns two 16-byte chunks of a row (8 + 8 of the 512 features: a quarter of the load instructions of the 8-byte
-// version); gamma / beta sit in shared memory (read once per CTA instead of once per row); the raw 16-bit words of the NEXT
-// row are in flight while the current one is normalised; statistics are fp32, two-pass, in registers.
-template <bool F16>
-__device__ __forceinline__ void ln_unpack8(const uint4& u, float* v, bool add) {
-  const float2 a = unpack_h<F16>(u.x), b = unpack_h<F16>(u.y), c = unpack_h<F16>(u.z), d = unpack_h<F16>(u.w);
-  if (add) { v[0] += a.x; v[1] += a.y; v[2] += b.x; v[3] += b.y; v[4] += c.x; v[5] += c.y; v[6] += d.x; v[7] += d.y; }
-  else { v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y; v[4] = c.x; v[5] = c.y; v[6] = d.x; v[7] = d.y; }
-}
-template <bool F16>
-__device__ __forceinline__ uint4 ln_pack8(const float* v) {
-  return make_uint4(pack_h<F16>(v[0], v[1]), pack_h<F16>(v[2], v[3]), pack_h<F16>(v[4], v[5]), pack_h<F16>(v[6], v[7]));
-}
-// normalise the 16 values of this lane (row of 512 over the warp) with gamma / beta from shared memory
-__device__ __forceinline__ void ln16(float (&v)[16], const float* __restrict__ sg, const float* __restrict__ sb, int lane) {
-  float s = 0.f;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) s += v[i];
-  const float mean = warp_sum(s) * (1.0f / 512.0f);
-  float q = 0.f;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) { v[i] -= mean; q = fmaf(v[i], v[i], q); }
-  const float rstd = rsqrtf(warp_sum(q) * (1.0f / 512.0f) + 1e-5f);
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    const float4 g0 = *reinterpret_cast<const float4*>(sg + h * 256 + lane * 8), g1 = *reinterpret_cast<const float4*>(sg + h * 256 + lane * 8 + 4);
-    const float4 b0 = *reinterpret_cast<const float4*>(sb + h * 256 + lane * 8), b1 = *reinterpret_cast<const float4*>(sb + h * 256 + lane * 8 + 4);
-    float* w = v + 8 * h;
-    w[0] = fmaf(w[0] * rstd, g0.x, b0.x); w[1] = fmaf(w[1] * rstd, g0.y, b0.y); w[2] = fmaf(w[2] * rstd, g0.z, b0.z); w[3] = fmaf(w[3] * rstd, g0.w, b0.w);
-    w[4] = fmaf(w[4] * rstd, g1.x, b1.x); w[5] = fmaf(w[5] * rstd, g1.y, b1.y); w[6] = fmaf(w[6] * rstd, g1.z, b1.z); w[7] = fmaf(w[7] * rstd, g1.w, b1.w);
-  }
-}
-
-template <int D, bool F16, int kLnRows>
-__global__ void __launch_bounds__(256) ln_kernel(LnParams p) {
-  static_assert(D == 512, "lane layout: two 8-element chunks per lane");
-  griddep_launch();
-  __shared__ __align__(16) float sgb[4][D];          // g1, b1, g2, b2
-  for (int i = threadIdx.x; i < D; i += blockDim.x) {
-    sgb[0][i] = p.g1[i]; sgb[1][i] = p.b1[i];
-    sgb[2][i] = p.g2 ? p.g2[i] : 0.f; sgb[3][i] = p.b2 ? p.b2[i] : 0.f;
-  }
-  griddep_wait();
-  __syncthreads();
-  const int lane = threadIdx.x & 31;
-  const int row0 = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * kLnRows;
-  const int c0 = lane * 8, c1 = 256 + lane * 8;
-  struct Raw { uint4 y0, y1, r0, r1, a0, a1; };
-  auto load = [&](int row, Raw& w) {
-    if (row >= p.M) return;
-    const bf16* y = p.y + (int64_t)row * D;
-    w.y0 = *reinterpret_cast<const uint4*>(y + c0); w.y1 = *reinterpret_cast<const uint4*>(y + c1);
-    if (p.resid != nullptr) {
-      const bf16* r = p.resid + (int64_t)row * D;
-      w.r0 = *reinterpret_cast<const uint4*>(r + c0); w.r1 = *reinterpret_cast<const uint4*>(r + c1);
-    }
-    const int s = row / p.T, tok = row - s * p.T;
-    if (p.add != nullptr && tok > 0) {
-      const bf16* a = p.add + ((int64_t)s * (p.T - 1) + (tok - 1)) * D;
-      w.a0 = __ldg(reinterpret_cast<const uint4*>(a + c0)); w.a1 = __ldg(reinterpret_cast<const uint4*>(a + c1));
-    }
-  };
-  Raw cur, nxt;
-  load(row0, cur);
-#pragma unroll
-  for (int i = 0; i < kLnRows; ++i) {
-    const int row = row0 + i;
-    if (i + 1 < kLnRows) load(row + 1, nxt);
-    if (row < p.M) {
-      const int s = row / p.T, tok = row - s * p.T;
-      float v[16];
-      ln_unpack8<F16>(cur.y0, v, false); ln_unpack8<F16>(cur.y1, v + 8, false);
-      if (p.resid != nullptr) {  // x + sublayer(x): the residual add of the post-LN layer (model.py:874-878)
-        ln_unpack8<F16>(cur.r0, v, true); ln_unpack8<F16>(cur.r1, v + 8, true);
-      }
-      if (!(tok == 0 && p.skip_tok0)) {
-        ln16(v, sgb[0], sgb[1], lane);
-        if (tok == 0 && p.x0 != nullptr) {
-          bf16* o = p.x0 + (int64_t)s * D;
-          *reinterpret_cast<uint4*>(o + c0) = ln_pack8<F16>(v); *reinterpret_cast<uint4*>(o + c1) = ln_pack8<F16>(v + 8);
-        } else {
-          if (p.add != nullptr && tok > 0) {
-            // x1 is rounded to 16 bits where the reference's next sub-layer reads it; keep the same rounding point
-            ln_unpack8<F16>(cur.a0, v, true); ln_unpack8<F16>(cur.a1, v + 8, true);
-            ln16(v, sgb[2], sgb[3], lane);
-          }
-          bf16* o = p.out + (int64_t)row * D;
-          *reinterpret_cast<uint4*>(o + c0) = ln_pack8<F16>(v); *reinterpret_cast<uint4*>(o + c1) = ln_pack8<F16>(v + 8);
-        }
-      }
-    }
-    cur = nxt;
-  }
-}
-// Default kernel: one row per warp, 8-byte loads, parameters from global memory (46 registers: high occupancy)
+// LayerNorm chain of the post-LN layers: out = LN2(LN1(y + resid) + add) (LN3: out = LN(y + resid)).  One row per warp,
+// 8-byte loads, parameters from global memory (46 registers: high occupancy).  Inside the replayed step y and the
+// residual stream come out of L2 (ncu --cache-control none: 90% L2 hits, 2.5 MB of DRAM traffic) and occupancy (2664
+// CTAs at configuration 3) hides the load latency: a kernel with 16-byte loads, gamma / beta in shared memory and the next
+// row's loads in flight measured 1.2% slower per step with 6 rows per warp (one wave of 444 CTAs) and 3% slower with 4.
 template <int D, bool F16>
-__global__ void __launch_bounds__(256) ln_kernel_v1(LnParams p) {
-  griddep_launch();
-  griddep_wait();
+__global__ void __launch_bounds__(256) ln_kernel(LnParams p) {
   constexpr int NV = D / 32;
   const int lane = threadIdx.x & 31;
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -530,7 +351,6 @@ __global__ void __launch_bounds__(256) ln_kernel_v1(LnParams p) {
 #pragma unroll
     for (int i = 0; i < NV / 4; ++i) load_h4<F16, true>(r + i * 128 + lane * 4, v + 4 * i);
   }
-  if (tok == 0 && p.skip_tok0) return;
   ln_row<D>(v, p.g1, p.b1, lane);
   if (tok == 0 && p.x0 != nullptr) {
 #pragma unroll
@@ -551,155 +371,8 @@ __global__ void __launch_bounds__(256) ln_kernel_v1(LnParams p) {
 int ln_launch(const LnParams& p, cudaStream_t st) {
   MSMD_REQUIRE(p.d == 512, "ln: only d_model = 512 is instantiated (got %d)", p.d);
   ProfileScope prof(p.add ? "ln1_ln2" : "ln3", st);
-  // MSMD_LN_ROWS (A/B): 0 = one row per warp with 8-byte loads (default: measured fastest inside the replayed step, where
-  // y and the residual stream come out of L2 and occupancy - 46 registers, 2664 CTAs - hides the load latency);
-  // 1 / 4 / 6 = the 16-byte-load kernel with that many rows per warp (6: one wave of 444 CTAs at configuration 3;
-  // measured 1.2% SLOWER per step than 0 on the same box, 4 rows 3% slower)
-  static const int rows = [] { const char* e = getenv("MSMD_LN_ROWS"); return e ? atoi(e) : 0; }();
-  if (rows == 0) {
-    MSMD_CHECK_CUDA(launch_pdl(p.fp16 ? ln_kernel_v1<512, true> : ln_kernel_v1<512, false>, dim3(cdiv(p.M, 8)), dim3(256), 0, st, p));
-  } else if (rows == 1 || p.M <= 148 * 3 * 8) {
-    MSMD_CHECK_CUDA(launch_pdl(p.fp16 ? ln_kernel<512, true, 1> : ln_kernel<512, false, 1>, dim3(cdiv(p.M, 8)), dim3(256), 0, st, p));
-  } else if (rows == 4 || p.M < 148 * 3 * 8 * 4) {
-    MSMD_CHECK_CUDA(launch_pdl(p.fp16 ? ln_kernel<512, true, 4> : ln_kernel<512, false, 4>, dim3(cdiv(p.M, 8 * 4)), dim3(256), 0, st, p));
-  } else {
-    MSMD_CHECK_CUDA(launch_pdl(p.fp16 ? ln_kernel<512, true, 6> : ln_kernel<512, false, 6>, dim3(cdiv(p.M, 8 * 6)), dim3(256), 0, st, p));
-  }
-  MSMD_CHECK_LAUNCH();
-  return MSMD_OK;
-}
-
-template <int D, bool F16>
-__global__ void __launch_bounds__(256) ln_row0_kernel(const bf16* __restrict__ y0, const bf16* __restrict__ resid0,
-                                                      const float* __restrict__ g, const float* __restrict__ b,
-                                                      bf16* __restrict__ out, bf16* __restrict__ out_c, int S, int T) {
-  griddep_launch();
-  griddep_wait();
-  constexpr int NV = D / 32;
-  const int lane = threadIdx.x & 31;
-  const int s = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (s >= S) return;
-  float v[NV];
-#pragma unroll
-  for (int i = 0; i < NV / 4; ++i) {
-    load_h4<F16, false>(y0 + (int64_t)s * D + i * 128 + lane * 4, v + 4 * i);
-    if (resid0 != nullptr) load_h4<F16, true>(resid0 + (int64_t)s * D + i * 128 + lane * 4, v + 4 * i);
-  }
-  ln_row<D>(v, g, b, lane);
-#pragma unroll
-  for (int i = 0; i < NV / 4; ++i) {
-    if (out) store_h4<F16>(out + (int64_t)s * T * D + i * 128 + lane * 4, v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
-    if (out_c) store_h4<F16>(out_c + (int64_t)s * D + i * 128 + lane * 4, v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
-  }
-}
-int ln_row0_launch(const bf16* y0, const bf16* resid0, const float* g, const float* b, bf16* out, bf16* out_c, int S,
-                   int T, int d, int fp16, cudaStream_t st) {
-  MSMD_REQUIRE(d == 512, "ln_row0: only d_model = 512 is instantiated");
-  ProfileScope prof("ln_row0", st);
-  MSMD_CHECK_CUDA(launch_pdl(fp16 ? ln_row0_kernel<512, true> : ln_row0_kernel<512, false>, dim3(cdiv(S, 8)), dim3(256), 0, st,
-                             y0, resid0, g, b, out, out_c, S, T));
-  MSMD_CHECK_LAUNCH();
-  return MSMD_OK;
-}
-
-// ------------------------------------------------------------------------------------------- row-0 cross attention
-// Person token (query row 0) over the Tk memory tokens (nn.MultiheadAttention inside _mha_block): one warp per
-// (sequence, head), no shared memory and no barriers.  K: lane j of key group g reads its key's 128-byte head
-// slice with 8 x 16-byte loads (the half-used sectors of one load are completed by the next, out of L1); V: lane
-// owns 2 of the 64 head dims, so a key's V slice is one coalesced 128-byte warp load, prefetched 28 keys ahead.
-// HBM-bound: 2 x Tk x d x 2 B per sequence per layer.
-constexpr int kCaBatch = 28;
-template <bool F16>
-__global__ void __launch_bounds__(128, 3) cross_attn_row0_kernel(const bf16* __restrict__ q0, const bf16* __restrict__ kv,
-                                                                 bf16* __restrict__ ctx0, int Tk, int H) {
-  griddep_launch();
-  griddep_wait();
-  constexpr int d = 512;
-  const int w = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;   // warp = (sequence, head)
-  const int s = w / H, h = w % H;
-  const bf16* kbase = kv + (int64_t)s * Tk * 2 * d + h * 64;
-  const uint32_t* vbase = reinterpret_cast<const uint32_t*>(kbase + d) + lane;
-  const int64_t vstride = d;   // one key row = 2d bf16 = d uint32
-
-  uint32_t vb[2][kCaBatch];
-  auto load_v = [&](int b, uint32_t (&dst)[kCaBatch]) {
-#pragma unroll
-    for (int u = 0; u < kCaBatch; ++u) {
-      const int j = b * kCaBatch + u;
-      dst[u] = j < Tk ? __ldg(vbase + (int64_t)j * vstride) : 0u;
-    }
-  };
-  load_v(0, vb[0]);
-
-  float q[64];
-  {
-    const uint4* qp = reinterpret_cast<const uint4*>(q0 + (int64_t)s * d + h * 64);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const uint4 u = __ldg(qp + i);
-      const uint32_t ww[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const float2 f = unpack_h<F16>(ww[k]);
-        q[i * 8 + 2 * k] = f.x;
-        q[i * 8 + 2 * k + 1] = f.y;
-      }
-    }
-  }
-  float sc[4];
-#pragma unroll
-  for (int grp = 0; grp < 4; ++grp) {
-    const int j = grp * 32 + lane;
-    float dot = -INFINITY;
-    if (j < Tk) {
-      const uint4* kp = reinterpret_cast<const uint4*>(kbase + (int64_t)j * 2 * d);
-      uint4 kr[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) kr[i] = __ldg(kp + i);
-      float acc = 0.f;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const uint32_t ww[4] = {kr[i].x, kr[i].y, kr[i].z, kr[i].w};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const float2 f = unpack_h<F16>(ww[k]);
-          acc = fmaf(q[i * 8 + 2 * k], f.x, acc);
-          acc = fmaf(q[i * 8 + 2 * k + 1], f.y, acc);
-        }
-      }
-      dot = acc * 0.125f;
-    }
-    sc[grp] = dot;
-  }
-  const float m = warp_max(fmaxf(fmaxf(sc[0], sc[1]), fmaxf(sc[2], sc[3])));
-  float l = 0.f;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { sc[i] = (sc[i] == -INFINITY) ? 0.f : __expf(sc[i] - m); l += sc[i]; }
-  l = warp_sum(l);
-  float oa = 0.f, ob = 0.f;
-  auto consume = [&](int b, const uint32_t (&src)[kCaBatch]) {
-#pragma unroll
-    for (int u = 0; u < kCaBatch; ++u) {
-      const int j = b * kCaBatch + u;            // compile-time after unrolling: sc[] stays in registers
-      const float p = __shfl_sync(0xffffffffu, sc[j >> 5], j & 31);
-      const float2 f = unpack_h<F16>(src[u]);
-      oa = fmaf(p, f.x, oa);
-      ob = fmaf(p, f.y, ob);
-    }
-  };
-  load_v(1, vb[1]); consume(0, vb[0]);
-  load_v(2, vb[0]); consume(1, vb[1]);
-  load_v(3, vb[1]); consume(2, vb[0]);
-  consume(3, vb[1]);
-  const float inv = 1.0f / l;
-  *reinterpret_cast<uint32_t*>(ctx0 + (int64_t)s * d + h * 64 + 2 * lane) = pack_h<F16>(oa * inv, ob * inv);
-}
-int cross_attn_row0_launch(const bf16* q0, const bf16* kv, bf16* ctx0, int S, int Tk, int H, int fp16, cudaStream_t st) {
-  MSMD_REQUIRE(Tk <= 4 * kCaBatch && H == 8, "cross_attn_row0: built for 8 heads x 64 and <= %d memory tokens (got %d, %d)",
-               4 * kCaBatch, H, Tk);
-  ProfileScope prof("cross_attn_row0", st);
-  MSMD_CHECK_CUDA(launch_pdl(fp16 ? cross_attn_row0_kernel<true> : cross_attn_row0_kernel<false>, dim3(S * H / 4), dim3(128), 0, st,
-                             q0, kv, ctx0, Tk, H));
+  if (p.fp16) ln_kernel<512, true><<<cdiv(p.M, 8), 256, 0, st>>>(p);
+  else ln_kernel<512, false><<<cdiv(p.M, 8), 256, 0, st>>>(p);
   MSMD_CHECK_LAUNCH();
   return MSMD_OK;
 }
@@ -737,8 +410,6 @@ __device__ __forceinline__ void split_target(const float* dec, const float* stat
 // stream-ordered copy): the captured step graph never bakes a caller pointer or scalar, so one instantiated graph
 // serves every window / call of the same shape.
 __global__ void __launch_bounds__(256) update_kernel(const UpdateParams* __restrict__ pp) {
-  griddep_launch();
-  griddep_wait();
   // the parameter block is read through shared memory: as a local copy of *pp its ~30 fields were re-fetched from global
   // memory (generic loads) all over the loop, one more dependent latency in front of every data load
   __shared__ __align__(16) unsigned char p_raw[sizeof(UpdateParams)];
@@ -958,7 +629,7 @@ int update_launch(const UpdateParams* d_p, int NX, int L, int dm, cudaStream_t s
   ProfileScope prof("update", st);
   // warp per row, ONE wave (2 CTAs of 123 registers per SM): every CTA starts with a chain of dependent scalar loads
   // (parameter block -> step index -> schedule coefficients, ~2 us); the 4-wave grid of round 1 paid it four times
-  MSMD_CHECK_CUDA(launch_pdl(update_kernel, dim3(std::min(cdiv(NX * L, 8), kNumSMs * 2)), dim3(256), 0, st, d_p));
+  update_kernel<<<std::min(cdiv(NX * L, 8), kNumSMs * 2), 256, 0, st>>>(d_p);
   MSMD_CHECK_LAUNCH();
   return MSMD_OK;
 }

@@ -32,8 +32,8 @@ struct EmbedParams {
   const float* indicator; // [S, L] or null (-> no indicator column)
   const float* WfT;       // [dm+1, d] feature_proj weight transposed (k-major), fp32
   const float* bf;        // [d]
-  const void* Wf16;       // [2][d][80] fp16: hi | lo halves of feature_proj.weight[:, :dm] (K zero-padded to 80), or null
-                          // (-> the CUDA-core kernel); the tensor-core embedding (embed_x_mma_kernel) needs d = 512, dm <= 80
+  const void* Wf16;       // [2][d][80] fp16: hi | lo halves of feature_proj.weight[:, :dm] (K zero-padded to 80); the
+                          // tensor-core embedding (embed_x_mma_kernel) needs d = 512, dm <= 80
   bf16* out;              // [S, 1+Lp+L, d]
   int S, NX, E, Lp, L, d, dm;
   int fp16;               // storage format of `out`
@@ -50,19 +50,10 @@ struct LnParams {
   const float* g2; const float* b2;   // used iff add != null
   bf16* out;                // [M, d]
   bf16* x0;                 // [S, d] or null
-  int skip_tok0;            // do not write token-0 rows at all (they are produced by the person-token stream)
   int M, T, d;
   int fp16;                 // storage format of y / resid / add / out / x0
 };
 int ln_launch(const LnParams& p, cudaStream_t st);
-// row-0 finish: LayerNorm(y0 [S,d]; g,b) -> out[s*T + 0]
-// LayerNorm(y0 + resid0) of the S person-token rows -> out[s*T + 0] (if out) and compact out_c[s] (if out_c)
-int ln_row0_launch(const bf16* y0, const bf16* resid0, const float* g, const float* b, bf16* out, bf16* out_c, int S,
-                   int T, int d, int fp16, cudaStream_t st);
-
-// row-0 cross attention: q0 [S,d]; kv [S*Tk, 2d] (k|v) -> ctx0 [S,d]
-int cross_attn_row0_launch(const bf16* q0, const bf16* kv, bf16* ctx0, int S, int Tk, int H, int fp16, cudaStream_t st);
-
 
 // One visited step t of a respaced schedule (msmd_sample_window_sched): x_s = c0 x_t + c1 out + c2 h_p + sigma z_t,
 // where out is the network output (x0_hat or eps_hat), h_p the data prediction of the previous step (history buffer;

@@ -27,11 +27,6 @@ static std::map<std::string, std::pair<double, long>> g_totals;
 
 bool profiling_on() { return g_prof; }
 
-bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("MSMD_PDL"); return e && atoi(e) != 0; }();
-  return on;
-}
-
 ProfileScope::ProfileScope(const char* n, cudaStream_t s) : name(n), st(s) {
   if (!g_prof) return;
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;

@@ -600,8 +600,7 @@ extern "C" int msmd_flame_decode(msmd_flame* fh, const float* betas, const float
   if (rc) return rc;
   {
     ProfileScope prof("flame_pose", st);
-    static const bool pose_mma_on = [] { const char* e = getenv("MSMD_FLAME_POSE_MMA"); return e ? atoi(e) != 0 : true; }();
-    if (pose_mma_on && fh->NB % 2 == 0 && fh->Jb16 != nullptr && reinterpret_cast<uintptr_t>(betas) % 8 == 0)   // (float2 loads of the coefficients)
+    if (fh->NB % 2 == 0 && fh->Jb16 != nullptr && reinterpret_cast<uintptr_t>(betas) % 8 == 0)   // (float2 loads of the coefficients)
       flame_pose_mma_kernel<5><<<cdiv(B, 32), 256, 0, st>>>(betas, pose, pose2rot, B, fh->NB, fh->KB, fh->Kpad, fh->Jt, fh->Jb16,
                                                            fh->d_parents, fh->A, impl == 0 ? fh->A_hi : nullptr,
                                                            impl == 0 ? fh->A_lo : nullptr, fh->xf, joints_out);

@@ -30,23 +30,19 @@ namespace msmd {
 
 namespace {
 
-#ifndef MSMD_FLAME_BK
-#define MSMD_FLAME_BK 64
-#endif
-// k-block depth: 64 (128-byte rows, SWIZZLE_128B, 2 stages x 64 KB; default) or 32 (64-byte rows, SWIZZLE_64B, 4 stages x
-// 32 KB: -DMSMD_FLAME_BK=32).  Both hold the same 128 KB of operands in flight.  The timeline of the 64-deep version shows the
-// MMA loop waiting on operand delivery (20.5K cycles per super-tile for 10.8K cycles of MMA); finer slots were tried to
-// keep more fills in flight and measured SLOWER on the same box (350.6 vs 337.8 us): the limit is the L2 -> SM delivery
-// rate (~7.2 TB/s chip-wide), not slot granularity, and 64-byte rows double the request count.
-constexpr int FT_BK = MSMD_FLAME_BK;
-static_assert(FT_BK == 32 || FT_BK == 64, "k-block depth");
-constexpr int FT_STAGES = FT_BK == 32 ? 4 : 2, FT_NQ = 4, FT_G = 2;       // FT_G column tiles share every A k-block
+// k-block depth 64: 128-byte rows, SWIZZLE_128B, 2 stages x 64 KB.  The timeline shows the MMA loop waiting on operand
+// delivery (20.5K cycles per super-tile for 10.8K cycles of MMA); 32-deep slots (64-byte rows, SWIZZLE_64B, 4 stages x
+// 32 KB: the same 128 KB in flight) were tried to keep more fills in flight and measured SLOWER on the same box (350.6
+// vs 337.8 us): the limit is the L2 -> SM delivery rate (~7.2 TB/s chip-wide), not slot granularity, and 64-byte rows
+// double the request count.
+constexpr int FT_BK = 64;
+constexpr int FT_STAGES = 2, FT_NQ = 4, FT_G = 2;       // FT_G column tiles share every A k-block
 constexpr int FT_BM = 128, FT_VERT = 42, FT_BN = 126, FT_UN = 128;
 constexpr int FT_ROW_BYTES = FT_BK * 2;                  // one operand row of a k-block
 constexpr int FT_TILE_BYTES = 128 * FT_ROW_BYTES;        // one operand tile: 128 rows
 constexpr int FT_BHALF_BYTES = 64 * FT_ROW_BYTES;        // this CTA's half of a basis tile: 64 rows
 __device__ __forceinline__ uint64_t ft_desc(uint32_t smem_addr) {
-  return FT_BK == 32 ? tc::make_smem_desc_sw64(smem_addr) : tc::make_smem_desc_sw128(smem_addr);
+  return tc::make_smem_desc_sw128(smem_addr);
 }
 constexpr int FT_STAGE_BYTES = 2 * FT_TILE_BYTES + FT_G * 2 * FT_BHALF_BYTES;   // A_hi, A_lo, then per column tile: B_hi half, B_lo half
 constexpr int FT_CHUNK_V = 8;                             // vertices per epilogue chunk (24 accumulator columns)
@@ -357,7 +353,7 @@ int flame_decode_tc(msmd_flame* fh, int64_t B, float* verts_out, cudaStream_t st
   int rc;
   const auto f32 = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   const uint64_t ldk = (uint64_t)fh->Kpad * 2;
-  const auto FT_SWZ = FT_BK == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
+  const auto FT_SWZ = CU_TENSOR_MAP_SWIZZLE_128B;
   if ((rc = make_tmap_2d(&p.a_hi, fh->A_hi, f32, fh->Kpad, rows, ldk, FT_BK, FT_BM, FT_SWZ))) return rc;
   if ((rc = make_tmap_2d(&p.a_lo, fh->A_lo, f32, fh->Kpad, rows, ldk, FT_BK, FT_BM, FT_SWZ))) return rc;
   if ((rc = make_tmap_2d(&p.b_hi, fh->basis_hi, f32, fh->Kpad, fh->N3pad, ldk, FT_BK, 64, FT_SWZ))) return rc;

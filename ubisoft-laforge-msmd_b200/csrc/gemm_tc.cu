@@ -137,23 +137,21 @@ static int launch_cfg2(const GemmDesc& d, cudaStream_t st) {
   snprintf(shape_name, sizeof(shape_name), "gemm_%dx%dx%d%s", d.M, d.N, d.K, Cfg::CTA2 ? "_pair" : "");
   ProfileScope prof2(profiling_on() ? strdup(shape_name) : "", st);
   if constexpr (Cfg::CTA2) {
-    const int sms = (d.max_ctas > 0 && d.max_ctas < kNumSMs) ? d.max_ctas : kNumSMs;
-    int pairs = tiles < sms / 2 ? tiles : sms / 2;
+    int pairs = tiles < kNumSMs / 2 ? tiles : kNumSMs / 2;
     cudaLaunchConfig_t cfg = {};
     cfg.blockDim = dim3(Cfg::THREADS);
     cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
     cfg.stream = st;
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     // Clusters of 4 = two pairs on neighbouring column tiles of the same rows, the A tile fetched once and multicast
-    // (default; MSMD_GEMM_CL4=0 disables).  Bit-identical results, -1.1% per sampling step on one box: the L2 reads
+    // (default).  Bit-identical results, -1.1% per sampling step on one box: the L2 reads
     // drop by a quarter but the main loop is bound on the SM side (TMA fill 64 B/clk + MMA operand reads 64 B/clk +
     // epilogue staging against 128 B/clk of shared-memory bandwidth at MMA peak), not by L2.  Needs an even number of
     // column tiles (both pairs of a cluster then always have a tile) and enough co-resident 4-CTA clusters that no
     // round is added to the persistent schedule.
-    static const int cl4_env = [] { const char* e = getenv("MSMD_GEMM_CL4"); return e ? atoi(e) : 1; }();
-    if (cl4_env && Cfg::NSPLIT == 1 && p.tiles_n % 2 == 0 && d.max_ctas <= 0 && tiles >= 4) {
+    if (Cfg::NSPLIT == 1 && p.tiles_n % 2 == 0 && tiles >= 4) {
       static int max_cl4 = -1;     // per instantiation
       if (max_cl4 < 0) {
         cfg.gridDim = dim3(kNumSMs / 4 * 4);
@@ -175,15 +173,12 @@ static int launch_cfg2(const GemmDesc& d, cudaStream_t st) {
       }
     }
     cfg.gridDim = dim3(2 * pairs);
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    cfg.numAttrs = 1;
     MSMD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
   } else {
-    const int sms = (d.max_ctas > 0 && d.max_ctas < kNumSMs) ? d.max_ctas : kNumSMs;
-    const int grid = tiles < sms ? tiles : sms;
-    MSMD_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, p));
+    const int grid = tiles < kNumSMs ? tiles : kNumSMs;
+    kern<<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, st>>>(p);
   }
   MSMD_CHECK_LAUNCH();
   if (env_trace) {
@@ -223,13 +218,10 @@ static int dispatch16(const GemmDesc& d, cudaStream_t st) {
   const bool aux = d.aux != nullptr;
   // narrow outputs (N <= 128) use the 128-wide tile so small problems still spread over SMs
   const bool narrow = d.N <= 128;
-  static const int cta2_mode = [] { const char* e = getenv("MSMD_GEMM_CTA2"); return e ? atoi(e) : 1; }();  // 0 = never use CTA pairs
-  const bool cta2_env = cta2_mode != 0;
   // measured on B200 (tools/pair_probe.py, M = 21312): the single-CTA 128x256 tile needs 96 B/clk of operands per SM
   // at MMA peak and the L2->SM path delivers ~60, so its main loop runs at ~1.3 PFLOP/s; the pair (64 B/clk) is
   // MMA-bound.  Pair vs single: 1536x512 31.8/33.5 us, 2048x512+GELU 50.0/53.2, 512x2048 41.4/46.1, 512x512 tie.
-  const bool pair = d.cta2 == 1 || (d.cta2 < 0 && cta2_env && !aux && !d.out_f32 && d.batch <= 1 && d.N >= 256 &&
-                                    d.M >= 2048);
+  const bool pair = !aux && !d.out_f32 && d.batch <= 1 && d.N >= 256 && d.M >= 2048;
   const bool epi8 = d.gelu_heavy != 0;
   if (pair) {
     if (epi8) return launch_cfg<GemmCfg<MODE, 256, 8, false, H, H, true>, MODE>(d, st);
@@ -269,9 +261,8 @@ int gemm_tc_launch(const GemmDesc& d, cudaStream_t st) {
   MSMD_REQUIRE(d.mode == 1 || d.mode == 2, "gemm: unknown mode %d", d.mode);
   MSMD_REQUIRE(d.out_f32 && (!aux || d.aux_f32), "gemm: the three-pass modes are fp32 out");
   if (d.mode == 2) {
-    static const bool cta2_env2 = [] { const char* e = getenv("MSMD_GEMM_CTA2"); return !e || atoi(e) != 0; }();
     if (aux) return launch_cfg<GemmCfg<2, 128, 4, true, float, float>, 2>(d, st);
-    if (d.cta2 != 0 && cta2_env2 && d.batch <= 1 && d.N >= 256 && d.M >= 2048)
+    if (d.batch <= 1 && d.N >= 256 && d.M >= 2048)
       return launch_cfg<GemmCfg<2, 128, 4, false, float, float, true>, 2>(d, st);
     return launch_cfg<GemmCfg<2, 128, 4, false, float, float>, 2>(d, st);
   }

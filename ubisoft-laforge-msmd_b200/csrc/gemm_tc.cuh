@@ -166,7 +166,6 @@ __global__ void __launch_bounds__(Cfg::THREADS, 1) gemm_tc_kernel(const __grid_c
   static_assert((2 * Cfg::STAGES + 4 + 2 * Cfg::EPI_WARPS) * 8 + 4 <= 256, "barrier block overflows its 256 bytes");
   if (threadIdx.x == 0 && reinterpret_cast<uint8_t*>(bias_tile) + 2 * 256 * 4 > smem_raw + Cfg::SMEM_BYTES) __trap();
 
-  griddep_launch();   // PDL: let the next kernel of the stream get scheduled behind this one
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int crank = Cfg::CTA2 ? (int)cluster_ctarank() : 0;   // rank in the cluster (2 CTAs, or 4 = two pairs when p.cl4)
   const int cta_rank = crank & 1;                             // rank in the CTA pair
@@ -199,7 +198,6 @@ __global__ void __launch_bounds__(Cfg::THREADS, 1) gemm_tc_kernel(const __grid_c
   else __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  griddep_wait();     // PDL: everything above overlapped the previous kernel's tail; its outputs are visible from here
 
   auto tile_coords = [&](int t, int& m0, int& n0, int& z) {
     const int per_z = p.tiles_m * p.tiles_n;
@@ -577,8 +575,6 @@ struct GemmDesc {
   int wz_mod = -1;              // see GemmParams (only read when batch > 1)
   int bias_zstride = 0;
   int gelu_heavy = 0;           // use 8 epilogue warps
-  int cta2 = -1;                // CTA-pair tiles: -1 auto (large bf16 GEMMs without aux), 0 off, 1 force
-  int max_ctas = 0;             // > 0: cap the persistent grid (leave SMs to a concurrent stream)
 };
 
 int gemm_tc_launch(const GemmDesc& d, cudaStream_t st);

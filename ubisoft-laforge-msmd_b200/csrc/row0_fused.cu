@@ -151,13 +151,12 @@ __device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], 
 template <bool F16>
 __global__ void __cluster_dims__(kHeads, 1, 1) __launch_bounds__(kThreads, 1) row0_fused_kernel(const Row0Params p) {
   extern __shared__ __align__(16) uint8_t sm[];
-  griddep_launch();
   r0_stamp(p.trace, 0);
   bf16* wq = reinterpret_cast<bf16*>(sm + kOffWq);
   bf16* wo = reinterpret_cast<bf16*>(sm + kOffWo);
   bf16* xs = reinterpret_cast<bf16*>(sm + kOffXs);
   float* qs = reinterpret_cast<float*>(sm + kOffQs);
-  bf16* cs = reinterpret_cast<bf16*>(sm + kOffCs);   // ctx_h of the group, 16-bit (the format the unfused chain stores it in)
+  bf16* cs = reinterpret_cast<bf16*>(sm + kOffCs);   // ctx_h of the group, 16-bit (the format every attention output is stored in)
   float* po = reinterpret_cast<float*>(sm + kOffPo);
   float* st = reinterpret_cast<float*>(sm + kOffSt);   // [2][32]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -167,7 +166,7 @@ __global__ void __cluster_dims__(kHeads, 1, 1) __launch_bounds__(kThreads, 1) ro
   const int s_begin = (int)(((int64_t)p.S * cid) / ncl), s_end = (int)(((int64_t)p.S * (cid + 1)) / ncl);
 
   // ---- phase 0a: weight slices, asynchronously (cp.async: all 16 chunks of a thread in flight at once; they are
-  // only needed by phase 1 / phase 3).  Independent of the previous kernel's output.
+  // only needed by phase 1 / phase 3).
 #pragma unroll
   for (int u = 0; u < kDh * (kD / 8) / kThreads; ++u) {        // Wq0 rows 64h..64h+63, 64 x 16-byte chunks each
     const int i = tid + u * kThreads, r = i >> 6, c = i & 63;
@@ -180,7 +179,6 @@ __global__ void __cluster_dims__(kHeads, 1, 1) __launch_bounds__(kThreads, 1) ro
     cp_async16(wo + r * kWoPitch + c * 8, p.Wo + (int64_t)r * kD + h * kDh + c * 8);
   }
   asm volatile("cp.async.commit_group;" ::: "memory");
-  griddep_wait();
 
   for (int s0 = s_begin; s0 < s_end; s0 += kMaxGroup) {
     const int n = min(kMaxGroup, s_end - s0);
@@ -491,7 +489,7 @@ int row0_fused_launch(const bf16* x0c, const bf16* Wq, const float* bq, const bf
   }
   const int ncl = S < max_clusters ? S : max_clusters;
   ProfileScope prof("row0_fused", st);
-  MSMD_CHECK_CUDA(launch_pdl(kern, dim3(ncl * kHeads), dim3(kThreads), kSmem, st, p));
+  kern<<<ncl * kHeads, kThreads, kSmem, st>>>(p);
   MSMD_CHECK_LAUNCH();
 #ifdef MSMD_ROW0_TRACE
   {

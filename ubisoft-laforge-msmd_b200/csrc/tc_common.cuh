@@ -220,17 +220,6 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr) {
   d |= (uint64_t)2 << 61;                       // SWIZZLE_128B
   return d;
 }
-// Same for rows of exactly 64 bytes, SWIZZLE_64B (TMA box {64B inner, rows}, CU_TENSOR_MAP_SWIZZLE_64B): 8-row groups
-// are 512 B apart; layout type 4.  Tile bases must be 512-byte aligned.
-__device__ __forceinline__ uint64_t make_smem_desc_sw64(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(512 >> 4) << 32;              // stride byte offset: 8 rows * 64 B
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)4 << 61;                       // SWIZZLE_64B
-  return d;
-}
 // Advance along K inside the 128-byte swizzle atom: +bytes/16 on the start-address field.
 __device__ __forceinline__ uint64_t desc_advance(uint64_t d, uint32_t bytes) { return d + (uint64_t)(bytes >> 4); }
 
