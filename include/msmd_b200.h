@@ -121,7 +121,7 @@ typedef struct {
   int d_style;          /* 256 */
   int d_shape;          /* 100 */
   int motion_dim;       /* 67  */
-  int n_basis;          /* 4   */
+  int n_basis;          /* 4;  >= 1 (the reference has no result for num_of_basis = 0), motion_dim + n_basis <= 80 */
   int n_diff_steps;     /* 500 */
   int use_indicator;    /* 1   */
   int align_mask_width; /* 1; >= 0.  Band of the cross-attention mask: motion token i sees memory tokens

@@ -358,7 +358,9 @@ extern "C" int msmd_create(const msmd_config* cfg, int device, msmd_model** out)
                "msmd_create: sequence 1 + n_prev_motions + n_motions = %d exceeds the 112-token attention tile "
                "(the released configuration is 1 + 10 + 100)", 1 + c.n_prev_motions + c.n_motions);
   MSMD_REQUIRE(c.n_layers > 0 && c.d_ff > 0 && c.d_ff % 8 == 0 && c.max_seqs > 0 && c.n_diff_steps > 0, "msmd_create: bad sizes");
-  MSMD_REQUIRE(c.motion_dim > 3 && c.n_basis >= 0 && c.motion_dim + c.n_basis <= 80, "msmd_create: motion_dim + n_basis > 80");
+  MSMD_REQUIRE(c.n_basis >= 1, "msmd_create: n_basis=%d (the network mixes its output from at least one static basis: "
+               "the reference cannot run num_of_basis = 0)", c.n_basis);
+  MSMD_REQUIRE(c.motion_dim > 3 && c.motion_dim + c.n_basis <= 80, "msmd_create: motion_dim + n_basis > 80");
   MSMD_REQUIRE(c.align_mask_width >= 0, "msmd_create: align_mask_width=%d (0 = no alignment mask, w >= 1 = band of 2w-1 "
                "memory tokens)", c.align_mask_width);
   MSMD_REQUIRE(c.precision >= 0 && c.precision <= 3,
@@ -577,17 +579,20 @@ extern "C" int msmd_window_begin(msmd_model* m, const float* audio, const float*
   MSMD_REQUIRE(S > 0 && NX > 0 && E > 0 && S == NX * E, "msmd_window_begin: S=%d must equal NX*E=%d*%d", S, NX, E);
   MSMD_REQUIRE(S <= c.max_seqs, "msmd_window_begin: %d sequences exceed the capacity %d given at create", S, c.max_seqs);
   MSMD_REQUIRE(E <= 3, "msmd_window_begin: at most 2 guidance conditions (3 entries)");
-  MSMD_REQUIRE(audio && person && style && prev_motion && prev_audio, "msmd_window_begin: null conditioning tensor");
+  const int d = c.d_model, Lp = c.n_prev_motions, dm = c.motion_dim;
+  // at n_prev_motions = 0 the context tensors are empty (an empty torch tensor has no storage: a null pointer)
+  MSMD_REQUIRE(audio && person && style && (Lp == 0 || (prev_motion && prev_audio)),
+               "msmd_window_begin: null conditioning tensor");
   MSMD_REQUIRE(!c.use_indicator || indicator, "Missing indicator: the model was built with use_indicator");
   int rc;
   if ((rc = poll_overflow(m, "msmd_window_begin"))) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int d = c.d_model, Lp = c.n_prev_motions, dm = c.motion_dim;
   m->S = S; m->NX = NX; m->E = E;
   // the conditioning the later (lazy) cache passes and every step read is copied into the handle: the caller's tensors
   // may be released as soon as this call returns, and the step graph only ever sees engine-owned addresses
   MSMD_CHECK_CUDA(cudaMemcpyAsync(m->w_audio, audio, (size_t)S * c.n_motions * d * 4, cudaMemcpyDeviceToDevice, st));
-  MSMD_CHECK_CUDA(cudaMemcpyAsync(m->w_prev_audio, prev_audio, (size_t)S * Lp * d * 4, cudaMemcpyDeviceToDevice, st));
+  if (Lp > 0)
+    MSMD_CHECK_CUDA(cudaMemcpyAsync(m->w_prev_audio, prev_audio, (size_t)S * Lp * d * 4, cudaMemcpyDeviceToDevice, st));
   if (c.use_indicator)
     MSMD_CHECK_CUDA(cudaMemcpyAsync(m->w_ind, indicator, (size_t)S * c.n_motions * 4, cudaMemcpyDeviceToDevice, st));
   m->indicator = c.use_indicator ? m->w_ind : nullptr;

@@ -152,6 +152,8 @@ def hybrid_bounds(timesteps, w1, w2, tol, err16, err_main, k32=None):
 def _engine_cfg(net, n_diff_steps, target, max_seqs, precision='bf16'):
     if precision not in PRECISIONS:
         raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
+    if net.num_of_basis < 1:     # the reference's alphas = out[:, :, -0:] / torch.stack([]) give no result to match
+        raise ValueError(f'num_of_basis={net.num_of_basis}: the engine needs at least one static basis')
     return dict(n_motions=net.n_motions, n_prev_motions=net.n_prev_motions, d_model=net.feature_dim,
                 n_heads=net.n_heads, n_layers=net.n_layers, d_ff=net.mlp_ratio * net.feature_dim,
                 d_style=net.style_feat_dim if net.use_style else 0, d_shape=net.shape_feat_dim,
